@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- KeypointsGauss heatmap inference images/s on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 64] [--precision bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 64] [--precision bf16] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -68,7 +68,12 @@ def parse_args():
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of CUDA-graph replay (profiling)")
     ap.add_argument("--profile-mode", action="store_true",
                     help="device-resident loop only: no e2e loop, no per-launch breakdown, no CPU baseline (for ncu runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) to DIR/<name>.npy, to compare two builds")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def load_peaks():
@@ -368,6 +373,28 @@ def per_launch_breakdown(engine, plan, decode=True):
     return rows
 
 
+HEAT_DUMP_VALUES = 1 << 23   # 32 MB of fp32: the dump stays well under 64 MB at any workload
+
+
+def dump_outputs(out_dir, plan):
+    """--dump-outputs: what a caller of the timed path receives (KeypointsGauss.heatmaps_and_keypoints / .keypoints), as the timed
+    loop's last step left it in the plan's buffers.  heatmaps.npy: the (B,K,H,W) fp32 heatmaps; above HEAT_DUMP_VALUES values, the
+    1-D sample at a fixed seeded set of sorted flat indices instead (the same set on every run of a workload).  keypoints_yx.npy:
+    (B,K,2) (row, col) as float64 (exact).  peak_values.npy: (B,K) fp32 heatmap value at each keypoint."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    heat = plan.heat
+    if heat.numel() > HEAT_DUMP_VALUES:
+        idx = np.sort(np.random.default_rng(0).integers(0, heat.numel(), HEAT_DUMP_VALUES))
+        idx = idx[np.diff(idx, prepend=-1) > 0]                       # drop repeats (np.unique is far slower at this size)
+        heat = heat.reshape(-1)[torch.from_numpy(idx).to(heat.device)]
+    arrays = {"heatmaps": heat.cpu().numpy(), "keypoints_yx": plan.yx.cpu().numpy().astype(np.float64),
+              "peak_values": plan.maxval.cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
 
@@ -417,6 +444,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     dev_ms = max_over_ranks(start.elapsed_time(stop))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, plan)
     value = world * B * args.steps / (dev_ms * 1e-3)
     launches_per_step = plan.launches
     if args.profile_mode:

@@ -26,6 +26,9 @@ BN_EPS = 1e-5  # torch default used by nn.BatchNorm2d at src/resnet.py:46,49,139
 BN_MOMENTUM = 0.1
 NUM_CLASSES = 1000  # src/resnet_dilated.py:6 -- KeypointsGauss never overrides it (src/model.py:17)
 PREFIX = "resnet.resnet34_8s."  # KeypointsGauss.resnet (model.py:17) . Resnet34_8s.resnet34_8s (resnet_dilated.py:17)
+# torch CPU threads of tests/golden/golden_v1.*: oneDNN blocks its fp32 convolutions (and so orders their sums) by the thread count,
+# so the bit-equal golden cases reproduce only at the count they were recorded with, whatever the host's core count
+GOLDEN_CPU_THREADS = 8
 
 
 class ConvSpec(NamedTuple):

@@ -39,7 +39,7 @@ def rand_img(seed, b, h, w):
 
 def main():
     os.makedirs(OUT, exist_ok=True)
-    torch.set_num_threads(os.cpu_count())
+    torch.set_num_threads(O.GOLDEN_CPU_THREADS)
     meta = {"torch": torch.__version__, "reference": "vainaviv/hulk-keypoints", "cases": {}}
     arrays = {}
 

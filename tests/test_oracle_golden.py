@@ -12,6 +12,15 @@ from oracle import keypoints_oracle as O
 warnings.filterwarnings("ignore")
 
 
+@pytest.fixture(autouse=True)
+def golden_cpu_threads():
+    """Run each case on the CPU thread count the goldens were recorded with (see O.GOLDEN_CPU_THREADS)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(O.GOLDEN_CPU_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.fixture(scope="module")
 def sd0(golden):
     _, meta = golden

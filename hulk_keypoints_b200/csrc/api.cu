@@ -1,4 +1,4 @@
-// Library-level entry points: version, error text, device check.
+// Library-level entry points (version, error text, device check) and the host helpers every launcher shares.
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -47,6 +47,52 @@ int sm_count() {
     cached_dev = dev;
   }
   return cached;
+}
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// The driver's cuTensorMapEncodeTiled, looked up once (nullptr when the driver does not provide it).
+static EncodeTiledFn get_encode_fn() {
+  static const EncodeTiledFn fn = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+                    q == cudaDriverEntryPointSuccess;
+    return ok ? reinterpret_cast<EncodeTiledFn>(p) : nullptr;
+  }();
+  return fn;
+}
+
+int tmap_encode(CUtensorMap* m, CUtensorMapDataType dtype, int rank, const void* p, const cuuint64_t* dims, const cuuint64_t* strides,
+                const cuuint32_t* box, const cuuint32_t* estr, CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* who,
+                const char* what) {
+  const EncodeTiledFn encode = get_encode_fn();
+  if (!encode) return fail(HK_ERR_CUDA, "%s: cuTensorMapEncodeTiled entry point not available", who);
+  const CUresult r = encode(m, dtype, (cuuint32_t)rank, const_cast<void*>(p), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "%s: cuTensorMapEncodeTiled(%s) failed: %d", who, what, (int)r);
+  return HK_OK;
+}
+
+int tmap_nhwc_bf16(CUtensorMap* m, const void* p, int n, int h, int w, int c, int box_w, int box_h, int step, const char* who,
+                   const char* what) {
+  const cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
+  const cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
+  const cuuint32_t box[4] = {64, (cuuint32_t)(box_w * step), (cuuint32_t)(box_h * step), 1};
+  const cuuint32_t estr[4] = {1, (cuuint32_t)step, (cuuint32_t)step, 1};
+  return tmap_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, p, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_128B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, who, what);
+}
+
+int tmap_kmajor_bf16(CUtensorMap* m, const void* p, long long k, int rows, int box_rows, const char* who, const char* what) {
+  const cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)k * 2};
+  const cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
+  const cuuint32_t estr[2] = {1, 1};
+  return tmap_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, p, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_128B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, who, what);
 }
 
 }  // namespace hk

@@ -243,37 +243,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant_
 }
 
 // ---------------- host side ----------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 template <int BLOCK_N>
 static int launch_tc(const CUtensorMap& mx, const CUtensorMap& mw, const ConvTcArgs& a, cudaStream_t s) {
   using Cfg = TcCfg<BLOCK_N>;
-  static bool attr_set = false;  // per-process; the attribute is per function per device -- set every time if multi-device
-  int dev = 0;
-  cudaGetDevice(&dev);
-  static int attr_dev_mask = 0;
-  if (!attr_set || !(attr_dev_mask & (1 << dev))) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "conv(tcgen05): smem attribute (%d B): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e));
-    attr_set = true;
-    attr_dev_mask |= (1 << dev);
-  }
+  if (int rc = opt_in_smem<conv_tc_kernel<BLOCK_N>>(Cfg::SMEM_BYTES, "conv(tcgen05)")) return rc;
   const int total = a.num_m_tiles * a.num_n_tiles;
   int grid = sm_count();
   if (grid > total) grid = total;
@@ -303,8 +276,6 @@ int conv_tc_launch(const HkConvDesc& d, const void* x, const void* w, const floa
   HK_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(w) & 15) == 0 &&
                  (reinterpret_cast<uintptr_t>(y) & 15) == 0 && (reinterpret_cast<uintptr_t>(residual) & 15) == 0,
              "conv(tcgen05): buffers must be 16-byte aligned");
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "conv(tcgen05): cuTensorMapEncodeTiled entry point not available");
 
   // layer1 shape (3x3, 64 -> 64, stride 1): resident weights + haloed boxes, 3.6x less L2->SM traffic
   const bool specialised = d.algo != HK_CONV_TCGEN05_1CTA;
@@ -318,27 +289,10 @@ int conv_tc_launch(const HkConvDesc& d, const void* x, const void* w, const floa
   const int block_n = d.out_c % 256 == 0 ? 256 : (d.out_c % 128 == 0 ? 128 : 64);
   const int ktot = d.kh * d.kw * d.in_c;
 
+  const char* who = "conv(tcgen05)";
   CUtensorMap mx, mw;
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.in_c, (cuuint64_t)d.in_w, (cuuint64_t)d.in_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.in_c * 2, (cuuint64_t)d.in_w * d.in_c * 2, (cuuint64_t)d.in_h * d.in_w * d.in_c * 2};
-    const cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)(TC_BOX_W * d.stride), (cuuint32_t)(TC_BOX_H * d.stride), 1};
-    const cuuint32_t estr[4] = {1, (cuuint32_t)d.stride, (cuuint32_t)d.stride, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05): cuTensorMapEncodeTiled(activations) failed with CUresult %d", (int)r);
-  }
-  {
-    const cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)d.out_c};
-    const cuuint64_t strides[1] = {(cuuint64_t)ktot * 2};
-    const cuuint32_t box[2] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)block_n};
-    const cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05): cuTensorMapEncodeTiled(weights) failed with CUresult %d", (int)r);
-  }
+  if (int rc = tmap_nhwc_bf16(&mx, x, d.batch, d.in_h, d.in_w, d.in_c, TC_BOX_W, TC_BOX_H, d.stride, who, "activations")) return rc;
+  if (int rc = tmap_kmajor_bf16(&mw, w, ktot, d.out_c, block_n, who, "weights")) return rc;
 
   ConvTcArgs a;
   a.scale = scale; a.bias = bias;

@@ -556,11 +556,6 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 #ifdef HK_DIAG
 static long long* g_tc2_dbg = nullptr;
 extern "C" __attribute__((visibility("default"))) void hk_debug_set_tc2_timeline(long long* dev_buf) { g_tc2_dbg = dev_buf; }
@@ -579,14 +574,7 @@ static int launch_tc2(const CUtensorMap& mx, const CUtensorMap& mw, const CUtens
   using Cfg = Tc2Cfg<BLOCK_N>;
   const int smem_bytes = Cfg::SMEM_BYTES + (STATS ? epi_stats_smem_bytes(a.Cout) : 0) + (HEAD ? T2_HEAD_SMEM_BYTES : 0);
   if (smem_bytes > 227 * 1024) return fail(HK_ERR_BAD_ARG, "conv(tcgen05,2cta): %d bytes of shared memory needed", smem_bytes);
-  static int attr_smem[16] = {0};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 16 && attr_smem[dev] < smem_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc2_kernel<BLOCK_N, DS, STATS, HEAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): smem attribute (%d B): %s", smem_bytes, cudaGetErrorString(e));
-    attr_smem[dev] = smem_bytes;
-  }
+  if (int rc = opt_in_smem<conv_tc2_kernel<BLOCK_N, DS, STATS, HEAD>>(smem_bytes, "conv(tcgen05,2cta)")) return rc;
   const int total = a.num_m_tiles * a.num_n_tiles;
   int clusters = sm_count() / 2;
   if (clusters > total) clusters = total;
@@ -615,60 +603,24 @@ struct ConvTc2Ds {
 static int conv_tc2_launch_impl(const HkConvDesc& d, const void* x, const void* w, const float* scale, const float* bias,
                                 const void* residual, void* y, const ConvTc2Ds* ds, void* bn_acc, cudaStream_t s,
                                 const ConvTc2Head* head = nullptr) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled entry point not available");
   const long long boxes_all = (long long)ceil_div(d.out_w, T2_BOX_W) * ceil_div(d.out_h, T2_BOX_H) * d.batch;
   // HEAD: 256-column tiles always -- exactly two N tiles (Cout = 512) must add into every logit for the sum to be order-independent
   const int block_n = head ? 256 : pick_block_n_pair(d.out_c, (boxes_all + 3) / 4);
   const int ktot = d.kh * d.kw * d.in_c;
-  CUtensorMap mx, mw;
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.in_c, (cuuint64_t)d.in_w, (cuuint64_t)d.in_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.in_c * 2, (cuuint64_t)d.in_w * d.in_c * 2, (cuuint64_t)d.in_h * d.in_w * d.in_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)(T2_BOX_W * d.stride), (cuuint32_t)(T2_BOX_H * d.stride), 1};
-    const cuuint32_t estr[4] = {1, (cuuint32_t)d.stride, (cuuint32_t)d.stride, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled(activations) failed: %d", (int)r);
-  }
-  auto encode_w = [&](CUtensorMap* m, const void* wp, int k) -> CUresult {
-    const cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)d.out_c};
-    const cuuint64_t strides[1] = {(cuuint64_t)k * 2};
-    const cuuint32_t box[2] = {64, (cuuint32_t)(block_n / 2)};
-    const cuuint32_t estr[2] = {1, 1};
-    return encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(wp), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  };
-  {
-    CUresult r = encode_w(&mw, w, ktot);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled(weights) failed: %d", (int)r);
-  }
-  auto encode_out = [&](CUtensorMap* m, const void* p) -> CUresult {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.out_c, (cuuint64_t)d.out_w, (cuuint64_t)d.out_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.out_c * 2, (cuuint64_t)d.out_w * d.out_c * 2, (cuuint64_t)d.out_h * d.out_w * d.out_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)T2_BOX_W, (cuuint32_t)T2_BOX_H, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    return encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  };
-  CUtensorMap my, mres;
-  {
-    CUresult r = encode_out(&my, y ? y : residual);   // HEAD: nothing is stored; the map only has to be well-formed
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled(output) failed: %d", (int)r);
-    mres = my;
-    if (residual) {
-      r = encode_out(&mres, residual);
-      if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled(residual) failed: %d", (int)r);
-    }
+  const char* who = "conv(tcgen05,2cta)";
+  CUtensorMap mx, mw, my, mres;
+  if (int rc = tmap_nhwc_bf16(&mx, x, d.batch, d.in_h, d.in_w, d.in_c, T2_BOX_W, T2_BOX_H, d.stride, who, "activations")) return rc;
+  if (int rc = tmap_kmajor_bf16(&mw, w, ktot, d.out_c, block_n / 2, who, "weights")) return rc;
+  // HEAD: nothing is stored; the output map only has to be well-formed
+  if (int rc = tmap_nhwc_bf16(&my, y ? y : residual, d.batch, d.out_h, d.out_w, d.out_c, T2_BOX_W, T2_BOX_H, 1, who, "output")) return rc;
+  mres = my;
+  if (residual) {
+    if (int rc = tmap_nhwc_bf16(&mres, residual, d.batch, d.out_h, d.out_w, d.out_c, T2_BOX_W, T2_BOX_H, 1, who, "residual")) return rc;
   }
   CUtensorMap mw2 = mw, my2 = my;
   if (ds) {
-    CUresult r = encode_w(&mw2, ds->w, d.in_c);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled(downsample weights) failed: %d", (int)r);
-    r = encode_out(&my2, ds->y);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,2cta): cuTensorMapEncodeTiled(downsample output) failed: %d", (int)r);
+    if (int rc = tmap_kmajor_bf16(&mw2, ds->w, d.in_c, d.out_c, block_n / 2, who, "downsample weights")) return rc;
+    if (int rc = tmap_nhwc_bf16(&my2, ds->y, d.batch, d.out_h, d.out_w, d.out_c, T2_BOX_W, T2_BOX_H, 1, who, "downsample output")) return rc;
   }
   ConvTc2Args a;
   a.scale = scale; a.bias = bias;

@@ -315,11 +315,6 @@ conv_tc2h_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 // HK_CONV_HALO=0 disables the variant, =1 forces it for every eligible shape, unset: the default policy below.
 bool conv_tc2h_applicable(const HkConvDesc& d) {
   const char* env = getenv("HK_CONV_HALO");  // read per launch: tests and A/B runs toggle it
@@ -348,14 +343,7 @@ static int launch_tc2h(const CUtensorMap& mx, const CUtensorMap& mw, const CUten
   a.a_slots = na;
   a.b_slots = nb;
   const int smem = 1024 + na * a.a_slot_bytes + nb * B_BYTES + TH_STAGING_BYTES + 512 + stats_bytes;
-  static int attr_smem[16] = {0};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 16 && attr_smem[dev] < smem) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc2h_kernel<BLOCK_N, STATS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): smem attribute (%d B): %s", smem, cudaGetErrorString(e));
-    attr_smem[dev] = smem;
-  }
+  if (int rc = opt_in_smem<conv_tc2h_kernel<BLOCK_N, STATS>>(smem, "conv(tcgen05,halo)")) return rc;
   const int total = a.num_m_tiles * a.num_n_tiles;
   int clusters = sm_count() / 2;
   if (clusters > total) clusters = total;
@@ -367,8 +355,6 @@ static int launch_tc2h(const CUtensorMap& mx, const CUtensorMap& mw, const CUten
 
 int conv_tc2h_launch(const HkConvDesc& d, const void* x, const void* w, const float* scale, const float* bias, const void* residual,
                      void* y, void* bn_acc, cudaStream_t s) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled entry point not available");
   // patch geometry: 8x16 patches over the rows that fill whole patch rows, 4x32 strips over a remainder of 1..4 rows (see the header)
   const char* strips_env = getenv("HK_CONV_STRIPS");
   const int rem_rows = d.out_h % TH_TILE_H;
@@ -385,67 +371,23 @@ int conv_tc2h_launch(const HkConvDesc& d, const void* x, const void* w, const fl
   const int ktot = 9 * d.in_c;
   const int box_rows = TH_TILE_H + 2 * d.dil;
   const int strip_box_rows = TH_TILE_H / 2 + 2 * d.dil;
+  const char* who = "conv(tcgen05,halo)";
   CUtensorMap mx, mw, my, mres;
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.in_c, (cuuint64_t)d.in_w, (cuuint64_t)d.in_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.in_c * 2, (cuuint64_t)d.in_w * d.in_c * 2, (cuuint64_t)d.in_h * d.in_w * d.in_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)TH_TILE_W, (cuuint32_t)box_rows, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(activations) failed: %d", (int)r);
-  }
-  {
-    const cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)d.out_c};
-    const cuuint64_t strides[1] = {(cuuint64_t)ktot * 2};
-    const cuuint32_t box[2] = {64, (cuuint32_t)(block_n / 2)};
-    const cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(weights) failed: %d", (int)r);
-  }
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.out_c, (cuuint64_t)d.out_w, (cuuint64_t)d.out_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.out_c * 2, (cuuint64_t)d.out_w * d.out_c * 2, (cuuint64_t)d.out_h * d.out_w * d.out_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)TH_TILE_W, (cuuint32_t)TH_TILE_H, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&my, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(output) failed: %d", (int)r);
-    mres = my;
-    if (residual) {
-      r = encode(&mres, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(residual), dims, strides, box, estr,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(residual) failed: %d", (int)r);
-    }
+  if (int rc = tmap_nhwc_bf16(&mx, x, d.batch, d.in_h, d.in_w, d.in_c, TH_TILE_W, box_rows, 1, who, "activations")) return rc;
+  if (int rc = tmap_kmajor_bf16(&mw, w, ktot, d.out_c, block_n / 2, who, "weights")) return rc;
+  if (int rc = tmap_nhwc_bf16(&my, y, d.batch, d.out_h, d.out_w, d.out_c, TH_TILE_W, TH_TILE_H, 1, who, "output")) return rc;
+  mres = my;
+  if (residual) {
+    if (int rc = tmap_nhwc_bf16(&mres, residual, d.batch, d.out_h, d.out_w, d.out_c, TH_TILE_W, TH_TILE_H, 1, who, "residual")) return rc;
   }
   CUtensorMap mxs = mx, mys = my, mress = mres;   // 4x32 strip flavours of the activation / output / residual maps
   if (use_strips) {
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    {
-      const cuuint64_t dims[4] = {(cuuint64_t)d.in_c, (cuuint64_t)d.in_w, (cuuint64_t)d.in_h, (cuuint64_t)d.batch};
-      const cuuint64_t strides[3] = {(cuuint64_t)d.in_c * 2, (cuuint64_t)d.in_w * d.in_c * 2, (cuuint64_t)d.in_h * d.in_w * d.in_c * 2};
-      const cuuint32_t box[4] = {64, (cuuint32_t)(2 * TH_TILE_W), (cuuint32_t)strip_box_rows, 1};
-      CUresult r = encode(&mxs, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(strip activations) failed: %d", (int)r);
-    }
-    const cuuint64_t dims[4] = {(cuuint64_t)d.out_c, (cuuint64_t)d.out_w, (cuuint64_t)d.out_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.out_c * 2, (cuuint64_t)d.out_w * d.out_c * 2, (cuuint64_t)d.out_h * d.out_w * d.out_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)(2 * TH_TILE_W), (cuuint32_t)(TH_TILE_H / 2), 1};
-    CUresult r = encode(&mys, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(strip output) failed: %d", (int)r);
+    const int strip_w = 2 * TH_TILE_W, strip_h = TH_TILE_H / 2;
+    if (int rc = tmap_nhwc_bf16(&mxs, x, d.batch, d.in_h, d.in_w, d.in_c, strip_w, strip_box_rows, 1, who, "strip activations")) return rc;
+    if (int rc = tmap_nhwc_bf16(&mys, y, d.batch, d.out_h, d.out_w, d.out_c, strip_w, strip_h, 1, who, "strip output")) return rc;
     mress = mys;
     if (residual) {
-      r = encode(&mress, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(residual), dims, strides, box, estr,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,halo): cuTensorMapEncodeTiled(strip residual) failed: %d", (int)r);
+      if (int rc = tmap_nhwc_bf16(&mress, residual, d.batch, d.out_h, d.out_w, d.out_c, strip_w, strip_h, 1, who, "strip residual")) return rc;
     }
   }
   ConvTc2hArgs a;

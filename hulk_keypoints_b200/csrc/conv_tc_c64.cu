@@ -290,11 +290,6 @@ conv_tc_c64_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 #ifdef HK_DIAG
 static long long* g_c64_dbg = nullptr;
 extern "C" __attribute__((visibility("default"))) void hk_debug_set_c64_timeline(long long* dev_buf) { g_c64_dbg = dev_buf; }
@@ -311,46 +306,15 @@ bool conv_tc_c64_applicable(const HkConvDesc& d) {
 
 int conv_tc_c64_launch(const HkConvDesc& d, const void* x, const void* w, const float* scale, const float* bias,
                        const void* residual, void* y, void* bn_acc, cudaStream_t s) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "conv(tcgen05,c64): cuTensorMapEncodeTiled entry point not available");
   const int box_rows = C64_TILE_H + 2 * d.dil;
-  CUtensorMap mx, mw;
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.in_c, (cuuint64_t)d.in_w, (cuuint64_t)d.in_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.in_c * 2, (cuuint64_t)d.in_w * d.in_c * 2, (cuuint64_t)d.in_h * d.in_w * d.in_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)C64_TILE_W, (cuuint32_t)box_rows, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,c64): cuTensorMapEncodeTiled(activations) failed: %d", (int)r);
-  }
-  {
-    const cuuint64_t dims[2] = {(cuuint64_t)(9 * 64), 64};
-    const cuuint64_t strides[1] = {(cuuint64_t)(9 * 64) * 2};
-    const cuuint32_t box[2] = {64, 64};
-    const cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,c64): cuTensorMapEncodeTiled(weights) failed: %d", (int)r);
-  }
-  CUtensorMap my, mres;
-  {
-    const cuuint64_t dims[4] = {64, (cuuint64_t)d.out_w, (cuuint64_t)d.out_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {128, (cuuint64_t)d.out_w * 128, (cuuint64_t)d.out_h * d.out_w * 128};
-    const cuuint32_t box[4] = {64, (cuuint32_t)C64_TILE_W, (cuuint32_t)C64_TILE_H, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&my, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,c64): cuTensorMapEncodeTiled(output) failed: %d", (int)r);
-    mres = my;
-    if (residual) {
-      r = encode(&mres, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(residual), dims, strides, box, estr,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "conv(tcgen05,c64): cuTensorMapEncodeTiled(residual) failed: %d", (int)r);
-    }
+  const char* who = "conv(tcgen05,c64)";
+  CUtensorMap mx, mw, my, mres;
+  if (int rc = tmap_nhwc_bf16(&mx, x, d.batch, d.in_h, d.in_w, d.in_c, C64_TILE_W, box_rows, 1, who, "activations")) return rc;
+  if (int rc = tmap_kmajor_bf16(&mw, w, 9 * 64, 64, 64, who, "weights")) return rc;
+  if (int rc = tmap_nhwc_bf16(&my, y, d.batch, d.out_h, d.out_w, 64, C64_TILE_W, C64_TILE_H, 1, who, "output")) return rc;
+  mres = my;
+  if (residual) {
+    if (int rc = tmap_nhwc_bf16(&mres, residual, d.batch, d.out_h, d.out_w, 64, C64_TILE_W, C64_TILE_H, 1, who, "residual")) return rc;
   }
   ConvC64Args a;
   a.has_residual = residual ? 1 : 0;
@@ -375,16 +339,7 @@ int conv_tc_c64_launch(const HkConvDesc& d, const void* x, const void* w, const 
   if (slots > C64_MAX_SLOTS) slots = C64_MAX_SLOTS;
   a.slots = slots;
   const int smem = fixed + slots * a.patch_bytes;
-  static int attr_smem[2][16] = {{0}, {0}};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const int which = bn_acc ? 1 : 0;
-  if (dev < 16 && attr_smem[which][dev] < smem) {
-    cudaError_t e = bn_acc ? cudaFuncSetAttribute(conv_tc_c64_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)
-                           : cudaFuncSetAttribute(conv_tc_c64_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "conv(tcgen05,c64): smem attribute (%d B): %s", smem, cudaGetErrorString(e));
-    attr_smem[which][dev] = smem;
-  }
+  if (int rc = bn_acc ? opt_in_smem<conv_tc_c64_kernel<true>>(smem, who) : opt_in_smem<conv_tc_c64_kernel<false>>(smem, who)) return rc;
   int grid = sm_count();
   if (grid > a.num_tiles) grid = a.num_tiles;
   cudaError_t le = bn_acc ? launch_pdl(conv_tc_c64_kernel<true>, dim3(grid), dim3(C64_THREADS), (size_t)smem, s, mx, mw, my, mres, a)

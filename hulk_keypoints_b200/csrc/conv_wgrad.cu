@@ -259,10 +259,6 @@ __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restri
     for (int j = 0; j < 4; ++j) dst[(size_t)j * taps] = (accumulate ? dst[(size_t)j * taps] : 0.f) + sv[j];
   }
 }
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
 
 struct WgradPlan {
   int block_n, m_tiles, n_tiles, taps, ksplit, boxes_per_split, num_boxes, tiles_x, tiles_per_img, tap_pairs, tap_units;
@@ -298,14 +294,7 @@ static WgradPlan wgrad_plan(const HkConvDesc& d) {
 template <int BLOCK_N>
 static int launch_wgrad(const CUtensorMap& mdy, const CUtensorMap& mx, const WgradArgs& a, cudaStream_t s) {
   using Cfg = WgCfg<BLOCK_N>;
-  static int attr_dev_mask = 0;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!(attr_dev_mask & (1 << dev))) {
-    cudaError_t e = cudaFuncSetAttribute(conv_wgrad_kernel<BLOCK_N>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "conv wgrad: smem attribute (%d B): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e));
-    attr_dev_mask |= (1 << dev);
-  }
+  if (int rc = opt_in_smem<conv_wgrad_kernel<BLOCK_N>>(Cfg::SMEM_BYTES, "conv wgrad")) return rc;
   const int total = a.ksplit * a.tap_units * a.m_tiles * a.n_tiles;
   int grid = sm_count();
   if (grid > total) grid = total;
@@ -337,29 +326,9 @@ int hk_conv_wgrad(const HkConvDesc* desc, const void* x, const void* dy, float* 
              "hk_conv_wgrad: buffers must be 16-byte aligned");
   const WgradPlan p = wgrad_plan(d);
   HK_REQUIRE(ws_bytes >= hk_conv_wgrad_workspace_bytes(desc), "hk_conv_wgrad: workspace too small");
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "hk_conv_wgrad: cuTensorMapEncodeTiled entry point not available");
   CUtensorMap mdy, mx;
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.out_c, (cuuint64_t)d.out_w, (cuuint64_t)d.out_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.out_c * 2, (cuuint64_t)d.out_w * d.out_c * 2, (cuuint64_t)d.out_h * d.out_w * d.out_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)WG_BOX_W, (cuuint32_t)WG_BOX_H, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&mdy, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(dy), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_conv_wgrad: cuTensorMapEncodeTiled(dy) failed: %d", (int)r);
-  }
-  {
-    const cuuint64_t dims[4] = {(cuuint64_t)d.in_c, (cuuint64_t)d.in_w, (cuuint64_t)d.in_h, (cuuint64_t)d.batch};
-    const cuuint64_t strides[3] = {(cuuint64_t)d.in_c * 2, (cuuint64_t)d.in_w * d.in_c * 2, (cuuint64_t)d.in_h * d.in_w * d.in_c * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)(WG_BOX_W * d.stride), (cuuint32_t)(WG_BOX_H * d.stride), 1};
-    const cuuint32_t estr[4] = {1, (cuuint32_t)d.stride, (cuuint32_t)d.stride, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_conv_wgrad: cuTensorMapEncodeTiled(x) failed: %d", (int)r);
-  }
+  if (int rc = tmap_nhwc_bf16(&mdy, dy, d.batch, d.out_h, d.out_w, d.out_c, WG_BOX_W, WG_BOX_H, 1, "hk_conv_wgrad", "dy")) return rc;
+  if (int rc = tmap_nhwc_bf16(&mx, x, d.batch, d.in_h, d.in_w, d.in_c, WG_BOX_W, WG_BOX_H, d.stride, "hk_conv_wgrad", "x")) return rc;
   WgradArgs a;
   a.ws = static_cast<float*>(ws);
   a.B = d.batch; a.Ho = d.out_h; a.Wo = d.out_w; a.Cout = d.out_c; a.Cin = d.in_c;

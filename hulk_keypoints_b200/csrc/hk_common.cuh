@@ -1,5 +1,6 @@
 // Shared host/device helpers for libhulk_sm100.so.
 #pragma once
+#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -23,6 +24,33 @@ inline long long ceil_div_ll(long long a, long long b) { return (a + b - 1) / b;
 
 // Number of SMs of the current device (cached).
 int sm_count();
+
+// TMA tensor maps.  Each returns HK_OK, or records "<who>: cuTensorMapEncodeTiled(<what>) failed: <CUresult>" and returns HK_ERR_CUDA.
+// bf16 NHWC (n, h, w, c): 64-channel x box_w x box_h boxes, SWIZZLE_128B, L2 promotion 128 B.  step > 1: the box spans step*box_w x
+// step*box_h pixels and TMA keeps every step-th (the activation operand of a strided conv).
+int tmap_nhwc_bf16(CUtensorMap* m, const void* p, int n, int h, int w, int c, int box_w, int box_h, int step, const char* who,
+                   const char* what);
+// bf16 K-major (rows, k), row pitch 2k bytes: 64 x box_rows boxes, SWIZZLE_128B, L2 promotion 256 B.
+int tmap_kmajor_bf16(CUtensorMap* m, const void* p, long long k, int rows, int box_rows, const char* who, const char* what);
+// Any other map: the raw cuTensorMapEncodeTiled arrays (no interleave; out-of-bounds elements read as zero).
+int tmap_encode(CUtensorMap* m, CUtensorMapDataType dtype, int rank, const void* p, const cuuint64_t* dims, const cuuint64_t* strides,
+                const cuuint32_t* box, const cuuint32_t* estr, CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* who,
+                const char* what);
+
+// Allow Kernel `bytes` of dynamic shared memory on the current device (the attribute is per function and per device).  Sets the
+// attribute only when `bytes` exceeds the largest size already set there.
+template <auto Kernel>
+int opt_in_smem(int bytes, const char* who) {
+  static int set_bytes[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  const bool tracked = dev >= 0 && dev < 64;  // beyond the table: set it every time
+  if (tracked && set_bytes[dev] >= bytes) return HK_OK;
+  const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e != cudaSuccess) return fail(HK_ERR_CUDA, "%s: smem attribute (%d B): %s", who, bytes, cudaGetErrorString(e));
+  if (tracked) set_bytes[dev] = bytes;
+  return HK_OK;
+}
 
 // N tile of the CTA-pair conv kernels.  256 columns amortise the activation tile best, but with few tiles the last wave of the
 // persistent grid is mostly idle (batch 4 of 60x80 maps: 75 tiles on 74 CTA pairs = 2 waves for 1.01 waves of work); 128-column tiles

@@ -175,12 +175,7 @@ extern "C" int hk_pack_conv_weights_many_tiled(const HkPackItem* items_dev, int 
   using namespace hk;
   HK_REQUIRE(items_dev && n_items > 0 && max_khw > 0 && max_khw <= 25 && max_elems > 0, "hk_pack_conv_weights_many_tiled: bad argument");
   const int smem = PK_CO * ((PK_CI * max_khw) | 1) * (int)sizeof(float);
-  static int attr_done = 0;
-  if (attr_done < smem) {
-    cudaError_t e = cudaFuncSetAttribute(pack_weights_many_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "hk_pack_conv_weights_many_tiled: smem attribute (%d B): %s", smem, cudaGetErrorString(e));
-    attr_done = smem;
-  }
+  if (int rc = opt_in_smem<pack_weights_many_tiled_kernel>(smem, "hk_pack_conv_weights_many_tiled")) return rc;
   long long bx = ceil_div_ll(max_elems, (long long)PK_CO * PK_CI * max_khw);   // tiles of the largest item
   if (bx > 64) bx = 64;
   if (bx < 1) bx = 1;

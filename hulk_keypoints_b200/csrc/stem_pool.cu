@@ -413,11 +413,6 @@ stem_pool_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 static int stem_pool_launch(const void* x, bool u8, const void* w_packed, const float* scale, const float* bias, void* y, int B, int H,
                             int W, void* stream) {
   HK_REQUIRE(x && w_packed && scale && bias && y, "hk_stem_pool_fwd: null pointer");
@@ -426,35 +421,25 @@ static int stem_pool_launch(const void* x, bool u8, const void* w_packed, const 
                  (reinterpret_cast<uintptr_t>(x) & 15) == 0, "hk_stem_pool_fwd: buffers must be 16-byte aligned");
   // TMA row pitch must be a multiple of 16 bytes
   HK_REQUIRE(u8 ? (3 * W) % 16 == 0 : W % 4 == 0, "hk_stem_pool_fwd: W must be a multiple of %d for the TMA input path", u8 ? 16 : 4);
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "hk_stem_pool_fwd: cuTensorMapEncodeTiled entry point not available");
+  const char* who = "hk_stem_pool_fwd";
   CUtensorMap mw, mx;
-  {
-    const cuuint64_t dims[2] = {256, 64};
-    const cuuint64_t strides[1] = {512};
-    const cuuint32_t box[2] = {64, 64};
-    const cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w_packed), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_stem_pool_fwd: cuTensorMapEncodeTiled(weights) failed: %d", (int)r);
-  }
+  if (int rc = tmap_kmajor_bf16(&mw, w_packed, 256, 64, 64, who, "weights")) return rc;
   if (u8) {
     const cuuint64_t dims[3] = {(cuuint64_t)3 * W, (cuuint64_t)H, (cuuint64_t)B};
     const cuuint64_t strides[2] = {(cuuint64_t)3 * W, (cuuint64_t)3 * W * H};
     const cuuint32_t box[3] = {(cuuint32_t)SP_U8_BOX, 2, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_stem_pool_fwd: cuTensorMapEncodeTiled(uint8 input) failed: %d", (int)r);
+    if (int rc = tmap_encode(&mx, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, x, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_NONE,
+                             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, who, "uint8 input"))
+      return rc;
   } else {
     const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
     const cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4, (cuuint64_t)W * H * 12};
     const cuuint32_t box[4] = {(cuuint32_t)SP_F32_BOX, 2, 3, 1};
     const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&mx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void*>(x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_stem_pool_fwd: cuTensorMapEncodeTiled(fp32 input) failed: %d", (int)r);
+    if (int rc = tmap_encode(&mx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, x, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_NONE,
+                             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, who, "fp32 input"))
+      return rc;
   }
   StemPoolArgs a;
   a.scale = scale; a.bias = bias; a.y = static_cast<__nv_bfloat16*>(y);
@@ -476,15 +461,7 @@ static int stem_pool_launch(const void* x, bool u8, const void* w_packed, const 
 #ifdef HK_DIAG
   { const char* m = getenv("HK_SP_DEBUG"); a.dbg_mode = m ? atoi(m) : 0; }
 #endif
-  static int attr_dev_mask[2] = {0, 0};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!(attr_dev_mask[u8] & (1 << dev))) {
-    cudaError_t e = u8 ? cudaFuncSetAttribute(stem_pool_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SP_SMEM_BYTES)
-                       : cudaFuncSetAttribute(stem_pool_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SP_SMEM_BYTES);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "hk_stem_pool_fwd: smem attribute: %s", cudaGetErrorString(e));
-    attr_dev_mask[u8] |= (1 << dev);
-  }
+  if (int rc = u8 ? opt_in_smem<stem_pool_kernel<true>>(SP_SMEM_BYTES, who) : opt_in_smem<stem_pool_kernel<false>>(SP_SMEM_BYTES, who)) return rc;
   int grid = sms;
   if (grid > a.num_units) grid = a.num_units;
   if (u8) stem_pool_kernel<true><<<grid, SP_THREADS, SP_SMEM_BYTES, as_stream(stream)>>>(mx, mw, a);

@@ -513,11 +513,6 @@ __global__ void __launch_bounds__(256) stem_wgrad_tc_finalize_kernel(const float
   dw[j] = (accumulate ? dw[j] : 0.f) + (float)((s0 + s1) + (s2 + s3));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 // OIHW (64,3,7,7) fp32 -> (64, 256) bf16 with k = r*32 + s*4 + c, zeros elsewhere
 __global__ void stem_pack_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -556,30 +551,11 @@ static int stem_launch(const void* x, bool u8, const void* w_packed, const float
   HK_REQUIRE(B > 0 && H >= 7 && W >= 7, "hk_stem_fwd: bad shape");
   HK_REQUIRE((reinterpret_cast<uintptr_t>(w_packed) & 15) == 0 && (reinterpret_cast<uintptr_t>(y_nhwc) & 15) == 0,
              "hk_stem_fwd: buffers must be 16-byte aligned");
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "hk_stem_fwd: cuTensorMapEncodeTiled entry point not available");
-  CUtensorMap mw;
-  {
-    const cuuint64_t dims[2] = {(cuuint64_t)ST_K, (cuuint64_t)ST_COUT};
-    const cuuint64_t strides[1] = {(cuuint64_t)ST_K * 2};
-    const cuuint32_t box[2] = {64, (cuuint32_t)ST_COUT};
-    const cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w_packed), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_stem_fwd: cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-  }
-  CUtensorMap my;
-  {
-    const int Ho = (H + 6 - 7) / 2 + 1, Wo = (W + 6 - 7) / 2 + 1;
-    const cuuint64_t dims[4] = {64, (cuuint64_t)Wo, (cuuint64_t)Ho, (cuuint64_t)B};
-    const cuuint64_t strides[3] = {128, (cuuint64_t)Wo * 128, (cuuint64_t)Ho * Wo * 128};
-    const cuuint32_t box[4] = {64, (cuuint32_t)ST_TILE_W, (cuuint32_t)ST_TILE_H, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&my, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y_nhwc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_stem_fwd: cuTensorMapEncodeTiled(output) failed with CUresult %d", (int)r);
-  }
+  const int Ho = (H + 6 - 7) / 2 + 1, Wo = (W + 6 - 7) / 2 + 1;
+  const char* who = "hk_stem_fwd";
+  CUtensorMap mw, my;
+  if (int rc = tmap_kmajor_bf16(&mw, w_packed, ST_K, ST_COUT, ST_COUT, who, "weights")) return rc;
+  if (int rc = tmap_nhwc_bf16(&my, y_nhwc, B, Ho, Wo, 64, ST_TILE_W, ST_TILE_H, 1, who, "output")) return rc;
   StemTcArgs a;
   a.x = x; a.scale = scale; a.bias = bias; a.y = static_cast<__nv_bfloat16*>(y_nhwc);
   a.B = B; a.H = H; a.W = W;
@@ -587,22 +563,14 @@ static int stem_launch(const void* x, bool u8, const void* w_packed, const float
   a.dbg = g_stem_dbg;
 #endif
   a.relu = relu;
-  a.Ho = (H + 6 - 7) / 2 + 1;
-  a.Wo = (W + 6 - 7) / 2 + 1;
+  a.Ho = Ho;
+  a.Wo = Wo;
   a.tiles_x = ceil_div(a.Wo, ST_TILE_W);
   a.tiles_per_img = a.tiles_x * ceil_div(a.Ho, ST_TILE_H);
   const long long nt = (long long)a.tiles_per_img * B;
   HK_REQUIRE(nt < 0x7fffffffLL, "hk_stem_fwd: too many tiles");
   a.num_tiles = (int)nt;
-  static int attr_dev_mask[2] = {0, 0};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!(attr_dev_mask[u8] & (1 << dev))) {
-    cudaError_t e = u8 ? cudaFuncSetAttribute(stem_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM_BYTES)
-                       : cudaFuncSetAttribute(stem_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM_BYTES);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "hk_stem_fwd: smem attribute: %s", cudaGetErrorString(e));
-    attr_dev_mask[u8] |= (1 << dev);
-  }
+  if (int rc = u8 ? opt_in_smem<stem_tc_kernel<true>>(ST_SMEM_BYTES, who) : opt_in_smem<stem_tc_kernel<false>>(ST_SMEM_BYTES, who)) return rc;
   int grid = 2 * sm_count();
   if (grid > a.num_tiles) grid = a.num_tiles;
   if (u8) stem_tc_kernel<true><<<grid, ST_THREADS, ST_SMEM_BYTES, as_stream(stream)>>>(mw, my, a);
@@ -635,20 +603,9 @@ int hk_stem_wgrad(const float* x_nchw, const void* dy_nhwc, float* dw_oihw, int 
   HK_REQUIRE(ws_bytes >= hk_stem_wgrad_workspace_bytes(), "hk_stem_wgrad: workspace too small");
   HK_REQUIRE((reinterpret_cast<uintptr_t>(dy_nhwc) & 15) == 0 && (reinterpret_cast<uintptr_t>(ws) & 15) == 0,
              "hk_stem_wgrad: buffers must be 16-byte aligned");
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return fail(HK_ERR_CUDA, "hk_stem_wgrad: cuTensorMapEncodeTiled entry point not available");
   const int Ho = (H + 6 - 7) / 2 + 1, Wo = (W + 6 - 7) / 2 + 1;
   CUtensorMap mdy;
-  {
-    const cuuint64_t dims[4] = {64, (cuuint64_t)Wo, (cuuint64_t)Ho, (cuuint64_t)B};
-    const cuuint64_t strides[3] = {128, (cuuint64_t)Wo * 128, (cuuint64_t)Ho * Wo * 128};
-    const cuuint32_t box[4] = {64, (cuuint32_t)ST_TILE_W, (cuuint32_t)ST_TILE_H, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&mdy, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(dy_nhwc), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(HK_ERR_CUDA, "hk_stem_wgrad: cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-  }
+  if (int rc = tmap_nhwc_bf16(&mdy, dy_nhwc, B, Ho, Wo, 64, ST_TILE_W, ST_TILE_H, 1, "hk_stem_wgrad", "dy")) return rc;
   StemWgradArgs a;
   a.x = x_nchw; a.partial = static_cast<float*>(ws);
   a.B = B; a.H = H; a.W = W; a.Ho = Ho; a.Wo = Wo;
@@ -657,14 +614,7 @@ int hk_stem_wgrad(const float* x_nchw, const void* dy_nhwc, float* dw_oihw, int 
   const long long nt = (long long)a.tiles_per_img * B;
   HK_REQUIRE(nt < 0x7fffffffLL, "hk_stem_wgrad: too many tiles");
   a.num_tiles = (int)nt;
-  static int attr_dev_mask = 0;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!(attr_dev_mask & (1 << dev))) {
-    cudaError_t e = cudaFuncSetAttribute(stem_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SWG_SMEM_BYTES);
-    if (e != cudaSuccess) return fail(HK_ERR_CUDA, "hk_stem_wgrad: smem attribute: %s", cudaGetErrorString(e));
-    attr_dev_mask |= (1 << dev);
-  }
+  if (int rc = opt_in_smem<stem_wgrad_tc_kernel>(SWG_SMEM_BYTES, "hk_stem_wgrad")) return rc;
   int grid = 2 * sm_count();
   if (grid > a.num_tiles) grid = a.num_tiles;
   stem_wgrad_tc_kernel<<<grid, ST_THREADS, SWG_SMEM_BYTES, as_stream(stream)>>>(mdy, a);

@@ -354,30 +354,44 @@ def test_conv_epilogue_statistics_match_standalone_reduction(case):
 def test_pack_weights_many_tiled_equals_elementwise():
     """hk_pack_conv_weights_many_tiled (shared-memory tiles) against hk_pack_conv_weights_many (element-wise gather) and against the
     single-conv packers: identical bf16 bytes in the forward (cout,kh,kw,cin) and the data-gradient (cin,kh,kw flipped,cout) layouts."""
-    import ctypes as C
-    import numpy as np
-    from hulk_keypoints_b200._lib import lib, ptr, check, stream_ptr
-    shapes = [(64, 64, 3), (128, 64, 3), (128, 64, 1), (256, 128, 3), (512, 256, 1), (512, 512, 3)]
-    g = torch.Generator().manual_seed(9)
-    ws = [torch.randn(co, ci, k, k, generator=g).to(DEV) for co, ci, k in shapes]
-    outs = {}
-    for tiled in (False, True):
-        f = [torch.zeros(co, k, k, ci, device=DEV, dtype=torch.bfloat16) for co, ci, k in shapes]
-        d = [torch.zeros(ci, k, k, co, device=DEV, dtype=torch.bfloat16) for co, ci, k in shapes]
-        dt = np.dtype([("w", "<u8"), ("f", "<u8"), ("d", "<u8"), ("cout", "<i4"), ("cin", "<i4"), ("khw", "<i4"), ("r", "<i4")])
-        arr = np.zeros(len(shapes), dtype=dt)
+    _check_pack_weights_many_tiled(DEV)
+
+
+def test_pack_weights_many_tiled_on_a_second_device():
+    """The same on cuda:0 and then on cuda:1 in one process: the shared-memory opt-in of the tiled packer is per device, so its first
+    launch on the second device must set it again."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two visible CUDA devices")
+    for dev in ("cuda:0", "cuda:1"):
+        _check_pack_weights_many_tiled(dev)
+
+
+def _check_pack_weights_many_tiled(dev):
+    with torch.cuda.device(dev):   # tensors, current stream and launch all on `dev`
+        import ctypes as C
+        import numpy as np
+        from hulk_keypoints_b200._lib import lib, ptr, check, stream_ptr
+        shapes = [(64, 64, 3), (128, 64, 3), (128, 64, 1), (256, 128, 3), (512, 256, 1), (512, 512, 3)]
+        g = torch.Generator().manual_seed(9)
+        ws = [torch.randn(co, ci, k, k, generator=g).to(dev) for co, ci, k in shapes]
+        outs = {}
+        for tiled in (False, True):
+            f = [torch.zeros(co, k, k, ci, device=dev, dtype=torch.bfloat16) for co, ci, k in shapes]
+            d = [torch.zeros(ci, k, k, co, device=dev, dtype=torch.bfloat16) for co, ci, k in shapes]
+            dt = np.dtype([("w", "<u8"), ("f", "<u8"), ("d", "<u8"), ("cout", "<i4"), ("cin", "<i4"), ("khw", "<i4"), ("r", "<i4")])
+            arr = np.zeros(len(shapes), dtype=dt)
+            for i, (co, ci, k) in enumerate(shapes):
+                arr[i] = (ws[i].data_ptr(), f[i].data_ptr(), d[i].data_ptr(), co, ci, k * k, 0)
+            items = torch.from_numpy(arr.view(np.uint8).copy()).to(dev)
+            mx = max(co * ci * k * k for co, ci, k in shapes)
+            if tiled:
+                check(lib().hk_pack_conv_weights_many_tiled(ptr(items), len(shapes), 9, C.c_longlong(mx), stream_ptr()), "tiled")
+            else:
+                check(lib().hk_pack_conv_weights_many(ptr(items), len(shapes), C.c_longlong(mx), stream_ptr()), "elementwise")
+            torch.cuda.synchronize()
+            outs[tiled] = (f, d)
         for i, (co, ci, k) in enumerate(shapes):
-            arr[i] = (ws[i].data_ptr(), f[i].data_ptr(), d[i].data_ptr(), co, ci, k * k, 0)
-        items = torch.from_numpy(arr.view(np.uint8).copy()).to(DEV)
-        mx = max(co * ci * k * k for co, ci, k in shapes)
-        if tiled:
-            check(lib().hk_pack_conv_weights_many_tiled(ptr(items), len(shapes), 9, C.c_longlong(mx), stream_ptr()), "tiled")
-        else:
-            check(lib().hk_pack_conv_weights_many(ptr(items), len(shapes), C.c_longlong(mx), stream_ptr()), "elementwise")
-        torch.cuda.synchronize()
-        outs[tiled] = (f, d)
-    for i, (co, ci, k) in enumerate(shapes):
-        assert torch.equal(outs[True][0][i], outs[False][0][i]) and torch.equal(outs[True][1][i], outs[False][1][i]), shapes[i]
-        wp, _, _ = ops.pack_conv_weights(ws[i], None, 1e-5, torch.bfloat16)
-        assert torch.equal(outs[True][0][i], wp)
-        assert torch.equal(outs[True][1][i], ops.pack_conv_weights_dgrad(ws[i]))
+            assert torch.equal(outs[True][0][i], outs[False][0][i]) and torch.equal(outs[True][1][i], outs[False][1][i]), shapes[i]
+            wp, _, _ = ops.pack_conv_weights(ws[i], None, 1e-5, torch.bfloat16)
+            assert torch.equal(outs[True][0][i], wp)
+            assert torch.equal(outs[True][1][i], ops.pack_conv_weights_dgrad(ws[i]))

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench_train.py -- BASELINE.json configs[3]: one KeypointsGauss training step per iteration.
 
-    python bench_train.py [--steps K] [--warmup W] [--batch 4]
+    python bench_train.py [--steps K] [--warmup W] [--batch 4] [--freeze {none,bn,torchvision,head}]
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench_train.py --gpus N
 
 step = Gaussian targets from (B,K,2) labels (generated on the fly inside the fused loss kernel) + forward (train-mode
@@ -9,7 +9,9 @@ BN, per-replica statistics) + fused sigmoid/BCE forward+backward (hk_bce_fwd_bwd
 all-reduce (NCCL, bucketed) + Adam(lr 1e-4, wd 1e-4) -- the sequence of reference train.py:33-36.
 --backend hk (default): the whole step runs on libhulk_sm100 kernels (TrainEngine: tcgen05 forward / dgrad / wgrad, train-mode
 BN kernels, fused loss, FusedAdam; one CUDA graph).  --backend autograd: the backbone runs on torch autograd / cuDNN fp32 (the
-same-box competitor).  Secondary benchmark: the headline metric is bench.py (inference images/s).
+same-box competitor).  --freeze: fine-tuning presets (train_ops.freeze_preset): "bn" every BatchNorm in eval() mode with
+gamma / beta trained, "torchvision" every BatchNorm frozen with gamma / beta plus conv1 + layer1 frozen, "head" only fc trained.
+Secondary benchmark: the headline metric is bench.py (inference images/s).
 """
 from __future__ import annotations
 
@@ -40,6 +42,8 @@ def main():
     ap.add_argument("--backend", default="hk", choices=["hk", "autograd"],
                     help="hk: whole step on libhulk_sm100 kernels (TrainEngine, bf16 tcgen05, one CUDA graph); "
                          "autograd: backbone on torch autograd / cuDNN fp32 (the same-box competitor and the parity checker)")
+    ap.add_argument("--freeze", default="none", choices=["none", "bn", "torchvision", "head"],
+                    help="fine-tuning preset: frozen BatchNorms (eval() mode) and frozen parameters (requires_grad=False)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -54,6 +58,8 @@ def main():
     torch.manual_seed(0)
     model = hk.KeypointsGauss(4, img_height=args.height, img_width=args.width).to(dev).train()
     parallel.broadcast_model(model)
+    if args.freeze != "none":
+        train_ops.freeze_preset(model, args.freeze)   # before the optimiser is built, as in torch
     if args.optimizer == "fused" and not args.reference_loss:
         from hulk_keypoints_b200.optim import FusedAdam
         opt = FusedAdam(model.parameters(), lr=1e-4, weight_decay=1e-4)
@@ -105,7 +111,7 @@ def main():
             "data": "synthetic", "loss": float(loss.item()),
             "config": {"workload": f"train step, per-GPU batch {B}, {H}x{W}, K=4, Adam lr 1e-4 wd 1e-4 (BASELINE.json configs[3])",
                        "loss_path": "torch BCELoss on fp64 targets" if args.reference_loss else "fused hk_bce_fwd_bwd, targets on the fly",
-                       "optimizer": type(opt).__name__,
+                       "optimizer": type(opt).__name__, "freeze": args.freeze,
                        "parallelism": f"data-parallel x{world}, NCCL all-reduce of the gradients"}}), flush=True)
     if world > 1:
         dist.destroy_process_group()

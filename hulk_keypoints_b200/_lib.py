@@ -33,6 +33,8 @@ EXPORTS = (
     # round 2
     "hk_soft_argmax_workspace_bytes", "hk_soft_argmax", "hk_l1_normalize_dim1", "hk_stem_pool_fwd", "hk_stem_pool_fwd_u8",
     "hk_conv_ds_fwd", "hk_bn_acc_bytes", "hk_bn_stats_acc", "hk_bn_apply_fwd_acc", "hk_bn_bwd_acc", "hk_conv_bn_stats_fwd", "hk_conv_head_fwd", "hk_head_upsample_fwd", "hk_pack_conv_weights_many_tiled", "hk_maxpool3x3s2_fwd_idx", "hk_maxpool3x3s2_bwd_idx",
+    # frozen BatchNorm (eval()-mode BN inside a train()-mode model)
+    "hk_bn_fold", "hk_bn_frozen_bwd",
 )
 
 
@@ -115,6 +117,10 @@ def _declare(lib):
     lib.hk_bn_bwd_acc.argtypes = [vp, vp, i, vp, vp, vp, vp, ll, i, vp, vp, vp, i, vp, vp, vp]
     lib.hk_bn_train_bwd.restype = i
     lib.hk_bn_train_bwd.argtypes = [vp, vp, i, vp, vp, vp, vp, ll, i, vp, vp, i, vp, vp, vp, sz, vp]
+    lib.hk_bn_fold.restype = i
+    lib.hk_bn_fold.argtypes = [vp, i, i, vp]
+    lib.hk_bn_frozen_bwd.restype = i
+    lib.hk_bn_frozen_bwd.argtypes = [vp, vp, i, vp, vp, vp, vp, ll, i, vp, vp, vp, i, vp, vp, vp]
     lib.hk_pack_conv_weights_dgrad.restype = i
     lib.hk_pack_conv_weights_dgrad.argtypes = [vp, i, i, i, i, vp, vp]
     lib.hk_zero_insert2x.restype = i

@@ -722,6 +722,174 @@ static int bn_grid_apply(K kernel, long long nvec, size_t smem) {
 }
 static bool bn_c_ok(int C) { return C >= 8 && C <= 2048 && (C & 7) == 0 && (BN_THREADS % (C >> 3)) == 0; }
 
+// ================================================================================================================================
+// Frozen BatchNorm: a BatchNorm module in eval() mode inside a train()-mode model (fine-tuning with frozen BN, as torchvision's
+// detection and keypoint models do).  torch then normalises with the running statistics, which are constants of the step:
+//   forward : out = relu?(scale*y + shift [+ residual]),  scale = gamma*invstd_r, shift = beta - mean_r*scale (bn_fold_kernel)
+//   backward: d' = dout*[out>0];  dy = scale*d'  -- no batch-statistics terms;  dbeta = sum d',  dgamma = sum d'*(y - mean_r)*invstd_r
+// The backward is one pass.  Where gamma or beta is trained it adds (sum d', sum d'*y) into the 128-bit accumulators of hk_bn_acc.cuh
+// and the last cluster to retire derives dgamma = invstd_r*(sum d'*y - mean_r*sum d') and dbeta = sum d' from the exact totals
+// (deterministic, no finalize launch).  The retire counter is the spare word of the first accumulator (zero with the accumulators).
+
+// per-channel fold of every frozen BatchNorm of a step in one launch: blockIdx.y = item
+__global__ void __launch_bounds__(256) bn_fold_kernel(const HkBnFoldItem* __restrict__ items) {
+  const HkBnFoldItem it = items[blockIdx.y];
+  const int c = blockIdx.x * 256 + threadIdx.x;
+  if (c >= it.C) return;
+  const float invstd = (float)(1.0 / sqrt((double)it.var[c] + (double)it.eps));
+  const float g = it.gamma ? it.gamma[c] : 1.f, bt = it.beta ? it.beta[c] : 0.f;
+  const float sc = g * invstd;
+  it.scale[c] = sc;
+  it.shift[c] = bt - it.mean[c] * sc;
+  if (it.invstd) it.invstd[c] = invstd;
+}
+
+// accumulator totals written by other CTAs' atomics: read through L2
+__device__ __forceinline__ double bn_acc_read_l2(const BnAcc* a) {
+  BnAcc v;
+  v.lo = __ldcg(&a->lo);
+  v.hi = __ldcg(&a->hi);
+  v.poison = __ldcg(&a->poison);
+  return bn_acc_read(&v);
+}
+
+// The bf16-mask variant keeps a third 16-byte operand per vector in flight: held to BN_APPLY_MINB blocks per SM it spills, so it runs
+// at one resident block fewer.
+template <bool BITS>
+__global__ void __cluster_dims__(BN_CLUSTER, 1, 1) __launch_bounds__(BN_THREADS, BITS ? BN_APPLY_MINB : BN_APPLY_MINB - 1)
+bn_frozen_bwd_kernel(const __nv_bfloat16* __restrict__ dout, const void* __restrict__ out_mask, const __nv_bfloat16* __restrict__ y,
+                     const float* __restrict__ scale, const float* __restrict__ mean, const float* __restrict__ invstd,
+                     BnAcc* __restrict__ acc, float* __restrict__ dgamma, float* __restrict__ dbeta, int accumulate,
+                     __nv_bfloat16* __restrict__ dy, __nv_bfloat16* __restrict__ dmasked, long long nvec, int C) {
+  // the channel group of a thread is the same for every vector it touches (the grid stride is a multiple of 256, 256 of C/8), and it is
+  // the one block_reduce_2x8_small expects (threadIdx % (C/8))
+  const int c0 = (threadIdx.x % (C >> 3)) * 8;
+  float k[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) k[j] = __ldg(scale + c0 + j);
+  float s1[8] = {0, 0, 0, 0, 0, 0, 0, 0}, s2[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  const bool sums = acc != nullptr;
+  const uint8_t* mbits = static_cast<const uint8_t*>(out_mask);
+  const __nv_bfloat16* mvals = static_cast<const __nv_bfloat16*>(out_mask);
+  auto finish = [&](long long i, const uint4& du, uint32_t m, const uint4& mu4, const uint4& vu) {
+    float d[8];
+    unpack_bf16x2(du.x, d[0], d[1]); unpack_bf16x2(du.y, d[2], d[3]); unpack_bf16x2(du.z, d[4], d[5]); unpack_bf16x2(du.w, d[6], d[7]);
+    if (out_mask) {
+      if constexpr (BITS) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) d[j] = (m >> j) & 1u ? d[j] : 0.f;
+      } else {
+        float mv[8];
+        unpack_bf16x2(mu4.x, mv[0], mv[1]); unpack_bf16x2(mu4.y, mv[2], mv[3]); unpack_bf16x2(mu4.z, mv[4], mv[5]); unpack_bf16x2(mu4.w, mv[6], mv[7]);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) d[j] = mv[j] > 0.f ? d[j] : 0.f;
+      }
+    }
+    if (dmasked) store8(dmasked + i * 8, d);
+    if (dy) {
+      float o[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) o[j] = k[j] * d[j];
+      store8(dy + i * 8, o);
+    }
+    if (sums) {
+      float v[8];
+      unpack_bf16x2(vu.x, v[0], v[1]); unpack_bf16x2(vu.y, v[2], v[3]); unpack_bf16x2(vu.z, v[4], v[5]); unpack_bf16x2(vu.w, v[6], v[7]);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) { s1[j] += d[j]; s2[j] = fmaf(d[j], v[j], s2[j]); }
+    }
+  };
+  auto load = [&](long long iu, uint4& du, uint32_t& m, uint4& mu4, uint4& vu) {
+    du = *reinterpret_cast<const uint4*>(dout + iu * 8);
+    vu = sums ? *reinterpret_cast<const uint4*>(y + iu * 8) : make_uint4(0, 0, 0, 0);
+    m = 0;
+    mu4 = make_uint4(0, 0, 0, 0);
+    if (out_mask) {
+      if constexpr (BITS) m = mbits[iu];
+      else mu4 = *reinterpret_cast<const uint4*>(mvals + iu * 8);
+    }
+  };
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  const long long us = BN_APPLY_CONTIG ? BN_THREADS : stride, adv = BN_APPLY_U * stride;
+  for (long long i = (long long)blockIdx.x * (BN_APPLY_CONTIG ? BN_APPLY_U * BN_THREADS : BN_THREADS) + threadIdx.x; i < nvec; i += adv) {
+    if (i + (BN_APPLY_U - 1) * us < nvec) {   // BN_APPLY_U vectors (x 1-3 loads) in flight per thread
+      uint4 du[BN_APPLY_U], mu4[BN_APPLY_U], vu[BN_APPLY_U];
+      uint32_t m[BN_APPLY_U];
+#pragma unroll
+      for (int u = 0; u < BN_APPLY_U; ++u) load(i + u * us, du[u], m[u], mu4[u], vu[u]);
+#pragma unroll
+      for (int u = 0; u < BN_APPLY_U; ++u) finish(i + u * us, du[u], m[u], mu4[u], vu[u]);
+    } else {
+      for (int u = 0; u < BN_APPLY_U && i + u * us < nvec; ++u) {
+        uint4 du, mu4, vu;
+        uint32_t m;
+        load(i + u * us, du, m, mu4, vu);
+        finish(i + u * us, du, m, mu4, vu);
+      }
+    }
+  }
+  if (!sums) return;
+  bn_cluster_emit(s1, s2, C, acc);
+  if (cg::this_cluster().block_rank() != 0) return;
+  // CTA 0 of every cluster has issued its cluster's atomics: the last one to get here turns the totals into dgamma / dbeta.  The flag
+  // lives in the dynamic buffer of bn_cluster_emit, free after its final cluster barrier (a static __shared__ variable here could be
+  // placed ahead of block_reduce_2x8_small's buffer and break the alignment of its float4 stores).
+  extern __shared__ float s_tot[];
+  volatile int* last = reinterpret_cast<volatile int*>(s_tot);
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) *last = atomicAdd(&acc[0].pad, 1ull) == (unsigned long long)(gridDim.x / BN_CLUSTER - 1) ? 1 : 0;
+  __syncthreads();
+  if (!*last) return;
+  __threadfence();
+  for (int c = threadIdx.x; c < C; c += BN_THREADS) {
+    const double t1 = bn_acc_read_l2(acc + c), t2 = bn_acc_read_l2(acc + C + c);
+    if (dbeta) dbeta[c] = (accumulate ? dbeta[c] : 0.f) + (float)t1;
+    if (dgamma) dgamma[c] = (accumulate ? dgamma[c] : 0.f) + (float)((double)invstd[c] * (t2 - (double)mean[c] * t1));
+  }
+  if (threadIdx.x == 0) acc[0].pad = 0;   // the buffer can be cleared and reused as before
+}
+
+// Grid of the frozen backward: chunks of BN_APPLY_U x 256 vectors shared equally (as bn_grid_apply), in whole 8-CTA clusters, at most one
+// resident wave of clusters (cudaOccupancyMaxActiveClusters, see bn_grid_acc_rows).
+template <int TAG, class K>
+static int bn_grid_frozen(K kernel, long long nvec, size_t smem) {
+  static int resident_by_dev[64] = {0};
+  int dev = 0;
+  (void)cudaGetDevice(&dev);
+  int fallback = 0;
+  int& resident = dev < 64 ? resident_by_dev[dev] : fallback;
+  if (resident == 0) {
+    int clusters = 0;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(BN_CLUSTER * (unsigned)sm_count(), 1, 1);
+    cfg.blockDim = dim3(BN_THREADS, 1, 1);
+    cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = BN_CLUSTER;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    if (cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg) == cudaSuccess && clusters > 0) {
+      resident = clusters * BN_CLUSTER;
+    } else {
+      (void)cudaGetLastError();
+      int occ = 0;
+      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, BN_THREADS, smem) != cudaSuccess || occ < 1) occ = 2;
+      resident = (occ * sm_count() / BN_CLUSTER - 8) * BN_CLUSTER;
+    }
+    if (resident < BN_CLUSTER) resident = BN_CLUSTER;
+  }
+  const long long chunks = ceil_div_ll(nvec, (long long)BN_THREADS * BN_APPLY_U);
+  const long long iters = ceil_div_ll(chunks, resident);
+  long long blocks = ceil_div_ll(ceil_div_ll(chunks, iters), BN_CLUSTER) * BN_CLUSTER;
+  if (blocks > resident) blocks = resident;
+  if (blocks < BN_CLUSTER) blocks = BN_CLUSTER;
+  return (int)blocks;
+}
+
 }  // namespace hk
 
 extern "C" {
@@ -837,6 +1005,39 @@ int hk_bn_bwd_acc(const void* dout, const void* out_mask_or_null, int mask_is_bi
     bn_bwd_apply_acc_kernel<false><<<ablocks, BN_THREADS, 3 * (size_t)C * 4, as_stream(stream)>>>(d, out_mask_or_null, yy, mean, invstd, gamma, a, P, dgamma, dbeta, accumulate,
                                                                                 static_cast<__nv_bfloat16*>(dy), static_cast<__nv_bfloat16*>(dmasked_or_null), nvec, C);
   return check_launch("bn_bwd_apply_acc_kernel");
+}
+
+int hk_bn_fold(const HkBnFoldItem* items_dev, int n_items, int max_c, void* stream) {
+  using namespace hk;
+  HK_REQUIRE(items_dev && n_items > 0 && n_items <= 65535 && max_c > 0, "hk_bn_fold: bad argument");
+  bn_fold_kernel<<<dim3(ceil_div(max_c, 256), n_items), 256, 0, as_stream(stream)>>>(items_dev);
+  return check_launch("bn_fold_kernel");
+}
+
+int hk_bn_frozen_bwd(const void* dout, const void* out_mask_or_null, int mask_is_bits, const void* y_or_null, const float* scale,
+                     const float* mean, const float* invstd, long long P, int C, void* acc_or_null, float* dgamma, float* dbeta,
+                     int accumulate, void* dy_or_null, void* dmasked_or_null, void* stream) {
+  using namespace hk;
+  HK_REQUIRE(dout && scale, "hk_bn_frozen_bwd: null pointer");
+  HK_REQUIRE(P > 0 && bn_c_ok(C), "hk_bn_frozen_bwd: unsupported shape P=%lld C=%d", P, C);
+  const bool sums = dgamma || dbeta;
+  HK_REQUIRE(!sums || (acc_or_null && y_or_null && mean && invstd), "hk_bn_frozen_bwd: dgamma/dbeta need y, mean, invstd and an accumulator buffer");
+  HK_REQUIRE(!acc_or_null || (reinterpret_cast<uintptr_t>(acc_or_null) & 31) == 0, "hk_bn_frozen_bwd: misaligned accumulator buffer");
+  HK_REQUIRE(sums || dy_or_null || dmasked_or_null, "hk_bn_frozen_bwd: nothing to compute");
+  const long long nvec = P * (C >> 3);
+  BnAcc* a = sums ? static_cast<BnAcc*>(acc_or_null) : nullptr;
+  const size_t smem = 2 * (size_t)C * 4;
+  const __nv_bfloat16* d = static_cast<const __nv_bfloat16*>(dout);
+  const __nv_bfloat16* yy = static_cast<const __nv_bfloat16*>(y_or_null);
+  __nv_bfloat16* dyp = static_cast<__nv_bfloat16*>(dy_or_null);
+  __nv_bfloat16* dm = static_cast<__nv_bfloat16*>(dmasked_or_null);
+  if (mask_is_bits)
+    bn_frozen_bwd_kernel<true><<<bn_grid_frozen<1>(bn_frozen_bwd_kernel<true>, nvec, smem), BN_THREADS, smem, as_stream(stream)>>>(
+        d, out_mask_or_null, yy, scale, mean, invstd, a, dgamma, dbeta, accumulate, dyp, dm, nvec, C);
+  else
+    bn_frozen_bwd_kernel<false><<<bn_grid_frozen<2>(bn_frozen_bwd_kernel<false>, nvec, smem), BN_THREADS, smem, as_stream(stream)>>>(
+        d, out_mask_or_null, yy, scale, mean, invstd, a, dgamma, dbeta, accumulate, dyp, dm, nvec, C);
+  return check_launch("bn_frozen_bwd_kernel");
 }
 
 }  // extern "C"

@@ -424,7 +424,7 @@ size_t hk_head_bwd_workspace_bytes(int B, int K, int C, int h, int w) {
 int hk_head_bwd(const float* g_up, const void* feat, const float* w_fc, float* dlogits_ws, void* dfeat, float* dw_fc, float* db_fc,
                 int accumulate, int B, int K, int C, int h, int w, int H, int W, void* ws, size_t ws_bytes, void* stream) {
   using namespace hk;
-  HK_REQUIRE(g_up && feat && w_fc && dlogits_ws && dfeat && dw_fc && db_fc && ws, "hk_head_bwd: null pointer");
+  HK_REQUIRE(g_up && feat && w_fc && dlogits_ws && ws, "hk_head_bwd: null pointer");
   HK_REQUIRE(B > 0 && K > 0 && C >= 8 && (C & 7) == 0 && h > 0 && w > 0 && H > 0 && W > 0, "hk_head_bwd: bad shape");
   HK_REQUIRE(ws_bytes >= hk_head_bwd_workspace_bytes(B, K, C, h, w), "hk_head_bwd: workspace too small");
   HK_REQUIRE((long long)B * K * h * w < 0x7fffffffLL, "hk_head_bwd: too many low-res elements");
@@ -444,18 +444,23 @@ int hk_head_bwd(const float* g_up, const void* feat, const float* w_fc, float* d
   }
   if (rc) return rc;
   const int hw = h * w;
-  fc_bwd_dfeat_kernel<<<grid_for((long long)B * hw * (C >> 3), 256), 256, 0, s>>>(dlogits_ws, w_fc, static_cast<__nv_bfloat16*>(dfeat), B, K,
-                                                                                 C, hw);
-  rc = check_launch("fc_bwd_dfeat_kernel");
-  if (rc) return rc;
-  const int nblk = (int)(((long long)B * hw + FCW_SLAB - 1) / FCW_SLAB);
-  fc_bwd_dw_partial_kernel<<<nblk, 256, 0, s>>>(dlogits_ws, static_cast<const __nv_bfloat16*>(feat), static_cast<float*>(ws), B, K, C, hw);
-  rc = check_launch("fc_bwd_dw_partial_kernel");
-  if (rc) return rc;
-  HK_REQUIRE(C % 32 == 0, "hk_head_bwd: C must be a multiple of 32");
-  fc_bwd_dw_finalize_kernel<<<dim3(C / 32, K), 256, 0, s>>>(static_cast<const float*>(ws), nblk, dw_fc, K, C, accumulate);
-  rc = check_launch("fc_bwd_dw_finalize_kernel");
-  if (rc) return rc;
+  if (dfeat) {
+    fc_bwd_dfeat_kernel<<<grid_for((long long)B * hw * (C >> 3), 256), 256, 0, s>>>(dlogits_ws, w_fc, static_cast<__nv_bfloat16*>(dfeat), B,
+                                                                                   K, C, hw);
+    rc = check_launch("fc_bwd_dfeat_kernel");
+    if (rc) return rc;
+  }
+  if (dw_fc) {
+    const int nblk = (int)(((long long)B * hw + FCW_SLAB - 1) / FCW_SLAB);
+    fc_bwd_dw_partial_kernel<<<nblk, 256, 0, s>>>(dlogits_ws, static_cast<const __nv_bfloat16*>(feat), static_cast<float*>(ws), B, K, C, hw);
+    rc = check_launch("fc_bwd_dw_partial_kernel");
+    if (rc) return rc;
+    HK_REQUIRE(C % 32 == 0, "hk_head_bwd: C must be a multiple of 32");
+    fc_bwd_dw_finalize_kernel<<<dim3(C / 32, K), 256, 0, s>>>(static_cast<const float*>(ws), nblk, dw_fc, K, C, accumulate);
+    rc = check_launch("fc_bwd_dw_finalize_kernel");
+    if (rc) return rc;
+  }
+  if (!db_fc) return 0;
   // the dw partials in `ws` are consumed: its head is reused for the B x K double partials of db
   HK_REQUIRE(ws_bytes >= (size_t)B * K * sizeof(double) && (reinterpret_cast<uintptr_t>(ws) & 7) == 0, "hk_head_bwd: workspace too small for db");
   fc_bwd_db_partial_kernel<<<dim3(K, B), 256, 0, s>>>(dlogits_ws, static_cast<double*>(ws), K, hw);

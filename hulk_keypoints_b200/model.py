@@ -238,6 +238,20 @@ class KeypointsGauss(nn.Module):
             return f"H and W must be multiples of 8 and >= 32, got {tuple(x.shape[2:])}"
         if not torch.is_grad_enabled():
             return "autograd is disabled (train-mode forward under no_grad; use model.eval() for inference)"
+        return self._bn_unsupported()
+
+    def _bn_unsupported(self):
+        """None when the training engine can express every BatchNorm of the backbone, else the reason as text.  The engine honours
+        bn.training (eval()-mode BatchNorm inside a train()-mode model: running statistics, buffers untouched) and requires_grad; it
+        has no path for cumulative averaging, batch statistics without running buffers, or a BatchNorm without gamma / beta."""
+        for name, m in self.resnet.resnet34_8s.named_modules():
+            if isinstance(m, nn.BatchNorm2d):
+                if m.momentum is None:
+                    return f"BatchNorm {name} has momentum=None (cumulative moving average), which the engine does not implement"
+                if not m.track_running_stats or m.running_mean is None:
+                    return f"BatchNorm {name} has track_running_stats=False, which the engine does not implement"
+                if not m.affine:
+                    return f"BatchNorm {name} has affine=False, which the engine does not implement"
         return None
 
     def forward_logits(self, x):

@@ -469,6 +469,55 @@ def bn_bwd_acc(dout: torch.Tensor, out_mask: Optional[torch.Tensor], y: torch.Te
     return dy
 
 
+BN_FOLD_ITEM = None   # numpy dtype of HkBnFoldItem (include/hulk_sm100.h), built on first use
+
+
+def bn_fold_items(items) -> torch.Tensor:
+    """[(gamma, beta, running_mean, running_var, eps, scale_out, shift_out, invstd_out_or_None), ...] -> the HkBnFoldItem array of
+    bn_fold as a uint8 CPU tensor (upload it once; the pointers are read by the kernel at every launch)."""
+    import numpy as np
+    global BN_FOLD_ITEM
+    if BN_FOLD_ITEM is None:
+        BN_FOLD_ITEM = np.dtype([("g", "<u8"), ("b", "<u8"), ("m", "<u8"), ("v", "<u8"), ("sc", "<u8"), ("sh", "<u8"), ("inv", "<u8"),
+                                 ("eps", "<f4"), ("C", "<i4")])
+    arr = np.zeros(len(items), dtype=BN_FOLD_ITEM)
+    for i, (g, b, m, v, eps, sc, sh, inv) in enumerate(items):
+        _need_cuda(g, b, m, v, sc, sh, inv)
+        Cc = m.numel()
+        if any(t is not None and (t.dtype != torch.float32 or t.numel() != Cc or not t.is_contiguous()) for t in (g, b, m, v, sc, sh, inv)):
+            raise ValueError("bn_fold: every tensor of an item must be a contiguous fp32 (C,) tensor")
+        arr[i] = tuple(0 if t is None else t.data_ptr() for t in (g, b, m, v, sc, sh, inv)) + (eps, Cc)
+    return torch.from_numpy(arr.view(np.uint8).copy())
+
+
+def bn_fold(items_dev: torch.Tensor, n_items: int, max_c: int) -> None:
+    """Frozen BatchNorms in one launch: scale = gamma/sqrt(running_var + eps), shift = beta - running_mean*scale, invstd (items of
+    bn_fold_items, on the device)."""
+    _need_cuda(items_dev)
+    check(lib().hk_bn_fold(ptr(items_dev), n_items, max_c, stream_ptr()), "hk_bn_fold")
+
+
+def bn_frozen_bwd(dout: torch.Tensor, out_mask: Optional[torch.Tensor], scale: torch.Tensor, dy: Optional[torch.Tensor],
+                  dmasked: Optional[torch.Tensor] = None, y: Optional[torch.Tensor] = None, mean: Optional[torch.Tensor] = None,
+                  invstd: Optional[torch.Tensor] = None, acc: Optional[torch.Tensor] = None, dgamma: Optional[torch.Tensor] = None,
+                  dbeta: Optional[torch.Tensor] = None, accumulate: bool = False) -> Optional[torch.Tensor]:
+    """Backward of a BatchNorm in eval() mode (running statistics) + the ReLU after it, one pass: d' = dout*[out>0] (out_mask: the
+    bf16 post-ReLU output or the uint8 bit mask of bn_apply; None = no ReLU), dy = scale*d', d' into `dmasked`; with dgamma / dbeta,
+    also dbeta = sum d' and dgamma = sum d'*(y - mean)*invstd through `acc` (zeroed, bn_acc_bytes(C)).  mean = running mean."""
+    _need_cuda(dout, out_mask, scale, dy, dmasked, y, mean, invstd, acc, dgamma, dbeta)
+    Cc = dout.shape[-1]
+    P = dout.numel() // Cc
+    for t in (out_mask, dy, dmasked, y):
+        if t is not None and t.dtype == torch.bfloat16 and t.shape != dout.shape:
+            raise ValueError(f"bn_frozen_bwd: shape {tuple(t.shape)} != dout {tuple(dout.shape)}")
+    if acc is not None and acc.numel() * acc.element_size() < bn_acc_bytes(Cc):
+        raise ValueError("accumulator buffer too small")
+    bits = out_mask is not None and out_mask.dtype == torch.uint8
+    check(lib().hk_bn_frozen_bwd(ptr(dout), ptr(out_mask), int(bits), ptr(y), ptr(scale), ptr(mean), ptr(invstd), C.c_longlong(P), Cc,
+                                 ptr(acc), ptr(dgamma), ptr(dbeta), int(accumulate), ptr(dy), ptr(dmasked), stream_ptr()), "hk_bn_frozen_bwd")
+    return dy
+
+
 def pack_conv_weights_dgrad(w_oihw: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """OIHW fp32 -> (cin, kh, kw, cout) bf16 with flipped taps: the weights of the data-gradient convolution."""
     _need_cuda(w_oihw, out)
@@ -585,9 +634,11 @@ def head_logits(feat: torch.Tensor, w_fc: torch.Tensor, b_fc: torch.Tensor, H: i
     return out
 
 
-def head_bwd(g_up: torch.Tensor, feat: torch.Tensor, w_fc: torch.Tensor, dfeat: torch.Tensor, dw_fc: torch.Tensor, db_fc: torch.Tensor,
-             dlogits_ws: Optional[torch.Tensor] = None, ws: Optional[torch.Tensor] = None, accumulate: bool = False):
-    """Backward of head_logits: g_up (B,K,H,W) fp32 -> dfeat (B,h,w,C) bf16, dw_fc (K,C) fp32, db_fc (K) fp32."""
+def head_bwd(g_up: torch.Tensor, feat: torch.Tensor, w_fc: torch.Tensor, dfeat: Optional[torch.Tensor], dw_fc: Optional[torch.Tensor],
+             db_fc: Optional[torch.Tensor], dlogits_ws: Optional[torch.Tensor] = None, ws: Optional[torch.Tensor] = None,
+             accumulate: bool = False):
+    """Backward of head_logits: g_up (B,K,H,W) fp32 -> dfeat (B,h,w,C) bf16, dw_fc (K,C) fp32, db_fc (K) fp32 (each may be None:
+    not computed)."""
     _need_cuda(g_up, feat, w_fc, dfeat, dw_fc, db_fc, dlogits_ws, ws)
     B, K, H, W = g_up.shape
     _, h, w, Cc = feat.shape

@@ -51,7 +51,8 @@ class FusedAdam:
         """Use an external flat gradient buffer with this optimiser's layout (TrainEngine.flat_grad): the engine's kernels then write
         the gradients exactly where the all-reduce and hk_adam_step read them -- no copy."""
         if flat_grad.shape != self.flat_grad.shape or flat_grad.dtype != torch.float32 or flat_grad.device != self.flat_grad.device:
-            raise ValueError("gradient buffer layout mismatch")
+            raise ValueError("gradient buffer layout mismatch (the optimiser was built for another set of trainable parameters: "
+                             "build it after setting requires_grad, as in torch)")
         self.flat_grad = flat_grad
         o = 0
         for p in self.params:

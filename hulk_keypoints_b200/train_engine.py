@@ -14,17 +14,149 @@ the 996 dead rows of the 1000-row scoring conv keep a zero gradient, as in the r
 Data layout in HBM (per engine, batch B of H x W): input (B,3,H,W) f32; per conv a raw output and an activation,
 (B,h,w,C) bf16 NHWC; (B,K,H,W) f32 upsampled logits and their gradient; scratch gradients sized by stage.
 The whole step is captured in one CUDA graph (~560 launches) and replayed.
+
+Fine-tuning: BatchNorms in eval() mode (running statistics, buffers untouched) and parameters with requires_grad=False follow torch's
+semantics; `backward_plan` decides from those flags what the backward computes and where it stops (DESIGN §3.5).
 """
 from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 
 from . import ops
 from ._lib import HK_BF16, check, lib, ptr, require_device, stream_ptr
+
+
+# ---------------------------------------------------------------------------------------------------------------- backward plan
+class ConvPlan(NamedTuple):
+    """What the step does for one conv + BatchNorm, from the torch flags (bn.training, p.requires_grad)."""
+    frozen: bool    # BatchNorm in eval() mode: normalises with the running statistics, writes none of its buffers
+    dgamma: bool    # gradients wanted for the BatchNorm's gamma / beta
+    dbeta: bool
+    wgrad: bool     # conv weight gradient
+    dgrad: bool     # gradient of the conv's input (something below still needs a gradient)
+    dy: bool        # gradient of the raw conv output (for wgrad and/or dgrad)
+    bwd: bool       # the BatchNorm backward runs at all
+
+
+_NO_BWD = dict(dgamma=False, dbeta=False, wgrad=False, dgrad=False, dy=False, bwd=False)
+
+
+class BackwardPlan(NamedTuple):
+    convs: Dict[str, ConvPlan]      # by TrainEngine conv name: "stem", "b{i}.c1", "b{i}.c2", "b{i}.ds"
+    fc_weight: bool
+    fc_bias: bool
+    dfeat: bool                     # the head backward hands a gradient to the backbone
+    grad_in: Tuple[bool, ...]       # per block: the gradient of the block's input is needed
+    lo: int                         # first block the backward visits (len(blocks): none)
+    stem: bool                      # max-pool + stem BatchNorm (+ stem weight gradient) backward run
+
+    @property
+    def frozen_any(self) -> bool:
+        return any(p.frozen for p in self.convs.values())
+
+    @property
+    def train_bn_any(self) -> bool:
+        return not all(p.frozen for p in self.convs.values())
+
+
+def _data_ptr(t) -> Optional[int]:
+    return None if t is None else t.data_ptr()
+
+
+def _trains(m: torch.nn.Module) -> bool:
+    return any(p.requires_grad for p in m.parameters())
+
+
+def backward_plan(net) -> BackwardPlan:
+    """The work of one training step under the current torch flags of the backbone `net` (model.resnet.resnet34_8s): which BatchNorms
+    are frozen, which convs need dy / a weight gradient / a data gradient, which BatchNorms need dgamma / dbeta.  The backward runs
+    from the head down to the earliest point that still needs a gradient and nothing below it.  Pure (no device work)."""
+    blocks = list(net.blocks())
+    nb = len(blocks)
+    convs: Dict[str, ConvPlan] = {}
+
+    def conv_plan(conv, bn, dgrad: bool, extra_bwd: bool = False) -> ConvPlan:
+        dg, db, wg = bn.weight is not None and bn.weight.requires_grad, bn.bias is not None and bn.bias.requires_grad, conv.weight.requires_grad
+        dy = wg or dgrad
+        return ConvPlan(frozen=not bn.training, dgamma=dg, dbeta=db, wgrad=wg, dgrad=dgrad, dy=dy, bwd=dy or dg or db or extra_bwd)
+
+    below = _trains(net.conv1) or _trains(net.bn1)
+    grad_in = []
+    for blk in blocks:
+        grad_in.append(below)
+        below = below or _trains(blk)
+    dfeat = below
+    lo = next((bi for bi in range(nb) if grad_in[bi] or _trains(blocks[bi])), nb)
+    for bi, blk in enumerate(blocks):
+        ds = blk.downsample
+        if bi < lo:
+            for name, bn in ((f"b{bi}.c1", blk.bn1), (f"b{bi}.c2", blk.bn2)) + (((f"b{bi}.ds", ds[1]),) if ds is not None else ()):
+                convs[name] = ConvPlan(frozen=not bn.training, **_NO_BWD)
+            continue
+        p1 = conv_plan(blk.conv1, blk.bn1, dgrad=grad_in[bi])
+        pd = conv_plan(ds[0], ds[1], dgrad=grad_in[bi]) if ds is not None else None
+        # conv2's BatchNorm backward also forms d' = dout*[out>0], the gradient of the shortcut branch
+        p2 = conv_plan(blk.conv2, blk.bn2, dgrad=p1.bwd, extra_bwd=pd.bwd if pd is not None else grad_in[bi])
+        convs[f"b{bi}.c1"], convs[f"b{bi}.c2"] = p1, p2
+        if pd is not None:
+            convs[f"b{bi}.ds"] = pd
+    st = conv_plan(net.conv1, net.bn1, dgrad=False)
+    convs["stem"] = st
+    return BackwardPlan(convs=convs, fc_weight=net.fc.weight.requires_grad, fc_bias=net.fc.bias is not None and net.fc.bias.requires_grad,
+                        dfeat=dfeat, grad_in=tuple(grad_in), lo=lo, stem=st.bwd)
+
+
+def step_launches(net, plan: BackwardPlan) -> int:
+    """Kernel launches of one TrainEngine.forward_backward step under `plan`, in the engine's default configuration (accumulator
+    BatchNorm path, epilogue statistics for the 3x3 convs with >= 256 channels, max-pool indices): what `TrainEngine.launches` reports."""
+    blocks = list(net.blocks())
+
+    def fwd(name, conv) -> int:
+        p = plan.convs[name]
+        if p.frozen:
+            return 2 if (p.dgamma or p.dbeta) else 1
+        return 2 if (conv.kernel_size[0] == 3 and conv.out_channels >= 256) else 3
+
+    def bn_bwd(name) -> int:
+        return 1 if plan.convs[name].frozen else 2
+
+    def dgrad(conv) -> int:
+        return 2 if conv.stride[0] == 2 else 1
+
+    n = 2 + (1 if plan.train_bn_any else 0) + (1 if plan.frozen_any else 0)                     # weight packs, accumulator memset, BN fold
+    st = plan.convs["stem"]
+    n += (2 if (st.dgamma or st.dbeta) else 1) if st.frozen else 3                                # stem conv + its BatchNorm
+    n += 1                                                                                        # max-pool
+    for bi, blk in enumerate(blocks):
+        n += fwd(f"b{bi}.c1", blk.conv1) + fwd(f"b{bi}.c2", blk.conv2)
+        if blk.downsample is not None:
+            n += fwd(f"b{bi}.ds", blk.downsample[0])
+    n += 2 + (1 if plan.train_bn_any else 0)                                                      # head logits, num_batches_tracked
+    n += 2                                                                                        # fused loss
+    # backward
+    users = [name for name, p in plan.convs.items() if p.bwd and (not p.frozen or p.dgamma or p.dbeta)]
+    n += 1 if users else 0                                                                        # backward accumulator memset
+    if plan.dfeat or plan.fc_weight or plan.fc_bias:
+        n += 5 - (not plan.dfeat) - 2 * (not plan.fc_weight) - 2 * (not plan.fc_bias)
+    for bi in range(len(blocks) - 1, plan.lo - 1, -1):
+        blk = blocks[bi]
+        p1, p2 = plan.convs[f"b{bi}.c1"], plan.convs[f"b{bi}.c2"]
+        if p2.bwd:
+            n += bn_bwd(f"b{bi}.c2")
+        if blk.downsample is not None:
+            pd = plan.convs[f"b{bi}.ds"]
+            if pd.bwd:
+                n += bn_bwd(f"b{bi}.ds") + (2 if pd.wgrad else 0) + (dgrad(blk.downsample[0]) if pd.dgrad else 0)
+        n += (2 if p2.wgrad else 0) + (dgrad(blk.conv2) if p2.dgrad else 0)
+        if p1.bwd:
+            n += bn_bwd(f"b{bi}.c1") + (2 if p1.wgrad else 0) + (dgrad(blk.conv1) if p1.dgrad else 0)
+    if plan.stem:
+        n += 1 + bn_bwd("stem") + (2 if st.wgrad else 0)                                          # max-pool, BatchNorm, weight gradient
+    return n
 
 
 class _ConvT:
@@ -60,14 +192,11 @@ class TrainEngine:
         self.model, self.net, self.device = model, net, dev
         self.B, self.H, self.W, self.K, self.sigma = B, H, W, int(model.num_keypoints), float(sigma)
         bf = torch.bfloat16
-        # ---- flat gradient buffer, FusedAdam layout (each tensor starts on a 16-byte boundary) ----
-        self.params: List[torch.nn.Parameter] = [p for p in model.parameters() if p.requires_grad]
-        offs, total = [], 0
-        for p in self.params:
-            offs.append(total)
-            total += (p.numel() + 3) // 4 * 4
-        self.flat_grad = torch.zeros(total, device=dev, dtype=torch.float32)
-        self.grad_of: Dict[int, torch.Tensor] = {id(p): self.flat_grad[o:o + p.numel()].view_as(p) for p, o in zip(self.params, offs)}
+        # first block of layer3: everything from here to the end of the parameter list (layer3, layer4, fc) is the "late" part
+        self.split_block = 7
+        self.all_params: List[torch.nn.Parameter] = list(model.parameters())   # the engine is bound to the model's modules, like its convs
+        self.params: List[torch.nn.Parameter] = []
+        self._build_grad_buffer([p for p in self.all_params if p.requires_grad])
         # ---- buffers ----
         self.x = torch.empty((B, 3, H, W), device=dev, dtype=torch.float32)
         self.uv = torch.zeros((B, self.K, 2), device=dev, dtype=torch.float32)
@@ -126,16 +255,15 @@ class TrainEngine:
         wg = max(ops.conv_wgrad_workspace_bytes(B, c.H, c.W, c.cin, c.cout, c.k, c.stride, c.pad, c.dil) for c in self.convs[1:])
         self.wgrad_ws = torch.empty(max(wg, int(lib().hk_stem_wgrad_workspace_bytes())), device=dev, dtype=torch.uint8)
         self.head_ws = torch.empty(int(lib().hk_head_bwd_workspace_bytes(B, K, 512, h, w)), device=dev, dtype=torch.uint8)
-        # first block of layer3: everything from here to the end of the parameter list (layer3, layer4, fc) is the "late" part
-        self.split_block = 7
-        first_late = self.blocks[self.split_block][0].conv.weight
         self.acc_early_bytes = offs_acc[self.convs.index(self.blocks[self.split_block][0])]   # accumulators of the stem + early blocks
-        self.late_offset = next(o for p, o in zip(self.params, offs) if p is first_late)
         self._bwd_state = None
         self._scratch: Dict[Tuple, torch.Tensor] = {}
         self._pack_key = None
         self._pack_items: Optional[torch.Tensor] = None
-        self._bn_counters = [c.bn.num_batches_tracked for c in self.convs]
+        self._fold_key = None
+        self._fold_items: Optional[torch.Tensor] = None
+        self._flags = None
+        self.sync_flags()          # flat gradient buffer, backward plan, BatchNorm counters
         self.graph: Optional[torch.cuda.CUDAGraph] = None
         self._graph_key = None
         self.use_cuda_graph = os.environ.get("HK_TRAIN_NO_GRAPH") is None   # eager launches for ncu launch lists
@@ -157,6 +285,39 @@ class TrainEngine:
                       for b in self.blocks for c in (b[2],) if c is not None)
             self.wgrad_ws_aux = torch.empty(wga, device=dev, dtype=torch.uint8)
         self.launches = 0
+
+    # ------------------------------------------------------------------ torch flags
+    def sync_flags(self) -> None:
+        """Read bn.training and p.requires_grad (torch's fine-tuning switches) and, when they changed since the last step, rebuild what
+        depends on them: the flat gradient buffer (trainable parameters only, FusedAdam's layout), the backward plan and the list of
+        BatchNorms whose num_batches_tracked advances.  The flags are part of every graph key, so no stale graph is replayed."""
+        params = self.all_params
+        flags = (tuple(c.bn.training for c in self.convs), tuple(p.requires_grad for p in params))
+        if flags == self._flags:
+            return
+        why = self.model._bn_unsupported()
+        if why is not None:
+            raise RuntimeError(f"TrainEngine cannot run this model: {why}")
+        trainable = [p for p in params if p.requires_grad]
+        if [id(p) for p in trainable] != [id(p) for p in self.params]:
+            self._build_grad_buffer(trainable)
+        self.plan = backward_plan(self.net)
+        self._bn_counters = [c.bn.num_batches_tracked for c in self.convs if c.bn.training]
+        self._flags = flags
+
+    def _build_grad_buffer(self, trainable: List[torch.nn.Parameter]) -> None:
+        """Flat gradient buffer of the trainable parameters, FusedAdam's layout (each tensor starts on a 16-byte boundary)."""
+        self.params = trainable
+        offs, total = [], 0
+        for p in self.params:
+            offs.append(total)
+            total += (p.numel() + 3) // 4 * 4
+        self.flat_grad = torch.zeros(total, device=self.device, dtype=torch.float32)
+        self.grad_of: Dict[int, torch.Tensor] = {id(p): self.flat_grad[o:o + p.numel()].view_as(p) for p, o in zip(self.params, offs)}
+        # the "late" part of the two-phase step (layer3, layer4, fc) starts at the first trainable parameter at or after layer3.0
+        late = {id(p) for blk in list(self.net.blocks())[self.split_block:] for p in blk.parameters()}
+        late |= {id(p) for p in self.net.fc.parameters()}
+        self.late_offset = next((o for p, o in zip(self.params, offs) if id(p) in late), total)
 
     # ------------------------------------------------------------------ helpers
     def _buf(self, role: str, shape) -> torch.Tensor:
@@ -207,8 +368,41 @@ class TrainEngine:
             n += 1
         return n
 
+    def _fold_frozen(self) -> int:
+        """scale / shift / invstd of every frozen BatchNorm from its running statistics and current gamma / beta, in one launch.  Inside
+        the step (graph): the optimiser may change gamma / beta through raw pointers between steps."""
+        frozen = [c for c in self.convs if self.plan.convs[c.name].frozen]
+        if not frozen:
+            return 0
+        key = tuple((c.name,) + tuple(_data_ptr(t) for t in (c.bn.weight, c.bn.bias, c.bn.running_mean, c.bn.running_var)) for c in frozen)
+        if self._fold_items is None or key != self._fold_key:
+            items = [(c.bn.weight.data if c.bn.weight is not None else None, c.bn.bias.data if c.bn.bias is not None else None,
+                      c.bn.running_mean, c.bn.running_var, c.bn.eps, c.scale, c.shift, c.invstd) for c in frozen]
+            self._fold_items = ops.bn_fold_items(items).to(self.device)
+            self._fold_key = key
+            self._fold_n, self._fold_c = len(frozen), max(c.cout for c in frozen)
+        ops.bn_fold(self._fold_items, self._fold_n, self._fold_c)
+        return 1
+
+    def _conv_bn_frozen(self, c: _ConvT, x, out, relu: bool, residual=None) -> int:
+        """BatchNorm in eval() mode: normalise with the running statistics (folded scale / shift), buffers untouched."""
+        p = self.plan.convs[c.name]
+        if not (p.dgamma or p.dbeta):
+            # one launch: the conv epilogue applies scale / shift (+ shortcut) (+ ReLU); the backward masks with the stored output
+            ops.conv_bn_act(x, c.w_fwd, c.scale, c.shift, stride=c.stride, pad=c.pad, dil=c.dil, relu=relu, residual=residual, out=out)
+            c.frozen_mask = out if relu else None
+            return 1
+        # gamma / beta trained: their gradients need the raw conv output y
+        ops.conv_bn_act(x, c.w_fwd, c.one_out, c.zero_out, stride=c.stride, pad=c.pad, dil=c.dil, relu=False, out=c.y)
+        bits = c.relu_bits if relu and self.use_relu_bits else None
+        ops.bn_apply(c.y, c.scale, c.shift, relu=relu, residual=residual, out=out, relu_bits=bits)
+        c.frozen_mask = (bits if bits is not None else out) if relu else None
+        return 2
+
     def _conv_bn(self, c: _ConvT, x, out, relu: bool, residual=None, ws=None) -> int:
         """raw conv -> batch statistics (+ running stats) -> fused normalise (+ shortcut) (+ ReLU)."""
+        if self.plan.convs[c.name].frozen:
+            return self._conv_bn_frozen(c, x, out, relu, residual)
         bn = c.bn
         if self.use_bn_acc and self.fuse_conv_stats and ((c.k == 3 and c.cout >= 256) or (self.fuse_conv_stats_all and c is not self.stem)):
             # the conv epilogue gathers sum y / sum y^2 of the tile it stores: no statistics pass over the activation.  Only where the
@@ -248,14 +442,24 @@ class TrainEngine:
             torch.cuda.current_stream().wait_event(ev)
 
     def _bn_bwd(self, c: _ConvT, dout, relu: bool, dy, dmasked=None, ws=None) -> int:
-        """relu: the BN output went through a ReLU; its mask is c.relu_bits (written by the forward apply pass)."""
+        """relu: the BN output went through a ReLU; its mask is c.relu_bits (written by the forward apply pass).  dy None: the raw
+        conv output needs no gradient (only dgamma / dbeta / d' are wanted)."""
         bn = c.bn
+        p = self.plan.convs[c.name]
+        dg = self._g(bn.weight) if p.dgamma else None
+        db = self._g(bn.bias) if p.dbeta else None
+        if p.frozen:
+            sums = dg is not None or db is not None
+            ops.bn_frozen_bwd(dout, c.frozen_mask, c.scale, dy, dmasked=dmasked, y=c.y if sums else None, mean=bn.running_mean,
+                              invstd=c.invstd, acc=c.acc_b if sums else None, dgamma=dg, dbeta=db)
+            return 1
+        if dy is None:   # the batch-statistics backward kernels always write dy
+            dy = self._buf("dy_unused", c.y.shape)
         mask = None if not relu else (c.relu_bits if self.use_relu_bits else c.relu_out)
         if self.use_bn_acc:
-            ops.bn_bwd_acc(dout, mask, c.y, c.mean, c.invstd, bn.weight.data, c.acc_b, self._g(bn.weight), self._g(bn.bias), dy, dmasked=dmasked)
+            ops.bn_bwd_acc(dout, mask, c.y, c.mean, c.invstd, bn.weight.data, c.acc_b, dg, db, dy, dmasked=dmasked)
             return 2
-        ops.bn_train_bwd(dout, mask, c.y, c.mean, c.invstd, bn.weight.data, self._g(bn.weight), self._g(bn.bias), dy,
-                         self.bn_ws if ws is None else ws, dmasked=dmasked)
+        ops.bn_train_bwd(dout, mask, c.y, c.mean, c.invstd, bn.weight.data, dg, db, dy, self.bn_ws if ws is None else ws, dmasked=dmasked)
         return 3
 
     def _dy_buf(self, c: _ConvT, role: str = "dy") -> torch.Tensor:
@@ -313,19 +517,32 @@ class TrainEngine:
         check(lib().hk_stem_pack_weights(ptr(net.conv1.weight.data), ptr(self.stem_w), stream_ptr()), "hk_stem_pack_weights")
         self._on_wgrad_stream(self._pack_all)   # the block convs' weights are repacked while the stem, its BN and the maxpool run
         n += 2
-        if self.use_bn_acc:
+        if self.use_bn_acc and self.plan.train_bn_any:
             self.acc_fwd.zero_()                # the forward accumulators of every BatchNorm of this step
             n += 1
+        n += self._fold_frozen()                # eval()-mode BatchNorms: scale / shift from the running statistics
         # ---------------- forward (train mode) ----------------
         st = self.stem
-        ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
         bn = st.bn
-        if self.use_bn_acc:
+        sp = self.plan.convs[st.name]
+        if sp.frozen and not (sp.dgamma or sp.dbeta):
+            ops.stem_conv(self.x, self.stem_w, st.scale, st.shift, relu=True, out=self.a0)
+            st.frozen_mask = self.a0
+            n -= 3                              # conv + max-pool of the 5 counted below
+        elif sp.frozen:
+            ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
+            bits = st.relu_bits if self.use_relu_bits else None
+            ops.bn_apply(st.y, st.scale, st.shift, relu=True, out=self.a0, relu_bits=bits)
+            st.frozen_mask = bits if bits is not None else self.a0
+            n -= 2
+        elif self.use_bn_acc:
+            ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
             ops.bn_stats_acc(st.y, st.acc_f)
             ops.bn_apply_acc(st.y, st.acc_f, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, st.mean,
                              st.invstd, relu=True, out=self.a0, relu_bits=st.relu_bits if self.use_relu_bits else None)
             n -= 1
         else:
+            ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
             ops.bn_train_stats(st.y, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, st.mean, st.invstd,
                                st.scale, st.shift, self.bn_ws)
             ops.bn_apply(st.y, st.scale, st.shift, relu=True, out=self.a0, relu_bits=st.relu_bits if self.use_relu_bits else None)
@@ -355,11 +572,13 @@ class TrainEngine:
             n += self._conv_bn(c2, a1, out, relu=True, residual=shortcut)
             x = out
         feat = x
-        torch._foreach_add_(self._bn_counters, 1)
+        if self._bn_counters:                   # train-mode BatchNorms only
+            torch._foreach_add_(self._bn_counters, 1)
+            n += 1
         fc_w = net.fc.weight.data[:K].view(K, 512)
         fc_b = net.fc.bias.data[:K]
         ops.head_logits(feat, fc_w, fc_b, self.H, self.W, out=self.logits_up, logits_ws=self.logits_lr)
-        n += 3
+        n += 2
         return n
 
     def _enqueue_loss(self) -> int:
@@ -372,81 +591,116 @@ class TrainEngine:
                                    stream_ptr()), "hk_bce_fwd_bwd")
         return 2
 
+    def _acc_users(self, part: str) -> bool:
+        """Does a BatchNorm backward of this part fill an accumulator (train-mode BN, or frozen BN with dgamma / dbeta)?"""
+        e = self.convs.index(self.blocks[self.split_block][0])
+        convs = self.convs if part == "all" else self.convs[e:] if part == "late" else self.convs[:e]
+        for c in convs:
+            p = self.plan.convs[c.name]
+            if p.bwd and ((not p.frozen and self.use_bn_acc) or (p.frozen and (p.dgamma or p.dbeta))):
+                return True
+        return False
+
+    def has_early_backward(self) -> bool:
+        """The early part of the two-phase step (layers 2..1 + stem) has work: something there needs a gradient."""
+        return self.plan.lo < self.split_block
+
     def _enqueue_backward(self, part: str = "all") -> int:
         """From self.g_up = dL/d(upsampled logits) to every parameter gradient.  part "late" = head + layers 4..3 (the tail of the
         flat gradient buffer, 91 % of its bytes), part "early" = layers 2..1 + stem: the data-parallel step all-reduces the tail
-        while the early layers are still being differentiated."""
-        net, K, st = self.net, self.K, self.stem
+        while the early layers are still being differentiated.  Follows self.plan: nothing runs below the earliest point that still
+        needs a gradient, frozen parameters get no kernel."""
+        net, K, st, pl = self.net, self.K, self.stem, self.plan
         n = 0
         nb = len(self.blocks)
-        if self.use_bn_acc:   # the backward accumulators this part is going to fill
+        if self._acc_users(part):   # the backward accumulators this part is going to fill
             e = self.acc_early_bytes
             (self.acc_bwd if part == "all" else self.acc_bwd[e:] if part == "late" else self.acc_bwd[:e]).zero_()
             n += 1
         if part in ("all", "late"):
             feat = self.blocks[-1][5]
             fc_w = net.fc.weight.data[:K].view(K, 512)
-            d = self._buf("d0", feat.shape)
-            ops.head_bwd(self.g_up, feat, fc_w, d, self._g(net.fc.weight)[:K].view(K, 512), self._g(net.fc.bias)[:K],
-                         dlogits_ws=self.dlogits_lr, ws=self.head_ws)
-            n += 5
+            d = self._buf("d0", feat.shape) if pl.dfeat else None
+            dw = self._g(net.fc.weight)[:K].view(K, 512) if pl.fc_weight else None
+            db = self._g(net.fc.bias)[:K] if pl.fc_bias else None
+            if d is not None or dw is not None or db is not None:
+                ops.head_bwd(self.g_up, feat, fc_w, d, dw, db, dlogits_ws=self.dlogits_lr, ws=self.head_ws)
+                n += 5 - (d is None) - 2 * (dw is None) - 2 * (db is None)
             parity, hi = 1, nb
         else:
             d, parity, hi = self._bwd_state
-        lo = self.split_block if part == "late" else 0
+        lo = max(self.split_block if part == "late" else 0, pl.lo)
         for bi in range(hi - 1, lo - 1, -1):
             c1, c2, ds, a1, sc, out = self.blocks[bi]
+            p1, p2 = pl.convs[c1.name], pl.convs[c2.name]
+            pd = pl.convs[ds.name] if ds is not None else None
+            below = pl.grad_in[bi]
             x_in = self.blocks[bi - 1][5] if bi > 0 else self.p0
-            dy2 = self._dy_buf(c2)
-            dm = self._buf("dm", c2.y.shape)
-            n += self._bn_bwd(c2, d, True, dy2, dmasked=dm)            # d' = d*[out>0] also feeds the shortcut
+            dy2 = self._dy_buf(c2) if p2.dy else None
+            dm = self._buf("dm", c2.y.shape) if (pd.bwd if pd is not None else below) else None
+            if p2.bwd:
+                n += self._bn_bwd(c2, d, True, dy2, dmasked=dm)        # d' = d*[out>0] also feeds the shortcut
             dxd = None
-            if ds is not None:                                          # shortcut branch: needs only d'; joins at the residual add
-                dyd = self._dy_buf(ds, "dyd")
-                dxd = self._buf("dxd", x_in.shape)
+            if pd is not None and pd.bwd:                               # shortcut branch: needs only d'; joins at the residual add
+                dyd = self._dy_buf(ds, "dyd") if pd.dy else None
+                dxd = self._buf("dxd", x_in.shape) if pd.dgrad else None
                 aux = self._fork_aux()
                 with torch.cuda.stream(aux if aux is not None else torch.cuda.current_stream()):
                     n += self._bn_bwd(ds, dm, False, dyd, ws=self.bn_ws_aux)
-                    n += self._wgrad(ds, x_in, dyd, ws=self.wgrad_ws_aux)
-                    n += self._dgrad(ds, dyd, dxd, scratch="up_aux")
-            n += self._wgrad(c2, a1, dy2)
-            da1 = self._buf("da1", a1.shape)
-            n += self._dgrad(c2, dy2, da1)
-            dy1 = self._dy_buf(c1)
-            n += self._bn_bwd(c1, da1, True, dy1)
-            n += self._wgrad(c1, x_in, dy1)
-            dx = self._buf(f"d{parity}", x_in.shape)
-            if ds is not None:
+                    if pd.wgrad:
+                        n += self._wgrad(ds, x_in, dyd, ws=self.wgrad_ws_aux)
+                    if pd.dgrad:
+                        n += self._dgrad(ds, dyd, dxd, scratch="up_aux")
+            if p2.wgrad:
+                n += self._wgrad(c2, a1, dy2)
+            da1 = None
+            if p2.dgrad:
+                da1 = self._buf("da1", a1.shape)
+                n += self._dgrad(c2, dy2, da1)
+            dy1 = self._dy_buf(c1) if p1.dy else None
+            if p1.bwd:
+                n += self._bn_bwd(c1, da1, True, dy1)
+            if p1.wgrad:
+                n += self._wgrad(c1, x_in, dy1)
+            if pd is not None and pd.bwd:
                 self._join_aux()
-                n += self._dgrad(c1, dy1, dx, residual=dxd)
-            else:
-                n += self._dgrad(c1, dy1, dx, residual=dm)
+            if not below:
+                d = None
+                break
+            dx = self._buf(f"d{parity}", x_in.shape)
+            n += self._dgrad(c1, dy1, dx, residual=dxd if ds is not None else dm)
             d, parity = dx, parity ^ 1
         if part == "late":
-            # the hand-off gradient gets its own buffer: the early graph is executed more than once per capture (warm-up, capture,
-            # replay) and its ping-pong scratch would otherwise overwrite its own input
-            dh = self._buf("dh", d.shape)
-            dh.copy_(d)
-            self._bwd_state = (dh, parity, lo)
+            if self.has_early_backward():
+                # the hand-off gradient gets its own buffer: the early graph is executed more than once per capture (warm-up, capture,
+                # replay) and its ping-pong scratch would otherwise overwrite its own input
+                dh = self._buf("dh", d.shape)
+                dh.copy_(d)
+                self._bwd_state = (dh, parity, lo)
+                n += 1
             self._join_wgrad_stream()
-            return n + 1
-        da0 = self._buf("da0", self.a0.shape)
-        if self.maxpool_idx:
-            ops.maxpool3x3s2_bwd_idx(d, self.pool_idx, self.a0.shape[1], self.a0.shape[2], dx=da0)
-        else:
-            ops.maxpool3x3s2_bwd(d, self.a0, dx=da0, idx_ws=self.pool_idx)
-            n += 1
-        dy0 = self._dy_buf(st)
-        n += 1 + self._bn_bwd(st, da0, True, dy0)
-        self._on_wgrad_stream(lambda: ops.stem_wgrad(self.x, dy0, self._g(net.conv1.weight), ws=self.wgrad_ws))
+            return n
+        if pl.stem:
+            da0 = self._buf("da0", self.a0.shape)
+            if self.maxpool_idx:
+                ops.maxpool3x3s2_bwd_idx(d, self.pool_idx, self.a0.shape[1], self.a0.shape[2], dx=da0)
+            else:
+                ops.maxpool3x3s2_bwd(d, self.a0, dx=da0, idx_ws=self.pool_idx)
+                n += 1
+            sp = pl.convs[st.name]
+            dy0 = self._dy_buf(st) if sp.dy else None
+            n += 1 + self._bn_bwd(st, da0, True, dy0)
+            if sp.wgrad:
+                self._on_wgrad_stream(lambda: ops.stem_wgrad(self.x, dy0, self._g(net.conv1.weight), ws=self.wgrad_ws))
+                n += 2
         self._join_wgrad_stream()
-        n += 2
         return n
 
     def _key(self):
         # sigma is passed by value to hk_bce_fwd_bwd, i.e. baked into a captured graph: a new sigma needs a new capture
-        return (tuple(p.data_ptr() for p in self.params), None if self.target is None else (self.target.data_ptr(), self.target.dtype),
-                self.sigma)
+        # the torch flags (bn.training, requires_grad) choose the kernels: a toggled flag needs a new capture
+        return (tuple(p.data_ptr() for p in self.all_params), None if self.target is None else (self.target.data_ptr(), self.target.dtype),
+                self.sigma, self._flags)
 
     def forward_backward(self, img: torch.Tensor, uv: Optional[torch.Tensor] = None, target: Optional[torch.Tensor] = None) -> torch.Tensor:
         """img (B,3,H,W) fp32 CUDA; labels uv (B,K,2) = (x,y) [Gaussian targets generated on the fly, dataset.py:36-44] or a
@@ -456,6 +710,7 @@ class TrainEngine:
             raise ValueError("pass exactly one of uv / target")
         if not img.is_cuda or tuple(img.shape) != (self.B, 3, self.H, self.W):
             raise ValueError(f"expected a CUDA image batch of shape {(self.B, 3, self.H, self.W)}, got {tuple(img.shape)} on {img.device}")
+        self.sync_flags()
         self.model.mark_weights_changed()   # BatchNorm running stats are advanced through raw pointers (tensor versions do not move)
         with torch.no_grad():
             self.x.copy_(img)
@@ -522,6 +777,7 @@ class TrainEngine:
             self.heat = torch.empty_like(self.logits_up)
             self.g_heat = torch.empty_like(self.logits_up)
         n = self.logits_up.numel()
+        self.sync_flags()
 
         def fn():
             k = self._enqueue_forward()
@@ -550,6 +806,7 @@ class TrainEngine:
         """Phase 1 of the data-parallel step: forward + loss + backward of head, layer4, layer3 (gradients flat_grad[late_offset:])."""
         if not img.is_cuda or tuple(img.shape) != (self.B, 3, self.H, self.W):
             raise ValueError(f"expected a CUDA image batch of shape {(self.B, 3, self.H, self.W)}")
+        self.sync_flags()
 
         def fn():
             return self._enqueue_forward() + self._enqueue_loss() + self._enqueue_backward("late")
@@ -562,7 +819,11 @@ class TrainEngine:
         return self.loss
 
     def backward_early(self) -> None:
-        """Phase 2: backward of layer2, layer1 and the stem (gradients flat_grad[:late_offset])."""
+        """Phase 2: backward of layer2, layer1 and the stem (gradients flat_grad[:late_offset]).  Nothing to do (no launch) when
+        nothing there needs a gradient."""
+        if not self.has_early_backward():
+            self.__dict__.setdefault("_split_launches", {})["bwd_early"] = 0
+            return
         with torch.no_grad():
             self._run("bwd_early", lambda: self._enqueue_backward("early"))
 

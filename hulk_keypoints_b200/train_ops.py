@@ -46,14 +46,14 @@ class _EngineStep(torch.autograd.Function):
     @staticmethod
     def forward(ctx, engine, img, target, uv, *params):
         loss = engine.forward_backward(img, uv=uv, target=target)
-        ctx.engine = engine
+        ctx.engine, ctx.params = engine, list(engine.params)
         return loss.clone()
 
     @staticmethod
     def backward(ctx, grad_out):
         eng = ctx.engine
         g = grad_out.to(torch.float32)
-        return (None, None, None, None) + tuple(eng.grad(p) * g for p in eng.params)
+        return (None, None, None, None) + tuple(eng.grad(p) * g for p in ctx.params)
 
 
 class _EngineForward(torch.autograd.Function):
@@ -63,25 +63,27 @@ class _EngineForward(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, engine, img, *params):
-        ctx.engine = engine
+        ctx.engine, ctx.params = engine, list(engine.params)
         return engine.forward_heatmaps(img).clone()
 
     @staticmethod
     def backward(ctx, grad_heat):
         eng = ctx.engine
         eng.backward_from_heatmap_grad(grad_heat.to(torch.float32).contiguous())
-        return (None, None) + tuple(eng.grad(p).clone() for p in eng.params)
+        return (None, None) + tuple(eng.grad(p).clone() for p in ctx.params)
 
 
 def engine_forward(model, img: torch.Tensor) -> torch.Tensor:
     """Differentiable train-mode heatmaps (B,K,H,W) computed by the TrainEngine (see _EngineForward)."""
     eng = model.train_engine(img.shape[0], img.shape[2], img.shape[3])
+    eng.sync_flags()   # only trainable parameters are inputs of the autograd node: frozen ones keep .grad None
     return _EngineForward.apply(eng, img.float().contiguous(), *eng.params)
 
 
 def engine_loss(model, img: torch.Tensor, target: Optional[torch.Tensor] = None, uv: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Differentiable fp64 loss of one batch computed by the B200 TrainEngine (bf16 tensor-core forward/backward)."""
     eng = model.train_engine(img.shape[0], img.shape[2], img.shape[3])
+    eng.sync_flags()
     return _EngineStep.apply(eng, img, target, uv, *eng.params)
 
 
@@ -111,6 +113,7 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
     if backend == "hk":
         eng = model.train_engine(img.shape[0], img.shape[2], img.shape[3])
         eng.sigma = float(sigma)
+        eng.sync_flags()   # bn.training / requires_grad of this step: the flat gradient buffer holds the trainable parameters only
         if fused:
             if optimizer.flat_grad.data_ptr() != eng.flat_grad.data_ptr():
                 optimizer.adopt_grad_buffer(eng.flat_grad)
@@ -153,3 +156,44 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
         allreduce(model.parameters())
     optimizer.step()
     return loss.detach()
+
+
+FREEZE_PRESETS = ("none", "bn", "torchvision", "head", "mixed")
+
+
+def freeze_preset(model, preset: str) -> None:
+    """Put `model` in train() mode and set the standard fine-tuning flags (torch's own switches, which the training engine honours):
+      none        every BatchNorm in train mode, every parameter trained (the default configuration)
+      bn          every BatchNorm in eval() mode (running statistics, buffers untouched); gamma / beta and all weights trained
+      torchvision every BatchNorm in eval() mode with gamma / beta frozen, and conv1 + layer1 frozen (torchvision's detection and
+                  keypoint models at trainable_backbone_layers=3)
+      head        only the scoring conv `fc` trained; every BatchNorm in eval() mode
+      mixed       BatchNorms of the stem and layers 1-2 in eval() mode, layers 3-4 in train mode; every parameter trained
+    Build the optimiser after freezing, as in torch: FusedAdam lays out the trainable parameters only."""
+    if preset not in FREEZE_PRESETS:
+        raise ValueError(f"freeze preset must be one of {FREEZE_PRESETS}")
+    net = model.resnet.resnet34_8s
+    model.train()
+    for p in model.parameters():
+        p.requires_grad_(True)
+    bns = [m for m in net.modules() if isinstance(m, torch.nn.BatchNorm2d)]
+    if preset in ("bn", "torchvision", "head"):
+        for bn in bns:
+            bn.eval()
+    if preset == "torchvision":
+        for bn in bns:
+            for p in bn.parameters():
+                p.requires_grad_(False)
+        for m in (net.conv1, net.bn1, net.layer1):
+            for p in m.parameters():
+                p.requires_grad_(False)
+    elif preset == "head":
+        for p in model.parameters():
+            p.requires_grad_(False)
+        for p in net.fc.parameters():
+            p.requires_grad_(True)
+    elif preset == "mixed":
+        for m in (net.bn1, net.layer1, net.layer2):
+            for bn in m.modules():
+                if isinstance(bn, torch.nn.BatchNorm2d):
+                    bn.eval()

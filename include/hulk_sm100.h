@@ -261,6 +261,31 @@ HK_API int hk_bn_bwd_acc(const void* dout, const void* out_mask_or_null, int mas
                          const float* invstd, const float* gamma, long long P, int C, void* acc, float* dgamma, float* dbeta,
                          int accumulate, void* dy, void* dmasked_or_null, void* stream);
 
+/* Frozen BatchNorm: an nn.BatchNorm2d in eval() mode inside a train()-mode model normalises with its running statistics and leaves
+ * its buffers alone (torch's semantics).
+ *   hk_bn_fold       : for every item, scale = gamma*invstd_r, shift = beta - mean_r*scale, invstd = 1/sqrt(running_var + eps)
+ *                      (invstd nullable; gamma/beta NULL = 1/0), all items in one launch.  items_dev: device array of HkBnFoldItem;
+ *                      max_c = the largest C.  The forward is then hk_bn_apply_fwd (or a conv epilogue) with this scale/shift.
+ *   hk_bn_frozen_bwd : d' = dout*[out>0] (mask as for hk_bn_train_bwd, NULL = no ReLU), dy = scale*d' (nullable), d' into
+ *                      dmasked_or_null; when dgamma or dbeta is given: acc (zeroed, hk_bn_acc_bytes(C)) += (sum d', sum d'*y), and
+ *                      dbeta = sum d', dgamma = invstd*(sum d'*y - mean*sum d') from the exact totals (accumulate != 0 adds).  One pass,
+ *                      one launch; y, mean (running mean) and invstd are only read for the sums. */
+typedef struct HkBnFoldItem {
+  const float* gamma;
+  const float* beta;
+  const float* mean;   /* running_mean */
+  const float* var;    /* running_var */
+  float* scale;
+  float* shift;
+  float* invstd;       /* or NULL */
+  float eps;
+  int32_t C;
+} HkBnFoldItem;
+HK_API int hk_bn_fold(const HkBnFoldItem* items_dev, int n_items, int max_c, void* stream);
+HK_API int hk_bn_frozen_bwd(const void* dout, const void* out_mask_or_null, int mask_is_bits, const void* y_or_null, const float* scale,
+                            const float* mean, const float* invstd, long long P, int C, void* acc_or_null, float* dgamma, float* dbeta,
+                            int accumulate, void* dy_or_null, void* dmasked_or_null, void* stream);
+
 /* Train-mode forward of one conv + the statistics pass of its BatchNorm in ONE launch (src/resnet.py:56-57,60-61 under model.train()):
  * y = conv(x) (raw output: pass scale = 1, bias = 0; desc->relu must be 0) and acc += per-channel (sum y, sum y^2) of the bf16 values
  * stored, gathered in the epilogue of the tcgen05 kernel from the staged output tile -- the activation is not read again for its
@@ -319,7 +344,8 @@ HK_API int hk_maxpool3x3s2_bwd_idx(const void* dout, const void* idx, void* dx, 
 
 /* Head in training: K-row scoring conv + bilinear upsample WITHOUT the sigmoid (hk_bce_fwd_bwd takes logits), ATen's exact
  * operation order; and its backward: upsample-backward of g_up (B,K,H,W) to dlogits_ws (B,K,h,w), then
- * dfeat (B,h,w,C) bf16, dw_fc (K,C) fp32, db_fc (K) fp32.  Only the K live rows of fc get a gradient, as in the reference. */
+ * dfeat (B,h,w,C) bf16, dw_fc (K,C) fp32, db_fc (K) fp32.  Only the K live rows of fc get a gradient, as in the reference.
+ * dfeat, dw_fc and db_fc may each be NULL (frozen backbone / frozen fc): their kernels are skipped. */
 HK_API int hk_head_logits_fwd(const void* feat, int feat_dtype, const float* w_fc, const float* b_fc, float* logits_ws,
                               float* logits_up, int B, int K, int C, int h, int w, int H, int W, void* stream);
 HK_API size_t hk_head_bwd_workspace_bytes(int B, int K, int C, int h, int w);

@@ -25,6 +25,7 @@ EXPORTS = (
     "hk_maxpool3x3s2_fwd", "hk_head_fwd", "hk_argmax_workspace_bytes", "hk_argmax_decode",
     "hk_gauss_targets", "hk_bce_workspace_bytes", "hk_bce_fwd_bwd",
     "hk_stem_packed_weight_bytes", "hk_stem_pack_weights", "hk_stem_fwd", "hk_stem_fwd_u8", "hk_adam_step",
+    "hk_adam_step_segments",
     # training (SURVEY.md §8 f1)
     "hk_stem_conv_fwd", "hk_bn_workspace_bytes", "hk_bn_train_stats", "hk_bn_apply_fwd", "hk_bn_train_bwd",
     "hk_pack_conv_weights_dgrad", "hk_zero_insert2x", "hk_conv_wgrad_workspace_bytes", "hk_conv_wgrad",
@@ -42,6 +43,15 @@ class HkConvDesc(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "batch", "in_h", "in_w", "in_c", "out_h", "out_w", "out_c", "kh", "kw", "stride", "pad", "dil",
         "relu", "in_dtype", "out_dtype", "in_is_nchw", "algo")]
+
+
+# HkAdamSegment of include/hulk_sm100.h: one row of hk_adam_step_segments' table
+ADAM_MAX_SEGMENTS = 256
+
+
+class HkAdamSegment(C.Structure):
+    _fields_ = [("begin4", C.c_longlong), ("end4", C.c_longlong)] + [(n, C.c_float) for n in (
+        "lr_over_bc1", "inv_sqrt_bc2", "beta1", "beta2", "eps", "weight_decay", "decay")] + [("decoupled", C.c_int)]
 
 
 _lock = threading.Lock()
@@ -96,6 +106,8 @@ def _declare(lib):
     lib.hk_stem_pool_fwd_u8.argtypes = [vp, vp, vp, vp, vp, i, i, i, vp]
     lib.hk_adam_step.restype = i
     lib.hk_adam_step.argtypes = [vp, vp, vp, vp, C.c_longlong, f, f, f, f, f, i, vp]
+    lib.hk_adam_step_segments.restype = i
+    lib.hk_adam_step_segments.argtypes = [vp, vp, vp, vp, C.c_longlong, C.POINTER(HkAdamSegment), i, vp]
     lib.hk_stem_fwd_u8.restype = i
     lib.hk_stem_fwd_u8.argtypes = [vp, vp, vp, vp, vp, i, i, i, vp]
     ll = C.c_longlong

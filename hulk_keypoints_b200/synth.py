@@ -85,7 +85,8 @@ def fit_synthetic(model, steps: int, B: int, H: int, W: int, lr: float = 1e-3, w
     losses = []
     for step in range(steps):
         if step == int(decay_after * steps):
-            opt.lr = lr / 10
+            for g in opt.param_groups:
+                g["lr"] = lr / 10
         img, uv = disc_batch(gen, B, H, W, K)
         losses.append(float(train_ops.train_step(model, opt, img.to(dev), uv.to(dev), sigma=sigma).item()))
     return losses

@@ -8,7 +8,7 @@ which has no SyncBN) and updates running_mean / running_var / num_batches_tracke
 
 Per conv the forward is   y = conv(x) [raw, bf16]  ->  batch stats  ->  out = relu(gamma*xhat + beta [+ shortcut])
 and the backward          d' = dout*[out>0]  ->  (dgamma, dbeta, dy)  ->  dW = wgrad(x, dy),  dx = conv(dy, W flipped).
-All 110 parameter gradients land in ONE flat fp32 buffer laid out like FusedAdam's (one all-reduce, one update kernel);
+All 110 parameter gradients land in ONE flat fp32 buffer in the layout FusedAdam adopts (one all-reduce, one update kernel);
 the 996 dead rows of the 1000-row scoring conv keep a zero gradient, as in the reference.
 
 Data layout in HBM (per engine, batch B of H x W): input (B,3,H,W) f32; per conv a raw output and an activation,
@@ -289,7 +289,7 @@ class TrainEngine:
     # ------------------------------------------------------------------ torch flags
     def sync_flags(self) -> None:
         """Read bn.training and p.requires_grad (torch's fine-tuning switches) and, when they changed since the last step, rebuild what
-        depends on them: the flat gradient buffer (trainable parameters only, FusedAdam's layout), the backward plan and the list of
+        depends on them: the flat gradient buffer (trainable parameters only, the layout FusedAdam adopts), the backward plan and the list of
         BatchNorms whose num_batches_tracked advances.  The flags are part of every graph key, so no stale graph is replayed."""
         params = self.all_params
         flags = (tuple(c.bn.training for c in self.convs), tuple(p.requires_grad for p in params))
@@ -306,7 +306,7 @@ class TrainEngine:
         self._flags = flags
 
     def _build_grad_buffer(self, trainable: List[torch.nn.Parameter]) -> None:
-        """Flat gradient buffer of the trainable parameters, FusedAdam's layout (each tensor starts on a 16-byte boundary)."""
+        """Flat gradient buffer of the trainable parameters in model order, the layout FusedAdam adopts (each tensor 16-byte aligned)."""
         self.params = trainable
         offs, total = [], 0
         for p in self.params:

@@ -116,7 +116,8 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
         eng.sync_flags()   # bn.training / requires_grad of this step: the flat gradient buffer holds the trainable parameters only
         if fused:
             if optimizer.flat_grad.data_ptr() != eng.flat_grad.data_ptr():
-                optimizer.adopt_grad_buffer(eng.flat_grad)
+                # the engine's order is the flat layout (the two-phase split relies on it): FusedAdam reorders to it once
+                optimizer.adopt_grad_buffer(eng.flat_grad, eng.params)
         import torch.distributed as dist
         if not exchange:   # measurement only (bench.py: the step with its gradient exchange switched off = the compute-only time)
             loss = eng.forward_backward(img, uv=uv)
@@ -169,7 +170,8 @@ def freeze_preset(model, preset: str) -> None:
                   keypoint models at trainable_backbone_layers=3)
       head        only the scoring conv `fc` trained; every BatchNorm in eval() mode
       mixed       BatchNorms of the stem and layers 1-2 in eval() mode, layers 3-4 in train mode; every parameter trained
-    Build the optimiser after freezing, as in torch: FusedAdam lays out the trainable parameters only."""
+    Build the optimiser after freezing, as in torch: FusedAdam lays out the trainable parameters only (when unfreezing later, hand the
+    newly trainable parameters to `optimizer.add_param_group`)."""
     if preset not in FREEZE_PRESETS:
         raise ValueError(f"freeze preset must be one of {FREEZE_PRESETS}")
     net = model.resnet.resnet34_8s

@@ -211,6 +211,24 @@ HK_API int hk_bce_fwd_bwd(const float* pred, int pred_is_logits, const void* tar
 HK_API int hk_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, long long n,
                         float lr, float beta1, float beta2, float eps, float weight_decay, int step, void* stream);
 
+/* One Adam step over flat fp32 buffers whose runs differ in hyperparameters or step count (torch.optim.Adam / AdamW parameter
+ * groups, learning-rate schedules): ONE launch for any number of segments.  The segments cover [0, ceil(n/4)) in float4 units,
+ * non-empty, sorted and contiguous; the n % 4 tail belongs to the last one.  Per segment, computed in double on the host as
+ * hk_adam_step does: lr_over_bc1 = lr / (1 - beta1^t), inv_sqrt_bc2 = 1 / sqrt(1 - beta2^t).  decoupled == 0: coupled L2
+ * (g += weight_decay * p; bit-identical to hk_adam_step); decoupled != 0: p *= decay (= 1 - lr * weight_decay, rounded to fp32)
+ * before the update on the unmodified gradient.  The table is read during the call (it travels as a launch parameter), so the
+ * call is capturable and `segments` may be reused right after it returns.  At most HK_ADAM_MAX_SEGMENTS segments. */
+#define HK_ADAM_MAX_SEGMENTS 256
+typedef struct HkAdamSegment {
+  long long begin4, end4;
+  float lr_over_bc1, inv_sqrt_bc2;
+  float beta1, beta2, eps, weight_decay;
+  float decay;
+  int decoupled;
+} HkAdamSegment;
+HK_API int hk_adam_step_segments(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, long long n,
+                                 const HkAdamSegment* segments, int num_segments, void* stream);
+
 /* ---- training: backbone forward in train() mode and its backward (SURVEY.md §8 f1) ----
  * Replaces what torch autograd does for train.py:33-36 between the input batch and the parameter gradients.  Activations are
  * NHWC bf16 (P = B*H*W rows of C channels), statistics / parameters / parameter gradients fp32.  Every reduction is a fixed-order

@@ -270,19 +270,16 @@ static WgradPlan wgrad_plan(const HkConvDesc& d) {
   p.n_tiles = d.in_c / p.block_n;
   p.taps = d.kh * d.kw;
   // two taps per unit (the shift on dY): the 64-output-channel convs at stride 1 with equal input / output grids, i.e. layer 1
-  static const bool pairs_off = [] { const char* e = getenv("HK_WGRAD_TAP_PAIRS"); return e && e[0] == '0'; }();
-  p.tap_pairs = (!pairs_off && d.out_c == 64 && d.stride == 1 && d.in_h == d.out_h && d.in_w == d.out_w && p.taps > 1) ? 1 : 0;
+  p.tap_pairs = (d.out_c == 64 && d.stride == 1 && d.in_h == d.out_h && d.in_w == d.out_w && p.taps > 1) ? 1 : 0;
   p.tap_units = p.tap_pairs ? (p.taps + 1) / 2 : p.taps;
   p.tiles_x = ceil_div(d.out_w, WG_BOX_W);
   p.tiles_per_img = p.tiles_x * ceil_div(d.out_h, WG_BOX_H);
   p.num_boxes = p.tiles_per_img * d.batch;
   const int base = p.tap_units * p.m_tiles * p.n_tiles;
-  // K splits: enough units for `rounds` units per persistent CTA.  One round (default since round 2): half the fp32 partials to write
-  // and to reduce of the two-round plan of round 1, whose only merit -- the second unit's mainloop hiding the first one's epilogue -- is
-  // matched by having half as many epilogues; batch 4: 4.07 -> 3.89 ms per step, batch 32: 22.7 -> 22.5 ms (A/B on one box).
-  // HK_WGRAD_ROUNDS (read once) restores 2 for A/B runs.
-  static const int rounds = [] { const char* e = getenv("HK_WGRAD_ROUNDS"); const int r = e ? atoi(e) : 0; return r >= 1 && r <= 4 ? r : 1; }();
-  int ks = (rounds * sm_count()) / base;
+  // K splits: enough units for one unit per persistent CTA.  Half the fp32 partials to write and to reduce of the two-round plan of
+  // round 1, whose only merit -- the second unit's mainloop hiding the first one's epilogue -- is matched by having half as many
+  // epilogues; batch 4: 4.07 -> 3.89 ms per step, batch 32: 22.7 -> 22.5 ms (A/B on one box).
+  int ks = sm_count() / base;
   if (ks < 1) ks = 1;
   const int max_ks = p.num_boxes / 4 > 0 ? p.num_boxes / 4 : 1;  // at least 4 pipeline stages of work per unit
   if (ks > max_ks) ks = max_ks;

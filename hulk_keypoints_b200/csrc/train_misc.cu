@@ -433,9 +433,8 @@ int hk_head_bwd(const float* g_up, const void* feat, const float* w_fc, float* d
   const float rx = W > 1 ? (float)(w - 1) / (float)(W - 1) : 0.f;
   const int n = B * K * h * w;
   int rc;
-  static const bool old_upsample_bwd = [] { const char* e = getenv("HK_UPSAMPLE_BWD_ROWS"); return e && e[0] == '0'; }();   // A/B switch
   const size_t vbytes = (size_t)((W + 3) / 4 * 4) * sizeof(float);
-  if (!old_upsample_bwd && h <= 65535 && B * K <= 65535 && vbytes <= 48 * 1024 && (reinterpret_cast<uintptr_t>(g_up) & 15) == 0) {
+  if (h <= 65535 && B * K <= 65535 && vbytes <= 48 * 1024 && (reinterpret_cast<uintptr_t>(g_up) & 15) == 0) {
     upsample_bwd_rows_kernel<<<dim3(h, B * K), 256, vbytes, s>>>(g_up, dlogits_ws, h, w, H, W, ry, rx);
     rc = check_launch("upsample_bwd_rows_kernel");
   } else {

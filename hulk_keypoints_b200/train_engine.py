@@ -8,12 +8,15 @@ which has no SyncBN) and updates running_mean / running_var / num_batches_tracke
 
 Per conv the forward is   y = conv(x) [raw, bf16]  ->  batch stats  ->  out = relu(gamma*xhat + beta [+ shortcut])
 and the backward          d' = dout*[out>0]  ->  (dgamma, dbeta, dy)  ->  dW = wgrad(x, dy),  dx = conv(dy, W flipped).
+Batch statistics and their backward sums go through exact fixed-point accumulators, the ReLU mask through 1 bit per element, and the
+max-pool forward records the winning taps its backward routes through.  Weight gradients (and the per-step weight repack) run on a
+second stream, the downsample branches on a third, all inside the same graph.
 All 110 parameter gradients land in ONE flat fp32 buffer in the layout FusedAdam adopts (one all-reduce, one update kernel);
 the 996 dead rows of the 1000-row scoring conv keep a zero gradient, as in the reference.
 
 Data layout in HBM (per engine, batch B of H x W): input (B,3,H,W) f32; per conv a raw output and an activation,
 (B,h,w,C) bf16 NHWC; (B,K,H,W) f32 upsampled logits and their gradient; scratch gradients sized by stage.
-The whole step is captured in one CUDA graph (~560 launches) and replayed.
+The whole step is captured in one CUDA graph (287 launches when every BatchNorm and parameter trains) and replayed.
 
 Fine-tuning: BatchNorms in eval() mode (running statistics, buffers untouched) and parameters with requires_grad=False follow torch's
 semantics; `backward_plan` decides from those flags what the backward computes and where it stops (DESIGN §3.5).
@@ -27,7 +30,7 @@ from typing import Dict, List, NamedTuple, Optional, Tuple
 import torch
 
 from . import ops
-from ._lib import HK_BF16, check, lib, ptr, require_device, stream_ptr
+from ._lib import check, lib, ptr, require_device, stream_ptr
 
 
 # ---------------------------------------------------------------------------------------------------------------- backward plan
@@ -111,8 +114,7 @@ def backward_plan(net) -> BackwardPlan:
 
 
 def step_launches(net, plan: BackwardPlan) -> int:
-    """Kernel launches of one TrainEngine.forward_backward step under `plan`, in the engine's default configuration (accumulator
-    BatchNorm path, epilogue statistics for the 3x3 convs with >= 256 channels, max-pool indices): what `TrainEngine.launches` reports."""
+    """Kernel launches of one TrainEngine.forward_backward step under `plan`: what `TrainEngine.launches` reports."""
     blocks = list(net.blocks())
 
     def fwd(name, conv) -> int:
@@ -178,6 +180,7 @@ class _ConvT:
         self.y = torch.empty((B, self.Ho, self.Wo, self.cout), device=dev, dtype=bf)   # raw conv output (saved for BN backward)
         self.mean, self.invstd, self.scale, self.shift = (torch.empty(self.cout, device=dev) for _ in range(4))
         self.relu_bits = torch.empty(self.y.numel() // 8, device=dev, dtype=torch.uint8)  # ReLU mask of the BN output, 1 bit / element
+        self.dy: Optional[torch.Tensor] = None   # gradient of y, allocated by the first backward that needs it
 
 
 class TrainEngine:
@@ -208,6 +211,7 @@ class TrainEngine:
         self.stem = _ConvT("stem", net.conv1, net.bn1, B, H, W, dev)
         self.a0 = torch.empty((B, h2, w2, 64), device=dev, dtype=bf)
         self.p0 = torch.empty((B, h4, w4, 64), device=dev, dtype=bf)
+        # the max-pool forward records the winning taps: one pass over the stem map instead of a forward pass plus an arg-max pass
         self.pool_idx = torch.empty(B * h4 * w4 * 64, device=dev, dtype=torch.uint8)
         self.blocks = []
         h, w = h4, w4
@@ -224,16 +228,7 @@ class TrainEngine:
         self.convs: List[_ConvT] = [self.stem] + [c for b in self.blocks for c in (b[0], b[1], b[2]) if c is not None]
         # BatchNorm reductions through exact fixed-point accumulators (hk_bn_stats_acc / hk_bn_bwd_acc): no finalize launches, 72 fewer
         # launches per step.  One flat buffer per direction, sliced per conv in self.convs order (stem, then the blocks in order), so the
-        # early part of the two-phase backward (stem + blocks < split_block) is a prefix.  HK_BN_ACC=0: the three-launch path.
-        self.use_bn_acc = os.environ.get("HK_BN_ACC", "1") != "0"
-        # ... and the forward statistics gathered in the conv epilogues (hk_conv_bn_stats_fwd): 36 launches and one read of every raw conv
-        # output fewer.  HK_CONV_STATS=0: stand-alone hk_bn_stats_acc.
-        self.fuse_conv_stats = os.environ.get("HK_CONV_STATS", "1") != "0"
-        # HK_CONV_STATS=all: every conv with a specialised tcgen05 kernel gathers its statistics in the epilogue (A/B switch; at small batch
-        # the stand-alone reduction is a latency-bound launch, at large batch the epilogue-bound 64/128-channel layers lose more than it costs)
-        self.fuse_conv_stats_all = os.environ.get("HK_CONV_STATS", "1") == "all"
-        # max-pool forward records the winning taps (one pass over the stem map instead of two); HK_MAXPOOL_IDX=0: argmax pass in the backward
-        self.maxpool_idx = os.environ.get("HK_MAXPOOL_IDX", "1") != "0"
+        # early part of the two-phase backward (stem + blocks < split_block) is a prefix.
         offs_acc, tot = [], 0
         for c in self.convs:
             offs_acc.append(tot)
@@ -251,7 +246,6 @@ class TrainEngine:
         self.loss = torch.zeros((), device=dev, dtype=torch.float64)
         n = B * K * H * W
         self.bce_ws = torch.empty(int(lib().hk_bce_workspace_bytes(n)), device=dev, dtype=torch.uint8)
-        self.bn_ws = ops.bn_workspace(512, dev)
         wg = max(ops.conv_wgrad_workspace_bytes(B, c.H, c.W, c.cin, c.cout, c.k, c.stride, c.pad, c.dil) for c in self.convs[1:])
         self.wgrad_ws = torch.empty(max(wg, int(lib().hk_stem_wgrad_workspace_bytes())), device=dev, dtype=torch.uint8)
         self.head_ws = torch.empty(int(lib().hk_head_bwd_workspace_bytes(B, K, 512, h, w)), device=dev, dtype=torch.uint8)
@@ -264,27 +258,18 @@ class TrainEngine:
         self._fold_items: Optional[torch.Tensor] = None
         self._flags = None
         self.sync_flags()          # flat gradient buffer, backward plan, BatchNorm counters
-        self.graph: Optional[torch.cuda.CUDAGraph] = None
-        self._graph_key = None
         self.use_cuda_graph = os.environ.get("HK_TRAIN_NO_GRAPH") is None   # eager launches for ncu launch lists
-        # ReLU masks of the backward pass as 1 bit / element written by the forward apply pass (HK_BN_BITS=0: re-read the bf16 outputs)
-        self.use_relu_bits = os.environ.get("HK_BN_BITS", "1") != "0"
+        self._graphs: Dict[str, Tuple[torch.cuda.CUDAGraph, Tuple, int]] = {}   # by entry point: (graph, _key() at capture, launches)
         # Weight gradients are leaves of the backward chain (bn_bwd -> dgrad -> bn_bwd ...): they run on a second stream inside the same
         # graph, concurrently with the data-gradient chain (each conv then keeps its own dy buffer).  Measured on one box: per-GPU batch 4
-        # 5.74 -> 5.37 ms per step, batch 32 25.40 -> 24.53 ms.  HK_WGRAD_STREAM=0 keeps everything on one stream.
-        self.wgrad_stream = torch.cuda.Stream(device=dev) if os.environ.get("HK_WGRAD_STREAM", "1") != "0" else None
+        # 5.74 -> 5.37 ms per step, batch 32 25.40 -> 24.53 ms.  All of them share wgrad_ws: the stream runs them one after another.
+        self.wgrad_stream = torch.cuda.Stream(device=dev)
+        self._wgrad_pending = False
         # The 1x1 downsample branch of the three stride/channel-changing blocks (conv + BN forward; BN backward + dgrad) is independent
-        # of the block's main branch until the residual add: it runs on a third stream with its own BN workspace (HK_AUX_STREAM=0: off).
-        self.aux_stream = torch.cuda.Stream(device=dev) if os.environ.get("HK_AUX_STREAM", "1") != "0" else None
-        self.bn_ws_aux = ops.bn_workspace(512, dev) if self.aux_stream is not None else None
-        # HK_WGRAD_STREAM=0 with the aux stream on: the downsample conv's weight gradient then runs on the aux stream concurrently with
-        # conv2's on the main stream, so it needs its own split-K partials buffer
-        self.wgrad_ws_aux = None
-        if self.aux_stream is not None and self.wgrad_stream is None:
-            wga = max(ops.conv_wgrad_workspace_bytes(B, c.H, c.W, c.cin, c.cout, c.k, c.stride, c.pad, c.dil)
-                      for b in self.blocks for c in (b[2],) if c is not None)
-            self.wgrad_ws_aux = torch.empty(wga, device=dev, dtype=torch.uint8)
-        self.launches = 0
+        # of the block's main branch until the residual add: it runs on a third stream.
+        self.aux_stream = torch.cuda.Stream(device=dev)
+        self.launches = 0                                   # of the last forward_backward step
+        self._split_launches: Dict[str, int] = {}           # of the last run of each split entry point
 
     # ------------------------------------------------------------------ torch flags
     def sync_flags(self) -> None:
@@ -332,7 +317,9 @@ class TrainEngine:
         return self.grad_of[id(p)]
 
     def _pack_all(self) -> int:
-        """Every conv weight -> bf16 forward + data-gradient layouts in one launch (hk_pack_conv_weights_many)."""
+        """Every block conv weight -> bf16 forward + data-gradient layouts in one launch (hk_pack_conv_weights_many_tiled: shared-memory
+        tiles of 64 output x 32 input channels, contiguous reads and 64-byte writes; it needs cout % 64 == 0 and cin % 32 == 0, which
+        every block conv of the backbone meets)."""
         import numpy as np
         key = tuple(c.conv.weight.data_ptr() for c in self.convs)
         if self._pack_items is None or key != self._pack_key:
@@ -344,29 +331,12 @@ class TrainEngine:
             self._pack_key = key
             self._pack_max = max(c.cout * c.cin * c.k * c.k for c in self.convs[1:])
             self._pack_khw = max(c.k * c.k for c in self.convs[1:])
-            # shared-memory tiled repack (contiguous reads, 64-byte writes) when every conv tiles 64 x 32; HK_PACK_TILED=0: element-wise kernel
-            self._pack_tiled = (os.environ.get("HK_PACK_TILED", "1") != "0"
-                                and all(c.cout % 64 == 0 and c.cin % 32 == 0 for c in self.convs[1:]))
             for c in self.convs:  # scale = 1 / bias = 0 of the raw convs: constant
                 c.one_out.fill_(1.0)
                 c.zero_out.zero_()
-        if self._pack_tiled:
-            check(lib().hk_pack_conv_weights_many_tiled(ptr(self._pack_items), len(self.convs) - 1, self._pack_khw, C.c_longlong(self._pack_max),
-                                                        stream_ptr()), "hk_pack_conv_weights_many_tiled")
-        else:
-            check(lib().hk_pack_conv_weights_many(ptr(self._pack_items), len(self.convs) - 1, C.c_longlong(self._pack_max), stream_ptr()),
-                  "hk_pack_conv_weights_many")
+        check(lib().hk_pack_conv_weights_many_tiled(ptr(self._pack_items), len(self.convs) - 1, self._pack_khw, C.c_longlong(self._pack_max),
+                                                    stream_ptr()), "hk_pack_conv_weights_many_tiled")
         return 1
-
-    def _pack(self, c: _ConvT, with_dgrad: bool) -> int:
-        w = c.conv.weight.data
-        check(lib().hk_pack_conv_weights(ptr(w), None, None, None, None, C.c_float(1e-5), c.cout, c.cin, c.k, c.k, HK_BF16,
-                                         ptr(c.w_fwd), ptr(c.one_out), ptr(c.zero_out), stream_ptr()), "hk_pack_conv_weights")
-        n = 2
-        if with_dgrad:
-            ops.pack_conv_weights_dgrad(w, out=c.w_dgrad)
-            n += 1
-        return n
 
     def _fold_frozen(self) -> int:
         """scale / shift / invstd of every frozen BatchNorm from its running statistics and current gamma / beta, in one launch.  Inside
@@ -384,64 +354,61 @@ class TrainEngine:
         ops.bn_fold(self._fold_items, self._fold_n, self._fold_c)
         return 1
 
+    def _conv(self, c: _ConvT, x, scale, shift, out, relu: bool = False, residual=None) -> None:
+        """The forward conv of c with a per-channel scale / shift (+ shortcut) (+ ReLU) epilogue.  The stem has a kernel of its own on
+        its own packed weights (x: the fp32 NCHW input); the others run on the inference conv kernels."""
+        if c is self.stem:
+            ops.stem_conv(x, self.stem_w, scale, shift, relu=relu, out=out)
+        else:
+            ops.conv_bn_act(x, c.w_fwd, scale, shift, stride=c.stride, pad=c.pad, dil=c.dil, relu=relu, residual=residual, out=out)
+
     def _conv_bn_frozen(self, c: _ConvT, x, out, relu: bool, residual=None) -> int:
         """BatchNorm in eval() mode: normalise with the running statistics (folded scale / shift), buffers untouched."""
         p = self.plan.convs[c.name]
         if not (p.dgamma or p.dbeta):
             # one launch: the conv epilogue applies scale / shift (+ shortcut) (+ ReLU); the backward masks with the stored output
-            ops.conv_bn_act(x, c.w_fwd, c.scale, c.shift, stride=c.stride, pad=c.pad, dil=c.dil, relu=relu, residual=residual, out=out)
+            self._conv(c, x, c.scale, c.shift, out, relu=relu, residual=residual)
             c.frozen_mask = out if relu else None
             return 1
         # gamma / beta trained: their gradients need the raw conv output y
-        ops.conv_bn_act(x, c.w_fwd, c.one_out, c.zero_out, stride=c.stride, pad=c.pad, dil=c.dil, relu=False, out=c.y)
-        bits = c.relu_bits if relu and self.use_relu_bits else None
+        self._conv(c, x, c.one_out, c.zero_out, c.y)
+        bits = c.relu_bits if relu else None
         ops.bn_apply(c.y, c.scale, c.shift, relu=relu, residual=residual, out=out, relu_bits=bits)
-        c.frozen_mask = (bits if bits is not None else out) if relu else None
+        c.frozen_mask = bits
         return 2
 
-    def _conv_bn(self, c: _ConvT, x, out, relu: bool, residual=None, ws=None) -> int:
-        """raw conv -> batch statistics (+ running stats) -> fused normalise (+ shortcut) (+ ReLU)."""
+    def _conv_bn(self, c: _ConvT, x, out, relu: bool, residual=None) -> int:
+        """raw conv -> batch statistics (+ running stats) -> fused normalise (+ shortcut) (+ ReLU, its mask as 1 bit per element)."""
         if self.plan.convs[c.name].frozen:
             return self._conv_bn_frozen(c, x, out, relu, residual)
         bn = c.bn
-        if self.use_bn_acc and self.fuse_conv_stats and ((c.k == 3 and c.cout >= 256) or (self.fuse_conv_stats_all and c is not self.stem)):
+        if c.k == 3 and c.cout >= 256:
             # the conv epilogue gathers sum y / sum y^2 of the tile it stores: no statistics pass over the activation.  Only where the
             # epilogue hides under a long mainloop (3x3 convs of layers 3-4: 36 / 72 K blocks per tile); the 64/128-channel layers and
             # the 1x1 downsample convs are epilogue-bound and lose more than the stand-alone reduction costs (measured per launch)
             ops.conv_bn_stats(x, c.w_fwd, c.one_out, c.zero_out, c.acc_f, stride=c.stride, pad=c.pad, dil=c.dil, out=c.y)
-            ops.bn_apply_acc(c.y, c.acc_f, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, c.mean, c.invstd,
-                             relu=relu, residual=residual, out=out, relu_bits=c.relu_bits if relu and self.use_relu_bits else None)
-            c.relu_out = out if relu else None
-            return 2
-        ops.conv_bn_act(x, c.w_fwd, c.one_out, c.zero_out, stride=c.stride, pad=c.pad, dil=c.dil, relu=False, out=c.y)
-        if self.use_bn_acc:
+            n = 2
+        else:
+            self._conv(c, x, c.one_out, c.zero_out, c.y)
             ops.bn_stats_acc(c.y, c.acc_f)
-            ops.bn_apply_acc(c.y, c.acc_f, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, c.mean, c.invstd,
-                             relu=relu, residual=residual, out=out, relu_bits=c.relu_bits if relu and self.use_relu_bits else None)
-            c.relu_out = out if relu else None
-            return 3
-        ops.bn_train_stats(c.y, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, c.mean, c.invstd,
-                           c.scale, c.shift, self.bn_ws if ws is None else ws)
-        ops.bn_apply(c.y, c.scale, c.shift, relu=relu, residual=residual, out=out, relu_bits=c.relu_bits if relu and self.use_relu_bits else None)
-        c.relu_out = out if relu else None
-        return 4
+            n = 3
+        ops.bn_apply_acc(c.y, c.acc_f, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, c.mean, c.invstd,
+                         relu=relu, residual=residual, out=out, relu_bits=c.relu_bits if relu else None)
+        return n
 
-    def _fork_aux(self):
-        """aux stream waits for everything enqueued on the current stream so far; returns the stream (None: stay on the current one)."""
-        if self.aux_stream is None:
-            return None
+    def _fork_aux(self) -> torch.cuda.Stream:
+        """The aux stream, made to wait for everything enqueued on the current stream so far."""
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream())
         self.aux_stream.wait_event(ev)
         return self.aux_stream
 
     def _join_aux(self) -> None:
-        if self.aux_stream is not None:
-            ev = torch.cuda.Event()
-            ev.record(self.aux_stream)
-            torch.cuda.current_stream().wait_event(ev)
+        ev = torch.cuda.Event()
+        ev.record(self.aux_stream)
+        torch.cuda.current_stream().wait_event(ev)
 
-    def _bn_bwd(self, c: _ConvT, dout, relu: bool, dy, dmasked=None, ws=None) -> int:
+    def _bn_bwd(self, c: _ConvT, dout, relu: bool, dy, dmasked=None) -> int:
         """relu: the BN output went through a ReLU; its mask is c.relu_bits (written by the forward apply pass).  dy None: the raw
         conv output needs no gradient (only dgamma / dbeta / d' are wanted)."""
         bn = c.bn
@@ -453,28 +420,19 @@ class TrainEngine:
             ops.bn_frozen_bwd(dout, c.frozen_mask, c.scale, dy, dmasked=dmasked, y=c.y if sums else None, mean=bn.running_mean,
                               invstd=c.invstd, acc=c.acc_b if sums else None, dgamma=dg, dbeta=db)
             return 1
-        if dy is None:   # the batch-statistics backward kernels always write dy
+        if dy is None:   # the batch-statistics backward kernel always writes dy
             dy = self._buf("dy_unused", c.y.shape)
-        mask = None if not relu else (c.relu_bits if self.use_relu_bits else c.relu_out)
-        if self.use_bn_acc:
-            ops.bn_bwd_acc(dout, mask, c.y, c.mean, c.invstd, bn.weight.data, c.acc_b, dg, db, dy, dmasked=dmasked)
-            return 2
-        ops.bn_train_bwd(dout, mask, c.y, c.mean, c.invstd, bn.weight.data, dg, db, dy, self.bn_ws if ws is None else ws, dmasked=dmasked)
-        return 3
+        ops.bn_bwd_acc(dout, c.relu_bits if relu else None, c.y, c.mean, c.invstd, bn.weight.data, c.acc_b, dg, db, dy, dmasked=dmasked)
+        return 2
 
-    def _dy_buf(self, c: _ConvT, role: str = "dy") -> torch.Tensor:
-        """dL/d(raw conv output) of conv c: shared scratch per shape, or (wgrads on their own stream) one buffer per conv, because the
-        weight gradient may still be reading it while the data-gradient chain has moved on."""
-        if self.wgrad_stream is None:
-            return self._buf(role, c.y.shape)
-        if getattr(c, "dy", None) is None:
+    def _dy_buf(self, c: _ConvT) -> torch.Tensor:
+        """dL/d(raw conv output) of conv c: one buffer per conv, because its weight gradient (on the wgrad stream) may still be reading
+        it while the data-gradient chain has moved on."""
+        if c.dy is None:
             c.dy = torch.empty_like(c.y)
         return c.dy
 
     def _on_wgrad_stream(self, fn) -> None:
-        if self.wgrad_stream is None:
-            fn()
-            return
         ready = torch.cuda.Event()
         ready.record(torch.cuda.current_stream())      # dy (just written on the main stream) is complete
         self.wgrad_stream.wait_event(ready)
@@ -483,15 +441,15 @@ class TrainEngine:
         self._wgrad_pending = True
 
     def _join_wgrad_stream(self) -> None:
-        if self.wgrad_stream is not None and getattr(self, "_wgrad_pending", False):
+        if self._wgrad_pending:
             done = torch.cuda.Event()
             done.record(self.wgrad_stream)
             torch.cuda.current_stream().wait_event(done)
             self._wgrad_pending = False
 
-    def _wgrad(self, c: _ConvT, x, dy, ws=None) -> int:
-        ws = self.wgrad_ws if ws is None else ws
-        self._on_wgrad_stream(lambda: ops.conv_wgrad(x, dy, self._g(c.conv.weight), k=c.k, stride=c.stride, pad=c.pad, dil=c.dil, ws=ws))
+    def _wgrad(self, c: _ConvT, x, dy) -> int:
+        self._on_wgrad_stream(lambda: ops.conv_wgrad(x, dy, self._g(c.conv.weight), k=c.k, stride=c.stride, pad=c.pad, dil=c.dil,
+                                                     ws=self.wgrad_ws))
         return 2
 
     def _dgrad(self, c: _ConvT, dy, dx, residual=None, scratch: str = "up") -> int:
@@ -512,59 +470,26 @@ class TrainEngine:
 
     def _enqueue_forward(self) -> int:
         net, K = self.net, self.K
-        n = 0
         # weights of this step (parameters change every optimizer step)
         check(lib().hk_stem_pack_weights(ptr(net.conv1.weight.data), ptr(self.stem_w), stream_ptr()), "hk_stem_pack_weights")
         self._on_wgrad_stream(self._pack_all)   # the block convs' weights are repacked while the stem, its BN and the maxpool run
-        n += 2
-        if self.use_bn_acc and self.plan.train_bn_any:
+        n = 2
+        if self.plan.train_bn_any:
             self.acc_fwd.zero_()                # the forward accumulators of every BatchNorm of this step
             n += 1
         n += self._fold_frozen()                # eval()-mode BatchNorms: scale / shift from the running statistics
         # ---------------- forward (train mode) ----------------
-        st = self.stem
-        bn = st.bn
-        sp = self.plan.convs[st.name]
-        if sp.frozen and not (sp.dgamma or sp.dbeta):
-            ops.stem_conv(self.x, self.stem_w, st.scale, st.shift, relu=True, out=self.a0)
-            st.frozen_mask = self.a0
-            n -= 3                              # conv + max-pool of the 5 counted below
-        elif sp.frozen:
-            ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
-            bits = st.relu_bits if self.use_relu_bits else None
-            ops.bn_apply(st.y, st.scale, st.shift, relu=True, out=self.a0, relu_bits=bits)
-            st.frozen_mask = bits if bits is not None else self.a0
-            n -= 2
-        elif self.use_bn_acc:
-            ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
-            ops.bn_stats_acc(st.y, st.acc_f)
-            ops.bn_apply_acc(st.y, st.acc_f, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, st.mean,
-                             st.invstd, relu=True, out=self.a0, relu_bits=st.relu_bits if self.use_relu_bits else None)
-            n -= 1
-        else:
-            ops.stem_conv(self.x, self.stem_w, st.one_out, st.zero_out, relu=False, out=st.y)
-            ops.bn_train_stats(st.y, bn.weight.data, bn.bias.data, bn.running_mean, bn.running_var, bn.momentum, bn.eps, st.mean, st.invstd,
-                               st.scale, st.shift, self.bn_ws)
-            ops.bn_apply(st.y, st.scale, st.shift, relu=True, out=self.a0, relu_bits=st.relu_bits if self.use_relu_bits else None)
-        st.relu_out = self.a0
-        if self.maxpool_idx:
-            ops.maxpool3x3s2_fwd_idx(self.a0, out=self.p0, idx=self.pool_idx)   # forward + the winning taps the backward routes through
-        else:
-            ops.maxpool3x3s2(self.a0, out=self.p0)
+        n += self._conv_bn(self.stem, self.x, self.a0, relu=True)
+        ops.maxpool3x3s2_fwd_idx(self.a0, out=self.p0, idx=self.pool_idx)   # forward + the winning taps the backward routes through
+        n += 1
         self._join_wgrad_stream()               # packed weights ready
-        n += 5
         x = self.p0
         for (c1, c2, ds, a1, sc, out) in self.blocks:
             if ds is not None:
-                aux = self._fork_aux()
-                if aux is not None:
-                    with torch.cuda.stream(aux):
-                        n += self._conv_bn(ds, x, sc, relu=False, ws=self.bn_ws_aux)
-                    n += self._conv_bn(c1, x, a1, relu=True)
-                    self._join_aux()
-                else:
-                    n += self._conv_bn(c1, x, a1, relu=True)
+                with torch.cuda.stream(self._fork_aux()):
                     n += self._conv_bn(ds, x, sc, relu=False)
+                n += self._conv_bn(c1, x, a1, relu=True)
+                self._join_aux()
                 shortcut = sc
             else:
                 n += self._conv_bn(c1, x, a1, relu=True)
@@ -597,7 +522,7 @@ class TrainEngine:
         convs = self.convs if part == "all" else self.convs[e:] if part == "late" else self.convs[:e]
         for c in convs:
             p = self.plan.convs[c.name]
-            if p.bwd and ((not p.frozen and self.use_bn_acc) or (p.frozen and (p.dgamma or p.dbeta))):
+            if p.bwd and (not p.frozen or p.dgamma or p.dbeta):
                 return True
         return False
 
@@ -642,13 +567,12 @@ class TrainEngine:
                 n += self._bn_bwd(c2, d, True, dy2, dmasked=dm)        # d' = d*[out>0] also feeds the shortcut
             dxd = None
             if pd is not None and pd.bwd:                               # shortcut branch: needs only d'; joins at the residual add
-                dyd = self._dy_buf(ds, "dyd") if pd.dy else None
+                dyd = self._dy_buf(ds) if pd.dy else None
                 dxd = self._buf("dxd", x_in.shape) if pd.dgrad else None
-                aux = self._fork_aux()
-                with torch.cuda.stream(aux if aux is not None else torch.cuda.current_stream()):
-                    n += self._bn_bwd(ds, dm, False, dyd, ws=self.bn_ws_aux)
+                with torch.cuda.stream(self._fork_aux()):
+                    n += self._bn_bwd(ds, dm, False, dyd)
                     if pd.wgrad:
-                        n += self._wgrad(ds, x_in, dyd, ws=self.wgrad_ws_aux)
+                        n += self._wgrad(ds, x_in, dyd)
                     if pd.dgrad:
                         n += self._dgrad(ds, dyd, dxd, scratch="up_aux")
             if p2.wgrad:
@@ -682,11 +606,7 @@ class TrainEngine:
             return n
         if pl.stem:
             da0 = self._buf("da0", self.a0.shape)
-            if self.maxpool_idx:
-                ops.maxpool3x3s2_bwd_idx(d, self.pool_idx, self.a0.shape[1], self.a0.shape[2], dx=da0)
-            else:
-                ops.maxpool3x3s2_bwd(d, self.a0, dx=da0, idx_ws=self.pool_idx)
-                n += 1
+            ops.maxpool3x3s2_bwd_idx(d, self.pool_idx, self.a0.shape[1], self.a0.shape[2], dx=da0)
             sp = pl.convs[st.name]
             dy0 = self._dy_buf(st) if sp.dy else None
             n += 1 + self._bn_bwd(st, da0, True, dy0)
@@ -711,7 +631,6 @@ class TrainEngine:
         if not img.is_cuda or tuple(img.shape) != (self.B, 3, self.H, self.W):
             raise ValueError(f"expected a CUDA image batch of shape {(self.B, 3, self.H, self.W)}, got {tuple(img.shape)} on {img.device}")
         self.sync_flags()
-        self.model.mark_weights_changed()   # BatchNorm running stats are advanced through raw pointers (tensor versions do not move)
         with torch.no_grad():
             self.x.copy_(img)
             if uv is not None:
@@ -723,51 +642,36 @@ class TrainEngine:
                 if self.target is None or self.target.dtype != target.dtype:
                     self.target = torch.empty_like(target, memory_format=torch.contiguous_format)
                 self.target.copy_(target)
-            if not self.use_cuda_graph:
-                self.launches = self._enqueue()
-                return self.loss
-            key = self._key()
-            if self.graph is None or key != self._graph_key:
-                # one eager step (lazy function attributes, scratch allocation), restoring the BN buffers it advanced
-                saved = [(c.bn.running_mean.clone(), c.bn.running_var.clone(), c.bn.num_batches_tracked.clone()) for c in self.convs]
-                self.launches = self._enqueue()
-                torch.cuda.current_stream().synchronize()
-                for c, (m, v, t) in zip(self.convs, saved):
-                    c.bn.running_mean.copy_(m); c.bn.running_var.copy_(v); c.bn.num_batches_tracked.copy_(t)
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g):
-                    self._enqueue()
-                self.graph, self._graph_key = g, key
-            self.graph.replay()
+            self.launches = self._run("step", self._enqueue, forward=True)
         return self.loss
 
-    # ------------------------------------------------------------------ split step: the caller owns the loss (unmodified train.py)
-    def _run(self, name: str, fn, name_key: Optional[str] = None) -> None:
-        """Eager, or capture-once / replay of one of the split graphs.  `name` "fwd" marks graphs that advance the BN buffers."""
-        if name == "fwd":
-            self.model.mark_weights_changed()   # BatchNorm running stats move (raw-pointer writes)
-        gname = name_key or name
-        counts = self.__dict__.setdefault("_split_launches", {})
+    def _run(self, name: str, fn, forward: bool = False) -> int:
+        """Run `fn` (enqueues work, returns its launch count) as eager launches, or as the CUDA graph `name`: captured on first use and
+        whenever _key() changes, replayed otherwise.  Returns the launch count.  forward: fn advances the BatchNorm buffers."""
+        if forward:
+            self.model.mark_weights_changed()   # BatchNorm running stats move (raw-pointer writes; tensor versions do not)
         if not self.use_cuda_graph:
-            counts[gname] = fn()
-            return
+            return fn()
         key = self._key()
-        graphs = self.__dict__.setdefault("_split_graphs", {})
-        ent = graphs.get(gname)
+        ent = self._graphs.get(name)
         if ent is None or ent[1] != key:
-            if name == "fwd":  # the warm-up run advances the BN buffers once more than the captured replay: restore them
+            # one eager run first (lazy function attributes, scratch allocation); it advances the BN buffers once more than the
+            # captured replay, so restore them
+            if forward:
                 saved = [(c.bn.running_mean.clone(), c.bn.running_var.clone(), c.bn.num_batches_tracked.clone()) for c in self.convs]
-            counts[gname] = fn()
+            n = fn()
             torch.cuda.current_stream().synchronize()
-            if name == "fwd":
+            if forward:
                 for c, (m, v, t) in zip(self.convs, saved):
                     c.bn.running_mean.copy_(m); c.bn.running_var.copy_(v); c.bn.num_batches_tracked.copy_(t)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 fn()
-            graphs[gname] = ent = (g, key)
+            self._graphs[name] = ent = (g, key, n)
         ent[0].replay()
+        return ent[2]
 
+    # ------------------------------------------------------------------ split step: the caller owns the loss (unmodified train.py)
     def forward_heatmaps(self, img: torch.Tensor) -> torch.Tensor:
         """Train-mode forward only: (B,3,H,W) -> sigmoid heatmaps (B,K,H,W) fp32 (model.py:19-22 under model.train()); activations
         are kept for backward_from_heatmap_grad().  Returns a view of an engine buffer."""
@@ -786,7 +690,7 @@ class TrainEngine:
 
         with torch.no_grad():
             self.x.copy_(img)
-            self._run("fwd", fn)
+            self._split_launches["fwd"] = self._run("fwd", fn, forward=True)
         return self.heat
 
     def backward_from_heatmap_grad(self, grad_heat: torch.Tensor) -> None:
@@ -799,7 +703,7 @@ class TrainEngine:
 
         with torch.no_grad():
             self.g_heat.copy_(grad_heat)
-            self._run("bwd", fn)
+            self._split_launches["bwd"] = self._run("bwd", fn)
 
     # ------------------------------------------------------------------ two-phase step for comm/compute overlap
     def forward_backward_late(self, img: torch.Tensor, uv: torch.Tensor) -> torch.Tensor:
@@ -815,21 +719,21 @@ class TrainEngine:
             self.x.copy_(img)
             self.uv.copy_(uv.reshape(self.B, self.K, 2))
             self.target = None
-            self._run("fwd", fn, name_key="late")
+            self._split_launches["late"] = self._run("late", fn, forward=True)
         return self.loss
 
     def backward_early(self) -> None:
         """Phase 2: backward of layer2, layer1 and the stem (gradients flat_grad[:late_offset]).  Nothing to do (no launch) when
         nothing there needs a gradient."""
         if not self.has_early_backward():
-            self.__dict__.setdefault("_split_launches", {})["bwd_early"] = 0
+            self._split_launches["bwd_early"] = 0
             return
         with torch.no_grad():
-            self._run("bwd_early", lambda: self._enqueue_backward("early"))
+            self._split_launches["bwd_early"] = self._run("bwd_early", lambda: self._enqueue_backward("early"))
 
     def split_launches(self) -> int:
-        """Kernel launches of the split graphs captured so far (two-phase data-parallel step: "late" + "bwd_early")."""
-        return int(sum(v or 0 for v in self.__dict__.get("_split_launches", {}).values()))
+        """Kernel launches of the split entry points run so far (two-phase data-parallel step: "late" + "bwd_early")."""
+        return sum(self._split_launches.values())
 
     def grad(self, p: torch.nn.Parameter) -> torch.Tensor:
         return self.grad_of[id(p)]

@@ -50,7 +50,7 @@ from oracle import keypoints_oracle as O
 DEV = "cuda:0"
 BF = torch.bfloat16
 LIMIT = 2 ** 22
-ENV_SWITCHES = ("HK_CONV_HALO", "HK_CONV_STRIPS", "HK_DISABLE_2CTA", "HK_DISABLE_C64", "HK_WGRAD_TAP_PAIRS", "HK_WGRAD_ROUNDS", "HK_DS_EARLY")
+ENV_SWITCHES = ("HK_CONV_HALO", "HK_CONV_STRIPS", "HK_DISABLE_2CTA", "HK_DISABLE_C64", "HK_DS_EARLY")
 _routes_overridden = pytest.mark.skipif(any(os.environ.get(v) is not None for v in ENV_SWITCHES),
                                         reason="conv / wgrad dispatch overridden: the cases are written for the default routes")
 

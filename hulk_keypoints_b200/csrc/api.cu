@@ -1,6 +1,5 @@
 // Library-level entry points (version, error text, device check) and the host helpers every launcher shares.
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "hk_common.cuh"
@@ -28,11 +27,6 @@ int check_launch(const char* what) {
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(HK_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e));
   return HK_OK;
-}
-
-bool pdl_enabled() {
-  const char* env = getenv("HK_PDL");  // read per launch: A/B runs toggle it
-  return !(env && env[0] == '0');
 }
 
 int sm_count() {

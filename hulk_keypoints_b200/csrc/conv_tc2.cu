@@ -62,7 +62,7 @@ struct ConvTc2Args {
   int num_m_tiles, num_n_tiles, cblocks;  // m tiles of 256 pixels (4 boxes)
   const float* scale2;   // DS kernels only: folded BN of the 1x1 downsample conv, ReLU flag of its epilogue (0 in the reference)
   const float* bias2;
-  int relu2, early_release, s_major;
+  int relu2, s_major;
   const float* head_w;   // HEAD kernels only: (head_k, Cout) fp32 scoring weights, (head_k) bias, (B, head_k, Ho, Wo) fp32 logits (zero on entry)
   const float* head_b;
   float* head_logits;
@@ -342,7 +342,7 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
         continue;
       }
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BLOCK_N;
-      if (DS && sub == 0 && a.early_release) {
+      if (DS && sub == 0) {
         // drain the whole accumulator first (affine + ReLU + bf16 pack in registers), hand it back to the MMA warp, then stage and store
         uint32_t pk[CHUNKS][16];
 #pragma unroll
@@ -564,8 +564,7 @@ extern "C" __attribute__((visibility("default"))) void hk_debug_set_tc2_timeline
 bool conv_tc2h_applicable(const HkConvDesc& d);
 
 bool conv_tc2_applicable(const HkConvDesc& d) {
-  static const bool disabled = getenv("HK_DISABLE_2CTA") != nullptr;
-  return !disabled && d.out_c % 128 == 0 && d.in_c % 64 == 0 && (d.stride == 1 || d.stride == 2);
+  return d.out_c % 128 == 0 && d.in_c % 64 == 0 && (d.stride == 1 || d.stride == 2);
 }
 
 template <int BLOCK_N, bool DS, bool STATS, bool HEAD = false>
@@ -641,7 +640,6 @@ static int conv_tc2_launch_impl(const HkConvDesc& d, const void* x, const void* 
   a.relu2 = ds ? ds->relu : 0;
   // K-block order of the kernel this conv would run on by itself (conv_tc2h accumulates tap column by tap column)
   a.s_major = ds && conv_tc2h_applicable(d);
-  { const char* e = getenv("HK_DS_EARLY"); a.early_release = !(e && e[0] == '0'); }   // A/B switch of the block-entry epilogue
 #ifdef HK_DIAG
   a.dbg = g_tc2_dbg;
   { const char* m = getenv("HK_TC2_DEBUG"); a.dbg_mode = m ? atoi(m) : 0; }

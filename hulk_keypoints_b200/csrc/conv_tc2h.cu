@@ -14,9 +14,8 @@
 // the MMAs at 60 rows): those bottom rows are covered by 4x32 STRIP patches instead -- same 128 accumulator rows, box (64 ch, 32 px,
 // 4 + 2*dil rows), vertical taps r*dil*4096 bytes apart.  Full patches are enumerated first, strips after them, and the boundary is
 // padded to an even index, because both CTAs of a pair must work on the same patch shape (the tap offset is part of the ONE A
-// descriptor of the cta_group::2 MMA).  HK_CONV_STRIPS=0 keeps 8x16 patches everywhere.
+// descriptor of the cta_group::2 MMA).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "hk_common.cuh"
 #include "hk_bn_acc.cuh"
@@ -315,17 +314,11 @@ conv_tc2h_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
   }
 }
 
-// HK_CONV_HALO=0 disables the variant, =1 forces it for every eligible shape, unset: the default policy below.
+// Measured per layer shape (B200): dilation 1 and 2 gain at 60x80 (+13 % / +1 %, the wasted half patch row included) and at 120x160
+// (+27 % / +6 %); the dilation-4 layer is MMA-bound either way and its 16-row boxes lose 14 % at 120x160, so it stays on the plain
+// kernel.
 bool conv_tc2h_applicable(const HkConvDesc& d) {
-  const char* env = getenv("HK_CONV_HALO");  // read per launch: tests and A/B runs toggle it
-  if (env && env[0] == '0') return false;
-  if (!(d.kh == 3 && d.kw == 3 && d.stride == 1 && d.pad == d.dil && d.out_c % 128 == 0 && d.in_c % 64 == 0)) return false;
-  if (d.dil != 1 && d.dil != 2 && d.dil != 4) return false;
-  if (env && env[0] == '1') return true;
-  // default (measured per layer shape, tools/diag_halo.py, B200): dilation 1 and 2 gain at 60x80 (+13 % / +1 %, the wasted half patch
-  // row included) and at 120x160 (+27 % / +6 %); the dilation-4 layer is MMA-bound either way and its 16-row boxes lose 14 % at
-  // 120x160, so it stays on the plain kernel
-  return d.dil <= 2;
+  return d.kh == 3 && d.kw == 3 && d.stride == 1 && d.pad == d.dil && d.out_c % 128 == 0 && d.in_c % 64 == 0 && (d.dil == 1 || d.dil == 2);
 }
 
 template <int BLOCK_N, bool STATS>
@@ -356,10 +349,8 @@ static int launch_tc2h(const CUtensorMap& mx, const CUtensorMap& mw, const CUten
 int conv_tc2h_launch(const HkConvDesc& d, const void* x, const void* w, const float* scale, const float* bias, const void* residual,
                      void* y, void* bn_acc, cudaStream_t s) {
   // patch geometry: 8x16 patches over the rows that fill whole patch rows, 4x32 strips over a remainder of 1..4 rows (see the header)
-  const char* strips_env = getenv("HK_CONV_STRIPS");
   const int rem_rows = d.out_h % TH_TILE_H;
-  // (dilation 4 strip boxes are 48 KB: three of them plus the weight ring do not fit next to the staging buffers)
-  const bool use_strips = !(strips_env && strips_env[0] == '0') && rem_rows >= 1 && rem_rows <= 4 && d.out_h > TH_TILE_H && d.dil <= 2;
+  const bool use_strips = rem_rows >= 1 && rem_rows <= 4 && d.out_h > TH_TILE_H;
   const int tiles_x = ceil_div(d.out_w, TH_TILE_W);
   const int tiles_y = use_strips ? d.out_h / TH_TILE_H : ceil_div(d.out_h, TH_TILE_H);
   const int strips_per_img = use_strips ? ceil_div(d.out_w, 2 * TH_TILE_W) : 0;

@@ -15,7 +15,6 @@
 //     8x the L1 wavefronts and made the epilogue as long as the MMA phase for this N=64 shape.
 // TMEM double buffering and the warp roles follow conv_tc_kernel.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "hk_common.cuh"
 #include "hk_bn_acc.cuh"
@@ -296,8 +295,6 @@ extern "C" __attribute__((visibility("default"))) void hk_debug_set_c64_timeline
 #endif
 
 bool conv_tc_c64_applicable(const HkConvDesc& d) {
-  static const bool disabled = getenv("HK_DISABLE_C64") != nullptr;
-  if (disabled) return false;
   if (!(d.kh == 3 && d.kw == 3 && d.stride == 1 && d.in_c == 64 && d.out_c == 64 && d.pad == d.dil)) return false;
   const int box_rows = C64_TILE_H + 2 * d.dil;
   const int smem_min = 1024 + C64_W_BYTES + 3 * box_rows * C64_ROW_BYTES + 2 * C64_STAGING_BYTES + 1024;  // at least one tile in flight

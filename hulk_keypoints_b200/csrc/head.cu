@@ -13,8 +13,6 @@
 //   2. head_upsample_sigmoid_kernel: one thread per 4 consecutive output x; ATen's align_corners
 //      arithmetic (scale=(in-1)/(out-1), src=scale*dst, lambda=src-floor) in fp32, sigmoid, float4 store.
 //      All index math is 32-bit (64-bit div/mod was the bottleneck of the first version).
-#include <stdlib.h>
-
 #include "hk_common.cuh"
 
 namespace hk {
@@ -186,7 +184,7 @@ head_upsample_sigmoid_kernel(const float* __restrict__ logits, float* __restrict
 }
 
 // ---- throughput-mode upsample: ROWS output rows per CTA, the x interpolation set-up amortised over them, optional fused argmax ----
-constexpr int kHeadRows = 32;   // rows-per-CTA sweep at 480x640 (tools/diag_upsample_rows.py): 8: 0.084 ms, 16: 0.077, 32: 0.076, 60: 0.078
+constexpr int kHeadRows = 32;   // rows-per-CTA sweep at 480x640 (B200): 8: 0.084 ms, 16: 0.077, 32: 0.076, 60: 0.078
 // grid (ceil(H / kHeadRows), B*K); each thread owns 4 consecutive output x (loops when W/4 > blockDim).  The source rows touched by the
 // CTA's output rows are staged once; per row three vertical lerps (the 4 outputs of a thread read at most 3 consecutive source columns)
 // and one horizontal lerp + sigmoid per output (the separable form of the kernel above).  (Fusing the argmax into this kernel was
@@ -327,13 +325,11 @@ static int head_upsample_impl(const float* logits_ws, float* heat, int B, int K,
   if (!sigmoid)  // training: upsampled logits in ATen's exact operation order; the sigmoid lives in hk_bce_fwd_bwd
     head_upsample_sigmoid_kernel<false, false><<<grid, threads, (size_t)2 * w * sizeof(float), s>>>(logits_ws, heat, h, w, H, W, wq, ry, rx);
   else if (fast && 3.0f * rx < 1.0f) {   // (the rows kernel assumes <= 3 source columns per 4 outputs)
-    int rows = kHeadRows;
-    { const char* e = getenv("HK_HEAD_ROWS"); if (e && atoi(e) > 0) rows = atoi(e); }   // A/B switch
-    const int nsrc = (int)(ry * (float)rows) + 3;
-    const dim3 grid2(ceil_div(H, rows), B * K);
+    const int nsrc = (int)(ry * (float)kHeadRows) + 3;
+    const dim3 grid2(ceil_div(H, kHeadRows), B * K);
     const size_t smem = (size_t)nsrc * w * sizeof(float);
     HK_REQUIRE(smem <= 48 * 1024, "hk_head_fwd: low-res row too wide for the staging buffer");
-    head_upsample_rows_kernel<<<grid2, threads, smem, s>>>(logits_ws, heat, h, w, H, W, wq, ry, rx, nsrc, rows);
+    head_upsample_rows_kernel<<<grid2, threads, smem, s>>>(logits_ws, heat, h, w, H, W, wq, ry, rx, nsrc, kHeadRows);
     return check_launch("head_upsample_rows_kernel");
   } else if (fast)
     head_upsample_sigmoid_kernel<true><<<grid, threads, (size_t)w * sizeof(float), s>>>(logits_ws, heat, h, w, H, W, wq, ry, rx);

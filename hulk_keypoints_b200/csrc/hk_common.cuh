@@ -66,8 +66,7 @@ inline int pick_block_n_pair(int out_c, long long m_tiles) {
 
 // Launch with programmatic stream serialization (PDL): the kernel may begin (prologue: barrier init, TMEM allocation, tensor-map
 // prefetch) while the previous kernel in the stream drains its last tiles; it MUST execute griddepcontrol.wait before its first
-// access to global memory.  HK_PDL=0 falls back to a plain launch.  Works under stream capture (programmatic graph edges).
-bool pdl_enabled();
+// access to global memory.  Works under stream capture (programmatic graph edges).
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
   cudaLaunchConfig_t cfg = {};
@@ -79,7 +78,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

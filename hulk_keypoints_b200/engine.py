@@ -15,7 +15,6 @@ and fp32 in precision="fp32" (all convs on the CUDA-core FFMA kernel).
 """
 from __future__ import annotations
 
-import os
 from typing import Dict, List, Optional, Tuple
 
 import torch
@@ -104,10 +103,10 @@ class InferenceEngine:
         self.use_cuda_graph = use_cuda_graph
         # stride-2 convs (layer2.0.conv1 and its 1x1 downsample) may be routed to the CUDA-core kernel
         self.stride2_algo = HK_CONV_TCGEN05
-        self.stem_on_tensor_cores = True  # bf16 mode: tcgen05 stem; False keeps the fp32 CUDA-core stem
-        self.fuse_stem_pool = os.environ.get("HK_STEM_POOL", "1") != "0"   # A/B switch: 0 = stem_tc_kernel + maxpool3x3s2_kernel
-        self.fuse_head = os.environ.get("HK_FUSE_HEAD", "1") != "0"        # A/B switch: 0 = last conv writes the feature map, head_logits_kernel reads it
-        self.fuse_downsample = os.environ.get("HK_FUSE_DS", "1") != "0"    # A/B switch: 0 = conv1 and the 1x1 downsample as two launches
+        # fused launches; False selects the unfused sequence (what the fp32 mode and unsupported shapes run), which tests compare against
+        self.fuse_stem_pool = True    # False: stem_tc_kernel + maxpool3x3s2_kernel
+        self.fuse_head = True         # False: the last conv writes the feature map, head_logits_kernel reads it
+        self.fuse_downsample = True   # False: conv1 and the 1x1 downsample as two launches
         self._packed: Optional[Dict[str, _PackedConv]] = None
         self._packed_key = None
         self._plans: Dict[Tuple[int, int, int, int], _Plan] = {}
@@ -142,7 +141,7 @@ class InferenceEngine:
         self.device = dev
         tc = self.precision == "bf16"
         packed: Dict[str, _PackedConv] = {"stem": self._pack_one(net.conv1, net.bn1, HK_CONV_FFMA)}
-        self._stem_w_tc = ops.stem_pack_weights(net.conv1.weight) if (tc and self.stem_on_tensor_cores) else None
+        self._stem_w_tc = ops.stem_pack_weights(net.conv1.weight) if tc else None
         for i, blk in enumerate(net.blocks()):
             def algo_for(conv):
                 if not tc:

@@ -51,7 +51,7 @@ typedef enum HkConvAlgo {
   HK_CONV_TCGEN05 = 0, /* bf16 operands, fp32 accumulate in TMEM, TMA-fed implicit GEMM            */
   HK_CONV_FFMA = 1,    /* fp32 CUDA-core implicit GEMM: the fp32 correctness mode (SURVEY.md §0.5) */
   HK_CONV_TCGEN05_1CTA = 2 /* force the generic single-CTA tcgen05 kernel (no cta_group::2 / layer1 specialisation);
-                              same results, kept for shapes the specialised kernels do not cover and for A/B runs */
+                              kept for shapes the specialised kernels do not cover and as the reference route tests compare against */
 } HkConvAlgo;
 
 /*

@@ -17,7 +17,6 @@ and with autograd on zero-mean gradients.  Here:
 
 Run with -s to see the measured errors.  The whole file takes about 7 s on a B200."""
 import math
-import os
 
 import numpy as np
 import pytest
@@ -301,15 +300,13 @@ CONV_CASES = [
 ]
 
 
-@pytest.mark.skipif(any(os.environ.get(v) is not None for v in ("HK_DISABLE_2CTA", "HK_DISABLE_C64", "HK_CONV_HALO")),
-                    reason="conv dispatch overridden: the cases would not reach the epilogue statistics they are written for")
 @pytest.mark.parametrize("case", CONV_CASES, ids=lambda c: "x".join(map(str, c)))
 def test_conv_epilogue_statistics_exact(case):
     """hk_conv_bn_stats_fwd with centre-tap weights w[co, co % cin] = 1 and a non-zero bias on the grid: y == x[..., co % cin] + bias
     exactly (every pad, dilation and stride), and the accumulators hold exactly the sums of y and y^2 over the image.  Every 8th channel
     has zero weights and bias +-1/8, so its sum is exactly +-P/8: a counted ragged or phantom-box row (which stages the bias) shows.
     Every case reaches a specialised epilogue kernel under the default dispatch (hk_conv_bn_stats_fwd falls back to conv + hk_bn_stats_acc only
-    outside them); the test is skipped when the dispatch switches are set."""
+    outside them)."""
     B, H, W, cin, cout, k, stride, dil = case
     pad = dil * (k - 1) // 2
     Ho, Wo = ops.conv_out_hw(H, W, k, stride, pad, dil)

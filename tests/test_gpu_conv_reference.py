@@ -32,11 +32,10 @@ What each case asserts, calling the ops exactly as TrainEngine and InferenceEngi
   E. conv_ds (both outputs), conv_head (fc rows on the 1/8 grid: the fp32 logits are exact, equal to the fp64 dot products of the
      bf16-rounded feature map), stem_pool (max-pool of the exact stem) at B = 1, 64: bit-exact.
   Route coverage: torch.profiler records the kernels one pass over the case list launches; every tcgen05 conv instance of the default
-  routes must appear.  The file is skipped when a conv / wgrad dispatch switch is set in the environment.
+  routes must appear.
 
 Run with -s to see the per-case timings.  The whole file takes about 9 s on a B200 (1000 W power limit)."""
 import math
-import os
 import re
 import zlib
 
@@ -50,13 +49,6 @@ from oracle import keypoints_oracle as O
 DEV = "cuda:0"
 BF = torch.bfloat16
 LIMIT = 2 ** 22
-ENV_SWITCHES = ("HK_CONV_HALO", "HK_CONV_STRIPS", "HK_DISABLE_2CTA", "HK_DISABLE_C64", "HK_DS_EARLY")
-_routes_overridden = pytest.mark.skipif(any(os.environ.get(v) is not None for v in ENV_SWITCHES),
-                                        reason="conv / wgrad dispatch overridden: the cases are written for the default routes")
-
-
-def gpu_test(fn):
-    return pytest.mark.gpu(_routes_overridden(fn))
 
 
 # ------------------------------------------------------------------ cases, from the network itself
@@ -252,7 +244,7 @@ def acc_values(acc, C):
 
 
 # ================================================================== A + B. forward: raw (train), epilogue statistics, folded
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", BLOCK_CASES + FWD_EDGE, ids=case_id)
 def test_forward_exact(case):
     """A: conv_bn_act with ones / zeros == the exact conv rounded once; the 3x3 Cout >= 256 convs also through conv_bn_stats (same y, sum y
@@ -292,7 +284,7 @@ def test_forward_exact(case):
 
 
 # ================================================================== C. data gradient, as TrainEngine._dgrad runs it
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", BLOCK_CASES + FWD_EDGE, ids=case_id)
 def test_dgrad_exact(case):
     """dx = conv(zero_insert2x(dy) or dy, flipped weights, pad = dil*(k-1) - pad) + residual == conv2d_input + residual, bit for bit."""
@@ -332,7 +324,7 @@ def _wgrad_check(what, run, ref, g):
     assert torch.equal(again.view(torch.int32), dw.view(torch.int32)), f"D {what}: second run not bit-identical"
 
 
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", BLOCK_CASES + FWD_EDGE + WGRAD_EDGE, ids=case_id)
 def test_wgrad_exact(case):
     """conv_wgrad (split-K tcgen05 + fixed-order reduce) == conv2d_weight exactly in fp32."""
@@ -360,7 +352,7 @@ def stem_ref(x, w):
     return nhwc(integral(F.conv2d(x.double(), w.double(), None, 2, 3, 1), "stem conv2d"))
 
 
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", STEM_CASES, ids=case_id)
 def test_stem_conv_exact(case):
     """stem_conv raw (train forward) and with a folded epilogue + ReLU, bit-exact."""
@@ -378,7 +370,7 @@ def test_stem_conv_exact(case):
     assert_exact(ops.stem_conv(x, wp, scale, shift, relu=True), rounded((ref * scale.double() + shift.double()).clamp_min(0)), "B stem_conv")
 
 
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", STEM_CASES, ids=case_id)
 def test_stem_wgrad_exact(case):
     _, B, H, W, *_ = case
@@ -391,7 +383,7 @@ def test_stem_wgrad_exact(case):
     _wgrad_check(f"stem_wgrad B{B}", lambda dw, a: ops.stem_wgrad(x, dy, dw, accumulate=a), ref, g)
 
 
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", POOL_CASES, ids=case_id)
 def test_stem_pool_exact(case):
     """E: stem_pool == max-pool 3x3 s2 p1 of the exact stem (negative scales included: the kernel pools the pre-activation extremes)."""
@@ -406,7 +398,7 @@ def test_stem_pool_exact(case):
 
 
 # ================================================================== E. inference launches at B = 1 and 64
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", DS_CASES, ids=case_id)
 def test_conv_ds_exact(case):
     """conv_ds: relu(scale*conv_kxk + shift) and scale_ds*conv_1x1 + shift_ds of the same input, both bit-exact."""
@@ -426,7 +418,7 @@ def test_conv_ds_exact(case):
     assert_exact(yds, rounded(ref_ds * sd.double() + bd.double()), f"E conv_ds downsample {name}")
 
 
-@gpu_test
+@pytest.mark.gpu
 @pytest.mark.parametrize("case", HEAD_CASES, ids=case_id)
 def test_conv_head_exact(case):
     """conv_head with K = 4 scoring rows on the 1/8 grid: the logits equal the fp64 dot products of the bf16-rounded feature map."""
@@ -502,7 +494,7 @@ def _launch_all():
                       torch.zeros(4, device=DEV), torch.empty(B, 4, H, W, device=DEV), stride=stride, pad=pad, dil=dil, residual=z(B, H, W, cout))
 
 
-@gpu_test
+@pytest.mark.gpu
 def test_cases_reach_every_default_route():
     """Every tcgen05 conv instance the default routes use is launched by the case list: conv_tc_c64, conv_tc2h at both BLOCK_N, conv_tc2
     at both BLOCK_N plus its block-entry (DS) and head instances, conv_tc_kernel<64> (the 64-channel data gradients of layer2.0),

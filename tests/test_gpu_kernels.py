@@ -481,11 +481,11 @@ def test_fused_adam_matches_torch_adam():
 
 
 HALO_CASES = [
-    (2, 60, 80, 128, 128, 3, 1, 1, True, True),     # layer2 shape (default route), height 60: half-empty last patch row
+    (2, 60, 80, 128, 128, 3, 1, 1, True, True),     # layer2 shape, height 60: half-empty last patch row
     (2, 60, 80, 128, 128, 3, 1, 1, False, False),
-    (1, 64, 80, 256, 256, 3, 1, 2, True, True),     # layer3-like, dilation 2, height multiple of 8 (default route)
-    (2, 60, 80, 128, 256, 3, 1, 2, False, True),    # layer3.0.conv1 (forced)
-    (1, 60, 80, 512, 512, 3, 1, 4, True, True),     # layer4 shape, dilation 4, 2 N tiles (forced)
+    (1, 64, 80, 256, 256, 3, 1, 2, True, True),     # layer3-like, dilation 2, height multiple of 8
+    (2, 60, 80, 128, 256, 3, 1, 2, False, True),    # layer3.0.conv1
+    (1, 60, 80, 512, 512, 3, 1, 4, True, True),     # layer4 shape, dilation 4, 2 N tiles: stays on the plain CTA-pair kernel
     (3, 21, 37, 128, 128, 3, 1, 1, True, True),     # ragged patches in both directions, odd patch count -> padding patch
     (5, 120, 160, 128, 128, 3, 1, 1, False, True),  # more tiles than clusters: ring wrap-around over many tiles
 ]
@@ -503,35 +503,30 @@ STRIP_CASES = [
 
 @pytest.mark.parametrize("case", STRIP_CASES)
 def test_conv_tcgen05_strip_patches(case):
-    """Strip patches against the oracle, and bit-identical to the all-8x16 schedule (same accumulation order per output element)."""
-    import os
-    os.environ["HK_CONV_HALO"] = "1"
-    try:
-        test_conv_tcgen05_vs_oracle(case)
-        B, H, W, cin, cout, k, stride, dil, residual, relu = case
-        x, w, s, b, res, pad = _conv_case(*case, seed=21)
-        xd = x.to(torch.bfloat16).permute(0, 2, 3, 1).contiguous().to(dev())
-        rd = None if res is None else res.to(torch.bfloat16).permute(0, 2, 3, 1).contiguous().to(dev())
-        wp, _, _ = ops.pack_conv_weights(w.to(dev()), None, 1e-5, torch.bfloat16)
-        run = lambda: ops.conv_bn_act(xd, wp, s.to(dev()), b.to(dev()), stride=stride, pad=pad, dil=dil, relu=relu, residual=rd)
-        y_strips = run()
-        os.environ["HK_CONV_STRIPS"] = "0"
-        y_plain = run()
-        assert torch.equal(y_strips, y_plain)
-    finally:
-        os.environ.pop("HK_CONV_HALO", None)
-        os.environ.pop("HK_CONV_STRIPS", None)
+    """Strip patches against the oracle, and bit-identical to the all-8x16 schedule (same accumulation order per output element).
+    The all-8x16 result comes from the same conv on the input (and residual) zero-extended at the bottom to a multiple of 8 rows:
+    output rows < H read only zeros below the input in both runs, so their first H rows must be equal."""
+    test_conv_tcgen05_vs_oracle(case)
+    B, H, W, cin, cout, k, stride, dil, residual, relu = case
+    He = -(-H // 8) * 8
+    assert H > 8 and 1 <= H % 8 <= 4 and He % 8 == 0   # strips here, none in the extended map
+    x, w, s, b, res, pad = _conv_case(*case, seed=21)
+    xd = x.to(torch.bfloat16).permute(0, 2, 3, 1).contiguous().to(dev())
+    rd = None if res is None else res.to(torch.bfloat16).permute(0, 2, 3, 1).contiguous().to(dev())
+    extend = lambda t: None if t is None else F.pad(t, (0, 0, 0, 0, 0, He - H))
+    wp, _, _ = ops.pack_conv_weights(w.to(dev()), None, 1e-5, torch.bfloat16)
+    run = lambda xx, rr: ops.conv_bn_act(xx, wp, s.to(dev()), b.to(dev()), stride=stride, pad=pad, dil=dil, relu=relu, residual=rr)
+    y_strips = run(xd, rd)
+    y_plain = run(extend(xd), extend(rd))
+    assert y_plain.shape[1] == He
+    assert torch.equal(y_strips, y_plain[:, :H])
 
 
 @pytest.mark.parametrize("case", HALO_CASES)
 def test_conv_tcgen05_haloed_operand_kernel(case):
-    """conv_tc2h (one haloed activation box per horizontal tap) against the oracle, forced on for every eligible shape."""
-    import os
-    os.environ["HK_CONV_HALO"] = "1"
-    try:
-        test_conv_tcgen05_vs_oracle(case)
-    finally:
-        os.environ.pop("HK_CONV_HALO", None)
+    """The shapes of the haloed-operand kernel (conv_tc2h, one haloed activation box per horizontal tap) against the oracle, and the
+    dilation-4 layer4 shape, which the default route keeps on conv_tc2."""
+    test_conv_tcgen05_vs_oracle(case)
 
 
 # ------------------------------------------------------------------ block entry: conv1 + 1x1 downsample in one launch (src/resnet.py:56-58,64-65,184-188)
@@ -547,11 +542,9 @@ DS_CASES = [
 
 
 @pytest.mark.parametrize("case", DS_CASES)
-@pytest.mark.parametrize("early", ["1", "0"])
-def test_conv_ds_block_entry(case, early):
+def test_conv_ds_block_entry(case):
     """hk_conv_ds_fwd: both outputs bit-identical to two hk_conv_bn_act_fwd launches, and within one bf16 rounding of the fp64 conv on
-    the same bf16 operands.  early = the accumulator-release order of the conv1 epilogue (HK_DS_EARLY)."""
-    import os
+    the same bf16 operands."""
     B, H, W, cin, cout, stride, dil = case
     g = torch.Generator().manual_seed(77)
     x = (torch.randn(B, cin, H, W, generator=g)).to(torch.bfloat16)
@@ -564,12 +557,8 @@ def test_conv_ds_block_entry(case, early):
     wdp, _, _ = ops.pack_conv_weights(wd.to(dev()), None, 1e-5, torch.bfloat16)
     sD, bD, sdD, bdD = s.to(dev()), b.to(dev()), sd.to(dev()), bd.to(dev())
     assert ops.conv_ds_supported(xd, wp, wdp, stride, dil, dil)
-    os.environ["HK_DS_EARLY"] = early
-    try:
-        y, yds = ops.conv_ds(xd, wp, sD, bD, wdp, sdD, bdD, stride=stride, pad=dil, dil=dil, relu=True)
-        torch.cuda.synchronize()
-    finally:
-        os.environ.pop("HK_DS_EARLY", None)
+    y, yds = ops.conv_ds(xd, wp, sD, bD, wdp, sdD, bdD, stride=stride, pad=dil, dil=dil, relu=True)
+    torch.cuda.synchronize()
     # the two-launch path with its default routing (dilation <= 2, stride 1 runs on the haloed kernel: hk_conv_ds_fwd then accumulates
     # its K blocks in that kernel's order, so the comparison is exact either way)
     y2 = ops.conv_bn_act(xd, wp, sD, bD, stride=stride, pad=dil, dil=dil, relu=True)
@@ -622,13 +611,10 @@ def test_conv_head_fused_logits(case):
     b_fc = (torch.randn(K, generator=g) * 0.1).to(dev())
     wp, _, _ = ops.pack_conv_weights(w, None, 1e-5, torch.bfloat16)
     assert ops.conv_head_supported(x, wp, w_fc, 1)
-    import os
-    os.environ["HK_CONV_HALO"] = "0"   # the reference feature map from the same (plain CTA-pair) kernel: the haloed one accumulates its K
-    try:                               # blocks in another order, which moves a few bf16 roundings of the feature map by one ulp
-        feat = ops.conv_bn_act(x, wp, s, b, stride=1, pad=dil, dil=dil, relu=True, residual=res)
-        torch.cuda.synchronize()
-    finally:
-        os.environ.pop("HK_CONV_HALO", None)
+    # the reference feature map from a kernel with the fused one's K-block order, (r, s, channel block): the haloed kernel, the default
+    # route at dilation 1 and 2, accumulates in another order, which moves a few bf16 roundings of the feature map by one ulp
+    feat = ops.conv_bn_act(x, wp, s, b, stride=1, pad=dil, dil=dil, relu=True, residual=res, algo=_lib.HK_CONV_TCGEN05_1CTA)
+    torch.cuda.synchronize()
     ref = torch.einsum("bhwc,kc->bkhw", feat.double(), w_fc.double()) + b_fc.double().view(1, K, 1, 1)
     logits = torch.full((B, K, H, W), float("nan"), device=dev())
     ops.conv_head(x, wp, s, b, w_fc, b_fc, logits, stride=1, pad=dil, dil=dil, relu=True, residual=res)

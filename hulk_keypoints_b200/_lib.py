@@ -36,6 +36,8 @@ EXPORTS = (
     "hk_conv_ds_fwd", "hk_bn_acc_bytes", "hk_bn_stats_acc", "hk_bn_apply_fwd_acc", "hk_bn_bwd_acc", "hk_conv_bn_stats_fwd", "hk_conv_head_fwd", "hk_head_upsample_fwd", "hk_pack_conv_weights_many_tiled", "hk_maxpool3x3s2_fwd_idx", "hk_maxpool3x3s2_bwd_idx",
     # frozen BatchNorm (eval()-mode BN inside a train()-mode model)
     "hk_bn_fold", "hk_bn_frozen_bwd",
+    # training-batch augmentation
+    "hk_augment_pick", "hk_augment_images",
 )
 
 
@@ -47,6 +49,7 @@ class HkConvDesc(C.Structure):
 
 # HkAdamSegment of include/hulk_sm100.h: one row of hk_adam_step_segments' table
 ADAM_MAX_SEGMENTS = 256
+AUGMENT_MAX_TRIES = 16   # HK_AUGMENT_MAX_TRIES
 
 
 class HkAdamSegment(C.Structure):
@@ -169,6 +172,10 @@ def _declare(lib):
     lib.hk_bce_workspace_bytes.argtypes = [C.c_longlong]
     lib.hk_bce_fwd_bwd.restype = i
     lib.hk_bce_fwd_bwd.argtypes = [vp, i, vp, i, vp, i, i, i, i, f, vp, vp, vp, sz, vp]
+    lib.hk_augment_pick.restype = i
+    lib.hk_augment_pick.argtypes = [vp, i, i, i, i, i, vp, vp, vp, vp]
+    lib.hk_augment_images.restype = i
+    lib.hk_augment_images.argtypes = [vp, vp, i, i, i, vp, i, vp, vp, f, C.c_uint64, vp]
 
 
 def lib():

@@ -341,6 +341,73 @@ def bce_fwd_bwd(pred: torch.Tensor, target: Optional[torch.Tensor] = None, uv: O
     return loss, grad
 
 
+def _overlap(a: torch.Tensor, b: torch.Tensor) -> bool:
+    """Do the memory ranges of two contiguous tensors intersect?"""
+    pa, pb = a.data_ptr(), b.data_ptr()
+    return pa < pb + b.numel() * b.element_size() and pb < pa + a.numel() * a.element_size()
+
+
+def _f32_contiguous(name: str, t: torch.Tensor, shape: Tuple[int, ...]) -> None:
+    if tuple(t.shape) != shape or t.dtype != torch.float32 or not t.is_contiguous():
+        raise ValueError(f"{name} must be a contiguous float32 tensor of shape {shape}, got {tuple(t.shape)} {t.dtype}")
+
+
+def augment_pick(fwd: torch.Tensor, uv: torch.Tensor, H: int, W: int, uv_out: Optional[torch.Tensor] = None,
+                 pick: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Per image the first of `tries` candidate label maps fwd (B,tries,2,3) fp32 that keeps all labels uv (B,K,2) inside
+    [0,W-1] x [0,H-1] -> (uv_out (B,K,2) fp32 = the moved labels, pick (B,) int32 = the candidate, -1 = none: identity).
+    uv_out must not overlap uv."""
+    _need_cuda(fwd, uv, uv_out, pick)
+    if uv.dim() != 3 or uv.shape[2] != 2 or fwd.dim() != 4:
+        raise ValueError(f"augment_pick: uv must be (B,K,2) and fwd (B,tries,2,3), got {tuple(uv.shape)} and {tuple(fwd.shape)}")
+    B, K, _ = uv.shape
+    tries = fwd.shape[1]
+    if not 1 <= tries <= _lib.AUGMENT_MAX_TRIES:
+        raise ValueError(f"augment_pick: tries must be in 1..{_lib.AUGMENT_MAX_TRIES}")
+    _f32_contiguous("uv", uv, (B, K, 2))
+    _f32_contiguous("fwd", fwd, (B, tries, 2, 3))
+    if uv_out is None:
+        uv_out = torch.empty_like(uv)
+    _f32_contiguous("uv_out", uv_out, (B, K, 2))
+    if pick is None:
+        pick = torch.empty(B, device=uv.device, dtype=torch.int32)
+    elif tuple(pick.shape) != (B,) or pick.dtype != torch.int32 or not pick.is_contiguous():
+        raise ValueError("augment_pick: pick must be a contiguous (B,) int32 tensor")
+    if _overlap(uv, uv_out):
+        raise ValueError("augment_pick: uv_out must not overlap uv (the labels are not moved in place)")
+    check(lib().hk_augment_pick(ptr(fwd), B, tries, K, H, W, ptr(uv), ptr(uv_out), ptr(pick), stream_ptr()), "hk_augment_pick")
+    return uv_out, pick
+
+
+def augment_images(img: torch.Tensor, inv: torch.Tensor, pick: torch.Tensor, photo: torch.Tensor, noise_std: float, key: int,
+                   out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """img (B,3,H,W) fp32 -> out: bilinear warp by inv[b, pick[b]] (identity for pick -1; zero outside the image), contrast / brightness
+    / per-channel gain from photo (B,5) = (c, beta, g0, g1, g2), Gaussian noise of std noise_std (Philox key `key`, 64 bits), clamp to
+    [0, 1].  One launch; out must not overlap img."""
+    _need_cuda(img, inv, pick, photo, out)
+    if img.dim() != 4 or img.shape[1] != 3 or inv.dim() != 4:
+        raise ValueError(f"augment_images: img must be (B,3,H,W) and inv (B,tries,2,3), got {tuple(img.shape)} and {tuple(inv.shape)}")
+    B, _, H, W = img.shape
+    tries = inv.shape[1]
+    if not 1 <= tries <= _lib.AUGMENT_MAX_TRIES:
+        raise ValueError(f"augment_images: tries must be in 1..{_lib.AUGMENT_MAX_TRIES}")
+    _f32_contiguous("img", img, (B, 3, H, W))
+    _f32_contiguous("inv", inv, (B, tries, 2, 3))
+    _f32_contiguous("photo", photo, (B, 5))
+    if tuple(pick.shape) != (B,) or pick.dtype != torch.int32 or not pick.is_contiguous():
+        raise ValueError("augment_images: pick must be a contiguous (B,) int32 tensor")
+    if not noise_std >= 0.0:
+        raise ValueError("augment_images: noise_std must be >= 0")
+    if out is None:
+        out = torch.empty_like(img)
+    _f32_contiguous("out", out, (B, 3, H, W))
+    if _overlap(img, out):
+        raise ValueError("augment_images: out must not overlap img (no in-place warp)")
+    check(lib().hk_augment_images(ptr(img), ptr(out), B, H, W, ptr(inv), tries, ptr(pick), ptr(photo), C.c_float(float(noise_std)),
+                                  C.c_uint64(int(key) & 0xFFFFFFFFFFFFFFFF), stream_ptr()), "hk_augment_images")
+    return out
+
+
 # ------------------------------------------------------------------------------------------------ training kernels
 def stem_conv(x: torch.Tensor, w_packed: torch.Tensor, scale: torch.Tensor, bias: torch.Tensor, relu: bool,
               out: Optional[torch.Tensor] = None) -> torch.Tensor:

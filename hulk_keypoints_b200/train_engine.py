@@ -622,21 +622,30 @@ class TrainEngine:
         return (tuple(p.data_ptr() for p in self.all_params), None if self.target is None else (self.target.data_ptr(), self.target.dtype),
                 self.sigma, self._flags)
 
-    def forward_backward(self, img: torch.Tensor, uv: Optional[torch.Tensor] = None, target: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward_backward(self, img: torch.Tensor, uv: Optional[torch.Tensor] = None, target: Optional[torch.Tensor] = None,
+                         augment=None) -> torch.Tensor:
         """img (B,3,H,W) fp32 CUDA; labels uv (B,K,2) = (x,y) [Gaussian targets generated on the fly, dataset.py:36-44] or a
         (B,K,H,W) fp64/fp32 target tensor (what KeypointsDataset returns).  Returns the fp64 mean-BCE loss (0-dim, a view of an
-        engine buffer); the gradients of all parameters are in `self.flat_grad` / `grad(p)`."""
+        engine buffer); the gradients of all parameters are in `self.flat_grad` / `grad(p)`.
+        augment: a `KeypointAugment`; its two launches write the augmented batch into the engine's input buffers in place of the copy
+        (labels only: a target tensor would need the same warp)."""
+        if augment is not None and target is not None:
+            raise ValueError("augment= moves labels (uv=); precomputed target tensors are not warped")
         if (uv is None) == (target is None):
             raise ValueError("pass exactly one of uv / target")
         if not img.is_cuda or tuple(img.shape) != (self.B, 3, self.H, self.W):
             raise ValueError(f"expected a CUDA image batch of shape {(self.B, 3, self.H, self.W)}, got {tuple(img.shape)} on {img.device}")
         self.sync_flags()
         with torch.no_grad():
-            self.x.copy_(img)
-            if uv is not None:
+            if augment is not None:
+                augment(img, uv.reshape(self.B, self.K, 2), out=self.x, uv_out=self.uv)
+                self.target = None
+            elif uv is not None:
+                self.x.copy_(img)
                 self.uv.copy_(uv.reshape(self.B, self.K, 2))
                 self.target = None
             else:
+                self.x.copy_(img)
                 if tuple(target.shape) != (self.B, self.K, self.H, self.W) or target.dtype not in (torch.float64, torch.float32):
                     raise ValueError("target must be (B,K,H,W) float64 or float32")
                 if self.target is None or self.target.dtype != target.dtype:
@@ -706,8 +715,9 @@ class TrainEngine:
             self._split_launches["bwd"] = self._run("bwd", fn)
 
     # ------------------------------------------------------------------ two-phase step for comm/compute overlap
-    def forward_backward_late(self, img: torch.Tensor, uv: torch.Tensor) -> torch.Tensor:
-        """Phase 1 of the data-parallel step: forward + loss + backward of head, layer4, layer3 (gradients flat_grad[late_offset:])."""
+    def forward_backward_late(self, img: torch.Tensor, uv: torch.Tensor, augment=None) -> torch.Tensor:
+        """Phase 1 of the data-parallel step: forward + loss + backward of head, layer4, layer3 (gradients flat_grad[late_offset:]).
+        augment: as for forward_backward."""
         if not img.is_cuda or tuple(img.shape) != (self.B, 3, self.H, self.W):
             raise ValueError(f"expected a CUDA image batch of shape {(self.B, 3, self.H, self.W)}")
         self.sync_flags()
@@ -716,8 +726,11 @@ class TrainEngine:
             return self._enqueue_forward() + self._enqueue_loss() + self._enqueue_backward("late")
 
         with torch.no_grad():
-            self.x.copy_(img)
-            self.uv.copy_(uv.reshape(self.B, self.K, 2))
+            if augment is not None:
+                augment(img, uv.reshape(self.B, self.K, 2), out=self.x, uv_out=self.uv)
+            else:
+                self.x.copy_(img)
+                self.uv.copy_(uv.reshape(self.B, self.K, 2))
             self.target = None
             self._split_launches["late"] = self._run("late", fn, forward=True)
         return self.loss

@@ -99,7 +99,7 @@ def loss_from_batch(sample_batched, model, use_cuda: bool = True, backend: str =
 
 
 def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: float = 8.0, allreduce=None,
-               backend: str = "hk", exchange: bool = True) -> torch.Tensor:
+               backend: str = "hk", exchange: bool = True, augment=None) -> torch.Tensor:
     """One step of reference train.py:33-36 (zero_grad, forward, backward, step) with targets generated from
     labels on the fly.  `optimizer` is a `hulk_keypoints_b200.optim.FusedAdam` (flat buffers: one all-reduce, one
     update kernel) or any torch optimizer; `allreduce(params)` (data-parallel exchange) runs between backward and step
@@ -108,7 +108,11 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
     `exchange=False` skips the data-parallel gradient exchange (a measurement switch: replicas then diverge).
     backend "hk" (default): the whole forward + loss + backward runs on libhulk_sm100 kernels (TrainEngine, one CUDA graph);
     with FusedAdam the engine writes the gradients straight into the optimiser's flat buffer.  backend "autograd": the
-    backbone runs on torch autograd (fp32 cuDNN) -- the checker of the parity tests, not a product path."""
+    backbone runs on torch autograd (fp32 cuDNN) -- the checker of the parity tests, not a product path.
+
+    `augment`: a `hulk_keypoints_b200.augment.KeypointAugment` applied to (img, uv) on the device before the step.  On the engine its
+    launches write the engine's input buffers (in place of the batch copy), outside the captured graph, so every step draws new
+    parameters; on the autograd backend the same augmenter runs first and the torch graph sees the same batch."""
     fused = hasattr(optimizer, "flat_grad")
     if backend == "hk":
         eng = model.train_engine(img.shape[0], img.shape[2], img.shape[3])
@@ -120,7 +124,7 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
                 optimizer.adopt_grad_buffer(eng.flat_grad, eng.params)
         import torch.distributed as dist
         if not exchange:   # measurement only (bench.py: the step with its gradient exchange switched off = the compute-only time)
-            loss = eng.forward_backward(img, uv=uv)
+            loss = eng.forward_backward(img, uv=uv, augment=augment)
             if not fused:
                 eng.grads_into_params()
             optimizer.step()
@@ -129,14 +133,14 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
             # data-parallel: the all-reduce of layer3/layer4/fc gradients (91 % of the bytes) overlaps the backward of layers 2..1 + stem.
             # (Also running the Adam update of that range beside the early backward was measured at 2 GPUs, batch 4: 3.957 ms against
             # 3.943 ms with one update at the end -- the update is an HBM stream that slows the backward it overlaps -- and dropped.)
-            loss = eng.forward_backward_late(img, uv)
+            loss = eng.forward_backward_late(img, uv, augment=augment)
             w1 = optimizer.all_reduce_range_async(eng.late_offset, optimizer.numel)
             eng.backward_early()
             w0 = optimizer.all_reduce_range_async(0, eng.late_offset)
             optimizer.finish_all_reduce([w1, w0])
             optimizer.step()
             return loss.detach().clone()
-        loss = eng.forward_backward(img, uv=uv)
+        loss = eng.forward_backward(img, uv=uv, augment=augment)
         if fused:
             optimizer.all_reduce_grads()
         else:
@@ -145,6 +149,8 @@ def train_step(model, optimizer, img: torch.Tensor, uv: torch.Tensor, sigma: flo
                 allreduce(model.parameters())
         optimizer.step()
         return loss.detach().clone()
+    if augment is not None:
+        img, uv = augment(img, uv)
     if fused:
         optimizer.zero_grad()
     else:

@@ -371,6 +371,28 @@ HK_API int hk_head_bwd(const float* g_up, const void* feat, const float* w_fc, f
                        float* db_fc, int accumulate, int B, int K, int C, int h, int w, int H, int W, void* ws, size_t ws_bytes,
                        void* stream);
 
+/* ---- training-batch augmentation ----
+ * Replaces the domain-randomisation pipeline of src/dataset.py:18-31 (imgaug, commented out there) and, for warped labels, the label
+ * clipping of :63-66: a random affine warp with the (x, y) pixel-index labels moved by the same map, then photometric jitter.  The
+ * caller draws per image `tries` candidate geometries A(p) = s*R(theta)*(p - ctr) + ctr + t, ctr = ((W-1)/2, (H-1)/2), as 2x3 row-major
+ * fp32 matrices: fwd (B, tries, 2, 3) maps labels, inv (B, tries, 2, 3) = A^-1 maps output pixels to input pixels.
+ *   hk_augment_pick   : pick (B) int32 = the first candidate under which all K labels of image b lie in [0, W-1] x [0, H-1], or -1
+ *                       (identity geometry) if none does; uv_out (B,K,2) = the labels under that candidate (x' = (m0*x + m1*y) + m2, one
+ *                       fp32 rounding per operation), or uv unchanged for -1.  uv_out must not overlap uv (HK_ERR_BAD_ARG).
+ *   hk_augment_images : in, out (B,3,H,W) fp32 NCHW, distinct and non-overlapping (HK_ERR_BAD_ARG otherwise).
+ *                       out(p) = bilinear(in, inv[b, pick[b]](p)) with pixel centres at integer coordinates and zero outside the image
+ *                       (grid_sample(align_corners=True, padding_mode="zeros")); then per channel, in fp32 and in this order:
+ *                       v = (v - 0.5)*c + 0.5 + beta; v *= g_ch; v += noise_std*n; v = clamp(v, 0, 1), with photo (B,5) = (c, beta,
+ *                       g0, g1, g2).  n ~ N(0,1) from Philox4x32-10 with the 64-bit `key` (low word first) and counter (x/4, y, channel, b),
+ *                       one Box-Muller output of four normals per 4 horizontally adjacent pixels.  With identity geometry, c = 1,
+ *                       beta = 0, g = 1 and noise_std = 0 an image with values in [0, 1] is returned bit for bit.
+ * Both are capturable (no allocation, no synchronisation). */
+#define HK_AUGMENT_MAX_TRIES 16
+HK_API int hk_augment_pick(const float* fwd, int B, int tries, int K, int H, int W, const float* uv, float* uv_out, int32_t* pick,
+                           void* stream);
+HK_API int hk_augment_images(const float* in, float* out, int B, int H, int W, const float* inv, int tries, const int32_t* pick,
+                             const float* photo, float noise_std, uint64_t key, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

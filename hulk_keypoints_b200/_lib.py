@@ -38,6 +38,8 @@ EXPORTS = (
     "hk_bn_fold", "hk_bn_frozen_bwd",
     # training-batch augmentation
     "hk_augment_pick", "hk_augment_images",
+    # every keypoint instance: thresholded local-maximum peaks
+    "hk_peak_workspace_bytes", "hk_peak_decode",
 )
 
 
@@ -50,6 +52,7 @@ class HkConvDesc(C.Structure):
 # HkAdamSegment of include/hulk_sm100.h: one row of hk_adam_step_segments' table
 ADAM_MAX_SEGMENTS = 256
 AUGMENT_MAX_TRIES = 16   # HK_AUGMENT_MAX_TRIES
+PEAK_MAX_PEAKS, PEAK_MAX_DISTANCE = 256, 16   # limits of hk_peak_decode
 
 
 class HkAdamSegment(C.Structure):
@@ -95,6 +98,10 @@ def _declare(lib):
     lib.hk_argmax_workspace_bytes.argtypes = [i, i, i, i]
     lib.hk_argmax_decode.restype = i
     lib.hk_argmax_decode.argtypes = [vp, i, i, i, i, vp, vp, vp, sz, vp]
+    lib.hk_peak_workspace_bytes.restype = sz
+    lib.hk_peak_workspace_bytes.argtypes = [i, i, i, i, i, i]
+    lib.hk_peak_decode.restype = i
+    lib.hk_peak_decode.argtypes = [vp, i, i, i, i, i, i, f, vp, vp, vp, vp, sz, vp]
     lib.hk_gauss_targets.restype = i
     lib.hk_gauss_targets.argtypes = [vp, i, i, i, i, f, vp, i, vp]
     lib.hk_stem_packed_weight_bytes.restype = sz

@@ -10,6 +10,7 @@ Data layout in HBM (per plan, B images of H x W):
   logits  (B,K,H/8,W/8)    fp32        -- K live rows of the scoring conv
   heat    (B,K,H,W)        fp32 NCHW   -- what KeypointsGauss.forward returns
   yx      (B,K,2)          int32       -- argmax decode
+  peaks   (B,K,N,2) int32, (B,K,N) fp32, (B,K) int32 + workspace -- peak decode, allocated on the first peaks() call
 act dtype is bf16 in precision="bf16" (tcgen05 convs; stem on the fp32 CUDA-core kernel with bf16 output)
 and fp32 in precision="fp32" (all convs on the CUDA-core FFMA kernel).
 """
@@ -78,8 +79,10 @@ class _Plan:
         self.yx = torch.empty((B, K, 2), device=dev, dtype=torch.int32)
         self.maxval = torch.empty((B, K), device=dev, dtype=torch.float32)
         self.argmax_ws = torch.empty(max(1, ops.argmax_workspace_bytes(B, K, H, W)), device=dev, dtype=torch.uint8)
+        self.peaks: Optional[Tuple[torch.Tensor, ...]] = None   # (yx, score, count, ws) of the peak decode, sized for (N, r)
+        self._peaks_r = 0
         self.graph: Optional[torch.cuda.CUDAGraph] = None
-        self.graph_decode: Optional[bool] = None
+        self.graph_decode = None   # (decode mode, input_is_u8) the graph was captured with
         self.launches = 0
 
     @property
@@ -88,6 +91,17 @@ class _Plan:
             shape, dev, adt = self._stem_spec
             self._stem = torch.empty(shape, device=dev, dtype=adt)
         return self._stem
+
+    def peak_buffers(self, N: int, r: int) -> Tuple[torch.Tensor, ...]:
+        K = self.heat.shape[1]
+        if self.peaks is None or self.peaks[0].shape[2] != N or self._peaks_r != r:
+            dev = self.heat.device
+            self.peaks = (torch.empty((self.B, K, N, 2), device=dev, dtype=torch.int32),
+                          torch.empty((self.B, K, N), device=dev, dtype=torch.float32),
+                          torch.empty((self.B, K), device=dev, dtype=torch.int32),
+                          torch.empty(max(8, ops.peak_workspace_bytes(self.B, K, self.H, self.W, N, r)), device=dev, dtype=torch.uint8))
+            self._peaks_r = r
+        return self.peaks
 
     def view(self, i: int, h: int, w: int, c: int) -> torch.Tensor:
         return self.pool[i][: self.B * h * w * c].view(self.B, h, w, c)
@@ -163,8 +177,9 @@ class InferenceEngine:
         ops.conv_bn_act(x, pc.w, pc.scale, pc.bias, stride=pc.stride, pad=pc.pad, dil=pc.dil, relu=relu, residual=residual,
                         out=out, algo=pc.algo, in_is_nchw=in_is_nchw)
 
-    def _enqueue(self, plan: _Plan, decode: bool) -> int:
-        """Enqueue the whole forward on the current stream.  Returns the number of kernel launches."""
+    def _enqueue(self, plan: _Plan, decode) -> int:
+        """Enqueue the whole forward on the current stream.  Returns the number of kernel launches.
+        decode: False (heatmaps only), True (argmax into plan.yx / plan.maxval) or ("peaks", N, threshold, r) (plan.peaks)."""
         net = self.model.resnet.resnet34_8s
         P = self._packed
         n = 0
@@ -216,7 +231,11 @@ class InferenceEngine:
             x, cur, h, w = y, free[2], ho, wo
         if not head_done:
             ops.head(x, self._fc_w, self._fc_b, plan.H, plan.W, heat=plan.heat, logits_ws=plan.logits); n += 2
-        if decode:
+        if isinstance(decode, tuple):
+            _, N, thr, r = decode
+            yx, score, count, ws = plan.peak_buffers(N, r)
+            ops.peak_decode(plan.heat, N, thr, r, yx=yx, score=score, count=count, ws=ws); n += 2
+        elif decode:
             ops.argmax_decode(plan.heat, yx=plan.yx, maxval=plan.maxval, ws=plan.argmax_ws, want_max=True); n += 2
         return n
 
@@ -243,8 +262,9 @@ class InferenceEngine:
             plan.x_u8 = torch.empty((B, H, W, 3), device=self.device, dtype=torch.uint8)
         return plan.x_u8
 
-    def run_plan(self, plan: _Plan, decode: bool) -> None:
-        """Run the forward on `plan.x` (already filled) into plan.heat / plan.yx."""
+    def run_plan(self, plan: _Plan, decode) -> None:
+        """Run the forward on `plan.x` (already filled) into plan.heat and the decode's buffers (decode as for _enqueue).  The graph is
+        recaptured whenever the decode mode, its peak parameters or the input dtype change."""
         if not self.use_cuda_graph:
             plan.launches = self._enqueue(plan, decode)
             return
@@ -258,8 +278,9 @@ class InferenceEngine:
             plan.graph, plan.graph_decode = g, (decode, plan.input_is_u8)
         plan.graph.replay()
 
-    def forward(self, x: torch.Tensor, decode: bool = False, clone: bool = True, slot: int = 0):
-        """(B,3,H,W) / (3,H,W) fp32, or (B,H,W,3) / (H,W,3) uint8 (cv2 layout), CUDA -> heat (B,K,H,W) fp32 [, yx (B,K,2)].
+    def forward(self, x: torch.Tensor, decode=False, clone: bool = True, slot: int = 0):
+        """(B,3,H,W) / (3,H,W) fp32, or (B,H,W,3) / (H,W,3) uint8 (cv2 layout), CUDA -> heat (B,K,H,W) fp32 [, yx (B,K,2)]
+        [, (yx (B,K,N,2), score (B,K,N), count (B,K)) for decode=("peaks", N, threshold, r)].
         clone=False returns views of the plan's buffers (valid until the next call on the same slot); when `x` IS the plan's own
         input buffer (staging_input) no copy is made."""
         u8 = x.dtype == torch.uint8
@@ -291,6 +312,9 @@ class InferenceEngine:
                 plan.input_is_u8 = False
             self.run_plan(plan, decode)
             heat = plan.heat.clone() if clone else plan.heat
+            if isinstance(decode, tuple):
+                peaks = plan.peaks[:3]
+                return heat, (tuple(t.clone() for t in peaks) if clone else peaks)
             if decode:
                 return heat, (plan.yx.clone() if clone else plan.yx)
             return heat

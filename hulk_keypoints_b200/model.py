@@ -279,6 +279,20 @@ class KeypointsGauss(nn.Module):
         H, W = (x.shape[1], x.shape[2]) if x.dtype == torch.uint8 else (x.shape[-2], x.shape[-1])
         return yx, eng.plan_for(B, H, W, slot).maxval
 
+    def peaks(self, x, max_peaks: int = 16, threshold: float = 0.5, min_distance: int = 8, slot: int = 0):
+        """Additive serving API: eval-mode forward + peak decode -> every instance of each keypoint channel, (yx int32 (B,K,N,2) as
+        (row, col), score fp32 (B,K,N), count int32 (B,K)), N = max_peaks.  A peak is a pixel >= threshold that is greater than every
+        earlier and at least every later pixel of its (2r+1)^2 window, r = min_distance (default: the training sigma, config.py's
+        GAUSS_SIGMA = 8); the top N per map by score, unused slots (-1, -1) / -inf.  Like keypoints(): one CUDA graph, no heatmap
+        copy, and the results are views of engine buffers, valid until the next call on the same `slot`."""
+        if self.training:
+            raise RuntimeError("peaks() is an inference call; use model.eval() first")
+        from .ops import check_peak_args
+
+        N, thr, r = check_peak_args(max_peaks, threshold, min_distance)
+        _, out = self.engine().forward(x, decode=("peaks", N, thr, r), clone=False, slot=slot)
+        return out
+
     def staging_input(self, batch: int, height: int, width: int, slot: int = 0, uint8: bool = False):
         """Device input buffer of serving slot `slot`: `buf.copy_(pinned_host_images, non_blocking=True)` then `keypoints(buf, slot)`;
         two slots give H2D / compute double buffering with no device-to-device copy."""

@@ -6,6 +6,7 @@ libhulk_sm100.so enqueued on torch's current stream.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional, Tuple
 
 import torch
@@ -270,6 +271,55 @@ def argmax_decode(heat: torch.Tensor, yx: Optional[torch.Tensor] = None, maxval:
     check(lib().hk_argmax_decode(ptr(heat), B, K, H, W, ptr(yx), ptr(maxval), ptr(ws), ws.numel() * ws.element_size(),
                                  stream_ptr()), "hk_argmax_decode")
     return (yx, maxval) if want_max else yx
+
+
+def check_peak_args(max_peaks: int, threshold: float, min_distance: int) -> Tuple[int, float, int]:
+    """Validate peak_decode's parameters -> (N, the threshold rounded to fp32 as the kernel sees it, r).  Raises ValueError."""
+    if isinstance(max_peaks, bool) or int(max_peaks) != max_peaks or not 1 <= max_peaks <= _lib.PEAK_MAX_PEAKS:
+        raise ValueError(f"max_peaks must be an integer in [1, {_lib.PEAK_MAX_PEAKS}], got {max_peaks!r}")
+    if isinstance(min_distance, bool) or int(min_distance) != min_distance or not 1 <= min_distance <= _lib.PEAK_MAX_DISTANCE:
+        raise ValueError(f"min_distance must be an integer in [1, {_lib.PEAK_MAX_DISTANCE}], got {min_distance!r}")
+    thr = C.c_float(float(threshold)).value
+    if not math.isfinite(thr):
+        raise ValueError(f"threshold must be finite in fp32, got {threshold!r}")
+    return int(max_peaks), thr, int(min_distance)
+
+
+def peak_workspace_bytes(B: int, K: int, H: int, W: int, max_peaks: int, min_distance: int) -> int:
+    return int(lib().hk_peak_workspace_bytes(B, K, H, W, max_peaks, min_distance))
+
+
+def peak_decode(heat: torch.Tensor, max_peaks: int, threshold: float, min_distance: int, yx: Optional[torch.Tensor] = None,
+                score: Optional[torch.Tensor] = None, count: Optional[torch.Tensor] = None, ws: Optional[torch.Tensor] = None):
+    """Every local maximum of each (H, W) map of a (B,K,H,W) fp32 heatmap: pixels >= threshold that are greater than every earlier
+    and at least every later pixel of their (2r+1)^2 window (r = min_distance; NaN counts as -inf), the top max_peaks per map by
+    value, ties by flat index.  Returns (yx (B,K,N,2) int32 (row, col), score (B,K,N) fp32, count (B,K) int32); unused slots hold
+    (-1, -1) and -inf."""
+    N, thr, r = check_peak_args(max_peaks, threshold, min_distance)
+    _need_cuda(heat, yx, score, count, ws)
+    if heat.dtype != torch.float32 or heat.dim() != 4 or not heat.is_contiguous():
+        raise ValueError("peak_decode needs a contiguous (B,K,H,W) fp32 heatmap")
+    B, K, H, W = heat.shape
+    if min(B, K, H, W) < 1 or B * K > 65535 or H * W >= 2 ** 31 - 1:
+        raise ValueError(f"peak_decode: unsupported shape {tuple(heat.shape)} (needs B*K <= 65535 and H*W < 2^31)")
+    for name, t, shape, dt in (("yx", yx, (B, K, N, 2), torch.int32), ("score", score, (B, K, N), torch.float32),
+                               ("count", count, (B, K), torch.int32)):
+        if t is not None and (tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous()):
+            raise ValueError(f"peak_decode: {name} must be a contiguous {dt} tensor of shape {shape}")
+    if yx is None:
+        yx = torch.empty((B, K, N, 2), device=heat.device, dtype=torch.int32)
+    if score is None:
+        score = torch.empty((B, K, N), device=heat.device, dtype=torch.float32)
+    if count is None:
+        count = torch.empty((B, K), device=heat.device, dtype=torch.int32)
+    nbytes = peak_workspace_bytes(B, K, H, W, N, r)
+    if ws is None:
+        ws = torch.empty(nbytes, device=heat.device, dtype=torch.uint8)
+    elif ws.numel() * ws.element_size() < nbytes:
+        raise ValueError(f"peak_decode: workspace of {ws.numel() * ws.element_size()} bytes, needs {nbytes}")
+    check(lib().hk_peak_decode(ptr(heat), B, K, H, W, N, r, C.c_float(thr), ptr(yx), ptr(score), ptr(count), ptr(ws),
+                               ws.numel() * ws.element_size(), stream_ptr()), "hk_peak_decode")
+    return yx, score, count
 
 
 def soft_argmax(heat: torch.Tensor, want_int: bool = True):

@@ -7,7 +7,8 @@ they normalise each image with its own batch statistics; the B200 inference path
 statistics instead ("BN folded at inference").  Pass bn_mode="as_written" to keep train-mode BN.
 
 Additive API: `decode(heatmap)` runs the argmax of reference prediction.py:46 on the GPU for EVERY batch
-element (the reference's `plot` decodes element 0 only, on the host).
+element (the reference's `plot` decodes element 0 only, on the host); `peaks(heatmap)` returns every thresholded local maximum of
+each channel, the top N per map.
 """
 from __future__ import annotations
 
@@ -43,6 +44,16 @@ class Prediction:
             heatmap = torch.from_numpy(np.ascontiguousarray(heatmap, dtype=np.float32)).cuda()
         heat = heatmap.detach().float().contiguous()
         return ops.argmax_decode(heat).cpu().numpy().astype(np.int64)
+
+    def peaks(self, heatmap, max_peaks: int = 16, threshold: float = 0.5, min_distance: int = 8):
+        """Additive API: every instance per channel of a (B,K,H,W) heatmap (CUDA tensor or numpy) -> numpy (yx int64 (B,K,N,2) as
+        (y, x), score float32 (B,K,N), count int64 (B,K)): local maxima >= threshold, at most one per (2r+1)^2 window (r =
+        min_distance), the top N = max_peaks per map by score; unused slots (-1, -1) / -inf.  See ops.peak_decode."""
+        ops.check_peak_args(max_peaks, threshold, min_distance)
+        if isinstance(heatmap, np.ndarray):
+            heatmap = torch.from_numpy(np.ascontiguousarray(heatmap, dtype=np.float32)).cuda()
+        yx, score, count = ops.peak_decode(heatmap.detach().float().contiguous(), max_peaks, threshold, min_distance)
+        return yx.cpu().numpy().astype(np.int64), score.cpu().numpy(), count.cpu().numpy().astype(np.int64)
 
     # ---- kept callable for API parity; host-side helpers of the reference (prediction.py:26-38) ----
     def softmax(self, x):

@@ -171,6 +171,18 @@ HK_API size_t hk_argmax_workspace_bytes(int B, int K, int H, int W);
 HK_API int hk_argmax_decode(const float* heat, int B, int K, int H, int W, int32_t* yx, float* maxval_or_null,
                      void* ws, size_t ws_bytes, void* stream);
 
+/* Every instance per channel (additive; the reference decodes one argmax per channel): thresholded local maxima, top N per map.
+ * Pixel p with value v is a peak iff v >= threshold, v > q for every neighbour q of its (2r+1)x(2r+1) window (clipped to the image)
+ * that precedes p in row-major order, and v >= q for every neighbour after p; NaN counts as -inf (never a peak, suppresses nothing).
+ * On a flat top only the first pixel survives; on a NaN-free map the top-1 peak is hk_argmax_decode's (row, col) and value.
+ *   heat (B,K,H,W) fp32 contiguous ; r = min_distance in [1, 16] ; N = max_peaks in [1, 256] ; threshold finite
+ *   yx (B,K,N,2) int32 = (row, col), score (B,K,N) fp32: the peaks by value descending, ties by flat index ascending; unused slots
+ *   hold (-1, -1) and -inf ; count (B,K) int32 = peaks kept (<= N)
+ *   ws : hk_peak_workspace_bytes(B,K,H,W,N,r) bytes of scratch, 8-byte aligned (0 for arguments out of range) */
+HK_API size_t hk_peak_workspace_bytes(int B, int K, int H, int W, int max_peaks, int min_distance);
+HK_API int hk_peak_decode(const float* heat, int B, int K, int H, int W, int max_peaks, int min_distance, float threshold,
+                          int32_t* yx, float* score, int32_t* count, void* ws, size_t ws_bytes, void* stream);
+
 /* Soft-argmax of every (H, W) map: Prediction.expectation, src/prediction.py:31-38 (called at :45), softmax (:26-29) included.
  * The reference's flattening quirk is kept: the map is flattened column-major (`d.T.ravel()`, flat index i = c*H + r) while the
  * index arrays assume row-major order (x' = i % W, y' = i // W).  One pass over the heatmaps (online softmax; fp32 exp, fp64 sums).
